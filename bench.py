@@ -7,7 +7,7 @@ whole cache: every group's K and V gathered and factorised (16 matrices of 65536
 consumed with inputs resident in HBM; `e2e` is the same through host buffers (pinned H2D of the KV and D2H of the
 factors inside the timed region); `decode` is the fused reconstruct + attention over the factors (tok/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5] [--dump-outputs DIR]
 
 N > 1 is launched with torchrun.  The headline `value` is the contract's weak-scaling number (every rank compresses a
 whole 8-group cache of its own: layer groups are independent, no data-path collective).  Two more multi-GPU records
@@ -33,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the source tree as it found it (it may be read-only)
 
 # BASELINE.json configs (index = position in `configs`, 1-based as SURVEY.md section 8 numbers them)
 CONFIGS = {
@@ -73,7 +74,14 @@ def parse_args():
                     "instead of reading the layer tensors in place")
     ap.add_argument("--factorize-opts", default="", help="JSON of FactorizeOptions overrides for the timed step (tuning experiments)")
     ap.add_argument("--no-graph", action="store_true", help="enqueue every kernel from the host instead of replaying a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the factors of the last step to DIR/<name>.npy (float32, sampled rows)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the factors of the xkv_b200 arm; the reference arm keeps no outputs")
+    return args
 
 
 def config_of(args):
@@ -351,6 +359,46 @@ class CompressStep:
             return self.out
         self.out = self.enqueue()
         return self.out
+
+
+DUMP_BYTES = 64 * 10**6     # --dump-outputs: all files together stay below this
+DUMP_SEED = 0
+
+
+def dump_outputs(factors, out_dir, budget=DUMP_BYTES):
+    """Write what one compress step returns (a GroupFactors per layer group) as float32 .npy files: for group g and side
+    s in (k, v), `group{g}_{s}_A` (token factor, tokens x rank), `group{g}_{s}_V` (right factor, n x rank) and
+    `group{g}_{s}_sigma` (leading singular values).  A 2-D factor with more rows than the budget allows is written as a
+    fixed sample of its rows: the ascending indices numpy.random.default_rng(DUMP_SEED).choice(rows, k, replace=False),
+    one k for every 2-D array, so equal shapes give equal rows in every run.  Returns {name: shape written}."""
+    import numpy as np
+    import torch
+
+    arrays = {}
+    for g, gf in enumerate(factors):
+        for side, f in (("k", gf.key), ("v", gf.value)):
+            if f is None:
+                continue
+            arrays[f"group{g}_{side}_A"] = f.A
+            arrays[f"group{g}_{side}_V"] = f.V
+            if f.sigma_lead is not None:
+                arrays[f"group{g}_{side}_sigma"] = f.sigma_lead
+    header = 256                # bound on a .npy header (128 bytes for these shapes)
+    fixed = header * len(arrays) + sum(4 * t.numel() for t in arrays.values() if t.dim() == 1)
+    cols = sum(t.shape[1] for t in arrays.values() if t.dim() == 2)
+    max_rows = (budget - fixed) // (4 * cols) if cols else 0
+    if cols and max_rows < 1:
+        raise ValueError(f"--dump-outputs: {len(arrays)} arrays do not fit in {budget} bytes")
+    os.makedirs(out_dir, exist_ok=True)
+    shapes = {}
+    for name, t in arrays.items():
+        if t.dim() == 2 and t.shape[0] > max_rows:
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(t.shape[0], max_rows, replace=False))
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        a = t.float().cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        shapes[name] = list(a.shape)
+    return shapes
 
 
 def gram_roofline(ctx, c, keys, ms_step):
@@ -792,6 +840,8 @@ def run_xkv_arm(args):
     ms_step = ctx.max_ms(e0.elapsed_time(e1)) / args.steps
     clocks = sampler.stop() if rank == 0 else None
     value = world * kv_bytes / (ms_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
 
     ridge = ctx.peak_tf * 1e12 / (ctx.peak_hbm * 1e9)
     # SURVEY 8d: the two-pass minimum does 4 m n r flops over 4 m n bytes, i.e. r flop/B: HBM-bound below the ridge

@@ -11,6 +11,8 @@ from xkv_b200 import cli
 from xkv_b200.configurations import xKVConfig
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# a checkout of the original xKV repository, when one is at hand: the reference-parity test below reads it
+REFERENCE = os.environ.get("XKV_REFERENCE_ROOT", "")
 
 
 def _parse(argv):
@@ -76,11 +78,12 @@ def test_root_utils_module_reexports():
     assert root_utils.apply_kv_compress_patch is cli.apply_kv_compress_patch
 
 
-@pytest.mark.skipif(not os.path.isfile("/root/reference/utils.py"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not (REFERENCE and os.path.isfile(os.path.join(REFERENCE, "utils.py"))),
+                    reason="needs XKV_REFERENCE_ROOT, a checkout of the original xKV repository")
 def test_flags_equal_the_reference_parser():
     """Every add_argument call of the reference's add_common_args (utils.py:96-137), read from its source text (the
     module itself imports loguru / the HF hub stack), against the parser built here: same flags, defaults, actions."""
-    src = open("/root/reference/utils.py").read()
+    src = open(os.path.join(REFERENCE, "utils.py")).read()
     body = src[src.index("def add_common_args"):]
     calls = re.findall(r"add_argument\(\s*(['\"])(--[\w]+)\1(.*?)\)\s*\n", body, flags=re.S)
     ours = {a.option_strings[0]: a for a in cli.add_common_args(argparse.ArgumentParser())._actions if a.option_strings

@@ -13,6 +13,8 @@ from xkv_b200.configurations import (
 )
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+# a checkout of the original xKV repository, when one is at hand: the reference-parity tests below read it
+REFERENCE = os.environ.get("XKV_REFERENCE_ROOT", "")
 
 
 def test_defaults_match_reference():
@@ -93,21 +95,22 @@ def test_shipped_configs_load(path):
         assert cfg.get_group_for_layer(g.layers[0]) is g
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/configs"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "configs"))),
+                    reason="needs XKV_REFERENCE_ROOT, a checkout of the original xKV repository")
 @pytest.mark.parametrize("name", ["example.yaml", "example_xkv_config.yaml", "grouped_layers.yaml"])
 def test_reference_yaml_files_load_unchanged(name):
     import importlib.util
 
-    cfg = xKVConfig.from_yaml(os.path.join("/root/reference/configs", name))
+    cfg = xKVConfig.from_yaml(os.path.join(REFERENCE, "configs", name))
     # the reference class, executed as the checker (loaded by path so it does not shadow the repo's xKV shim)
-    spec = importlib.util.spec_from_file_location("_ref_xkv_configurations", "/root/reference/xKV/configurations.py")
+    spec = importlib.util.spec_from_file_location("_ref_xkv_configurations", os.path.join(REFERENCE, "xKV", "configurations.py"))
     mod = importlib.util.module_from_spec(spec)
     import sys
 
     sys.modules[spec.name] = mod      # dataclasses resolves string annotations through sys.modules
     spec.loader.exec_module(mod)
     RefConfig = mod.xKVConfig
-    ref = RefConfig.from_yaml(os.path.join("/root/reference/configs", name))
+    ref = RefConfig.from_yaml(os.path.join(REFERENCE, "configs", name))
     assert cfg.to_dict() == ref.to_dict()
     assert [(g.layers, g.rank_k, g.rank_v, g.slerp_t, g.slerp_gamma) for g in cfg.layer_groups] == \
            [(g.layers, g.rank_k, g.rank_v, g.slerp_t, g.slerp_gamma) for g in ref.layer_groups]

@@ -76,7 +76,5 @@ def test_reference_import_paths_resolve():
 def test_ops_fail_loudly_without_a_gpu():
     from xkv_b200 import _lib, ops
 
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
     with pytest.raises(_lib.XkvError):
         ops.pack_group([torch.zeros(1, 1, 8, 8, dtype=torch.bfloat16)])
