@@ -94,10 +94,9 @@ typedef struct xkv_gemm_problem {
 XKV_API int xkv_gemm_grouped(const xkv_gemm_problem* problems_host, int num_problems, void* stream);
 /* sizeof(xkv_gemm_problem) of this build (bindings check their mirror of the struct against it) */
 XKV_API size_t xkv_gemm_problem_size(void);
-/* test / tuning hook: a launch whose problems are all Grams (G = X^T X: both operands MN-major, sym_upper, one term,
- * fp32 output) runs in CTA pairs (cta_group::2, one 256 x 256 tile per pair: gram_pair_kernel); 0 sends it through the
- * single-CTA 128 x 256 tiles of every other product, 1 (default) restores the pairs, 3 .. 7 = pairs with that many
- * 32 KiB ring stages per CTA instead of the default 6.  Same results bit for bit. */
+/* test hook: nonzero (default) lets a launch whose problems all qualify run in CTA pairs (cta_group::2, one 256 x bn
+ * tile per pair: gemm_pair_kernel -- the Gram, the projection, the power step, the triangular solve); 0 sends every
+ * launch through the single-CTA 128 x 256 tiles (gemm_kernel).  Same results bit for bit. */
 XKV_API void xkv_gemm_set_gram_pair(int on);
 
 /* ---- small fp32 helpers of the factorisation ------------------------------------------ */
@@ -169,9 +168,6 @@ XKV_API int xkv_cholesky_inverse(float* const* S_host, float* const* Linv_host, 
 XKV_API int xkv_cholesky_inverse_limbs(float* const* S_host, float* const* Linv_host, void* const* hi_host,
                                        void* const* mid_host, void* const* lo_host, int batch, int l, int64_t ld,
                                        int64_t ld_limb, float shift, float pivot_floor, void* stream);
-/* tuning hook: cap on the thread-block cluster size per matrix of the Cholesky launch (0 = automatic: 8 CTAs from 6 block
- * columns up, 16 from 20 up where the device can keep them resident).  Fewer CTAs per matrix hold fewer SMs for longer. */
-XKV_API void xkv_cholesky_set_cluster_cap(int cap);
 /* Shared-memory two-sided Jacobi eigen-solver for the Rayleigh-Ritz windows: `count` symmetric W x W
  * fp32 matrices (W even, <= 160), one CTA each. evals: eigenvalues sorted descending; Wt (optional):
  * eigenvectors as rows, same order. */
@@ -248,21 +244,6 @@ XKV_API int xkv_factorize_groups(const void* const* layer_ptrs_host, int batch, 
                                  int64_t ld_layer, int rank, const xkv_factorize_options* opts, void* const* A_host,
                                  void* const* Vt_host, void* const* V_host, float* const* sigma_host, void* workspace,
                                  size_t workspace_bytes, void* const* stage_events_host, void* stream);
-/* Matrices of DIFFERENT rank in one batch (ranks_host[b]; same shape): a layer group's K and V matrices share every
- * launch of the latency-bound stages (Cholesky clusters, Jacobi windows, the elementwise kernels), which otherwise run
- * once per rank value with half the matrices each.  The ranks of a batch must give one Rayleigh-Ritz window width
- * (always the case when every sketch is at least `window` wide).  sigma / workspace sizes: the _mixed size query. */
-XKV_API size_t xkv_factorize_workspace_bytes_mixed(int batch, int m, int n, const int32_t* ranks_host,
-                                                   const xkv_factorize_options* opts);
-XKV_API int xkv_factorize_groups_mixed(const void* const* layer_ptrs_host, int batch, int layers, int layer_cols, int m,
-                                       int64_t ld_layer, const int32_t* ranks_host, const xkv_factorize_options* opts,
-                                       void* const* A_host, void* const* Vt_host, void* const* V_host,
-                                       float* const* sigma_host, void* workspace, size_t workspace_bytes,
-                                       void* const* stage_events_host, void* stream);
-XKV_API int xkv_factorize_batch_mixed(const void* const* X_host, int batch, int m, int n, int64_t ldx,
-                                      const int32_t* ranks_host, const xkv_factorize_options* opts, void* const* A_host,
-                                      void* const* Vt_host, void* const* V_host, float* const* sigma_host, void* workspace,
-                                      size_t workspace_bytes, void* const* stage_events_host, void* stream);
 XKV_API int xkv_factorize_batch(const void* const* X_host, int batch, int m, int n, int64_t ldx, int rank,
                                 const xkv_factorize_options* opts, void* const* A_host, void* const* Vt_host,
                                 void* const* V_host, float* const* sigma_host, float* const* gram_host,
@@ -304,8 +285,6 @@ XKV_API void xkv_decode_force_tiled(int on);
  * cta_group::2, half a right-factor slice per CTA), 1 FFMA epilogue, 2 score MMA with one independent CTA per kv head,
  * 3 CTA pairs; 4 = automatic scores kernel, but slab reduction and combine as two launches (default: one cluster launch) */
 XKV_API void xkv_decode_set_variant(int variant);
-/* tuning hook: cap on the TMA ring depth (16 KiB slots of A_k in flight per CTA) of the pair kernel: 0 automatic, else >= 3 */
-XKV_API void xkv_decode_set_stages(int stages);
 /* Absorbed attention over a token factor: replaces, for the MLA latent slot (deepseek_v2.py:217-235: reconstructed
  * latents -> kv_a_layernorm -> kv_b_proj over the WHOLE cache -> attention, every decode step), the part that touches
  * the cache.  The latent of token t is c_t = V_l a_t and both attention products are linear in it, so with the query

@@ -17,7 +17,6 @@ ap = argparse.ArgumentParser()
 ap.add_argument("S", type=int, nargs="?", default=65536)
 ap.add_argument("layers", type=int, nargs="?", default=4)
 ap.add_argument("--variant", type=int, default=0)
-ap.add_argument("--stages", type=int, default=0)
 ap.add_argument("--graph", action="store_true")
 ap.add_argument("--rk", type=int, default=512)
 ap.add_argument("--rv", type=int, default=768)
@@ -36,7 +35,6 @@ q = torch.randn(HQ, D, device=dev).bfloat16()
 kt = torch.randn(H, 1, D, device=dev).bfloat16()
 vt = torch.randn(H, 1, D, device=dev).bfloat16()
 _lib.load().xkv_decode_set_variant(args.variant)
-_lib.load().xkv_decode_set_stages(args.stages)
 ws = torch.empty(ops.decode_workspace_bytes(HQ, S, 1, RV) + 4096, dtype=torch.uint8, device=dev)
 o = torch.empty(HQ, D, dtype=torch.bfloat16, device=dev)
 
@@ -57,7 +55,7 @@ run()
 e1.record()
 torch.cuda.synchronize()
 torch.cuda.profiler.stop()
-res = {"S": S, "layers": layers, "variant": args.variant, "stages": args.stages,
+res = {"S": S, "layers": layers, "variant": args.variant,
        "us_per_layer_host_enqueue": 1e3 * e0.elapsed_time(e1) / layers}
 if args.graph:
     g = torch.cuda.CUDAGraph()

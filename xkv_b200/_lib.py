@@ -121,7 +121,6 @@ SIGNATURES = {
     "xkv_set_launch_predicate": (None, [_vp]),
     "xkv_cholesky_inverse": (_i, [_pp, _pp, _i, _i, _i64, _f, _f, _vp]),
     "xkv_cholesky_inverse_limbs": (_i, [_pp, _pp, _pp, _pp, _pp, _i, _i, _i64, _i64, _f, _f, _vp]),
-    "xkv_cholesky_set_cluster_cap": (None, [_i]),
     "xkv_jacobi_eigh": (_i, [_pp, _pp, _pp, _i, _i, _i64, _i64, _i, _vp]),
     "xkv_convert_bf16": (_i, [_vp, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp]),
     "xkv_sqrt_clamp": (_i, [_vp, _vp, _i, _vp]),
@@ -137,7 +136,6 @@ SIGNATURES = {
     "xkv_decode_absorbed": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _vp, _vp, _i64, _i, _f, _vp, _vp, _vp, _sz, _vp]),
     "xkv_decode_force_tiled": (None, [_i]),
     "xkv_decode_set_variant": (None, [_i]),
-    "xkv_decode_set_stages": (None, [_i]),
     "xkv_rope_bf16": (_i, [_vp, _i64, _i, _i, _i, _vp, _vp, _i64, _vp]),
     "xkv_append_workspace_bytes": (_sz, [_i, _i, _i]),
     "xkv_append_project": (_i, [_vp, _i64, _i, _vp, _i64, _i, _i, _vp, _i64, _vp, _sz, _vp]),
@@ -148,11 +146,6 @@ SIGNATURES = {
     "xkv_gemm_set_gram_pair": (None, [_i]),
     "xkv_factorize_groups": (_i, [_pp, _i, _i, _i, _i, _i64, _i, C.POINTER(FactorizeOptions), _pp, _pp, _pp, _pp, _vp, _sz,
                                   _pp, _vp]),
-    "xkv_factorize_workspace_bytes_mixed": (_sz, [_i, _i, _i, _vp, C.POINTER(FactorizeOptions)]),
-    "xkv_factorize_groups_mixed": (_i, [_pp, _i, _i, _i, _i, _i64, _vp, C.POINTER(FactorizeOptions), _pp, _pp, _pp, _pp, _vp,
-                                        _sz, _pp, _vp]),
-    "xkv_factorize_batch_mixed": (_i, [_pp, _i, _i, _i, _i64, _vp, C.POINTER(FactorizeOptions), _pp, _pp, _pp, _pp, _vp, _sz,
-                                       _pp, _vp]),
     "xkv_factorize_batch": (_i, [_pp, _i, _i, _i, _i64, _i, C.POINTER(FactorizeOptions), _pp, _pp, _pp, _pp, _pp, _i,
                                  _vp, _sz, _pp, _vp]),
 }

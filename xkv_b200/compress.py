@@ -27,7 +27,6 @@ class GroupFactors:
 
 
 _side_streams = {}
-_MIXED_GROUPS_PER_JOB = 8     # K + V matrices of 8 groups = 16 matrices = XKV_MAX_BATCH per driver call
 
 
 def _side_stream(device: torch.device, index: int = 0, priority: int = 0) -> torch.cuda.Stream:
@@ -61,10 +60,6 @@ def compress_groups(
     extra_rows: int = 0,
     in_place: bool = True,
     job_events: Optional[list] = None,
-    mixed: bool = False,
-    priorities: Optional[Sequence[int]] = None,
-    stagger: bool = False,
-    v_first: bool = False,
 ) -> List[GroupFactors]:
     """Compress equally-shaped layer groups. keys[g][i] / values[g][i]: (1, H, S, D) bf16 of layer i of
     group g (keys PRE-RoPE, as the reference hands them over, llama.py:49).
@@ -72,15 +67,7 @@ def compress_groups(
     The K matrices and the V matrices are independent factorisations; they are cut into up to
     `num_streams` batches that run on separate CUDA streams, so that the latency-bound stages of one batch
     (Cholesky panels, Jacobi) overlap the tensor-core GEMMs of another.  `in_place=False` forces the gather kernel +
-    packed-matrix path (the two give bit-identical factors; tests compare them).  `mixed`: when both sides are compressed the
-    K and V matrices of a chunk of groups go through ONE driver call with per-matrix ranks, so that every latency-bound
-    launch (Cholesky clusters, Jacobi windows, elementwise kernels) carries both.  Built, parity-tested and measured
-    SLOWER at config 2 (48.4 ms against 18.3 + 24.4 ms for the two batches: the 16-matrix Gram launch alone takes 17.7 ms
-    against 6.9 + 6.6 ms — a power-capped part sustains a 7 ms tensor burst at a higher clock than a 17 ms one — and the
-    latency-bound stages did not shrink), so it is off by default; see DESIGN.md.  `priorities`: stream priority of job j
-    (jobs: the K chains in group order, then the V chains; cycled when shorter).  `stagger`: every chain's Gram launch waits
-    for the Gram of the chain enqueued before it (measured: within the noise of the simultaneous start, off by default);
-    `v_first`: enqueue the V chains before the K chains."""
+    packed-matrix path (the two give bit-identical factors; tests compare them)."""
     ng = len(keys)
     if ng == 0:
         return []
@@ -91,45 +78,6 @@ def compress_groups(
     if keys[0][0].shape[0] != 1:
         raise XkvError("compress: batch size 1 per call (the reference's batched SVD is one SVD per sample)")
     sides = (["k"] if merge_key else []) + (["v"] if merge_value else [])
-    if v_first:
-        sides.reverse()
-    # ---- K and V matrices of a chunk of groups in ONE driver call (different ranks, one set of launches) ----
-    # Needs token-major layer tensors (read in place) and sketch widths that share a Rayleigh-Ritz window.
-    if (mixed and in_place and len(sides) == 2 and rank_k != rank_v and len(keys[0]) <= 16
-            and factorize.mixed_ranks_ok([rank_k, rank_v], opts)):
-        rows_k = [[factorize.layer_rows(t) for t in grp] for grp in keys]
-        rows_v = [[factorize.layer_rows(t) for t in grp] for grp in values]
-        if all(r is not None for grp in rows_k + rows_v for r in grp):
-            per_job = max(1, min(_MIXED_GROUPS_PER_JOB, 32 // len(keys[0])))
-            njobs = max((ng + per_job - 1) // per_job, min(max(num_streams // 2, 1), ng))
-            size = (ng + njobs - 1) // njobs
-            used = []
-            for j, lo in enumerate(range(0, ng, size)):
-                hi = min(lo + size, ng)
-                stream = main if (lo + size >= ng or num_streams <= 1) else _side_stream(dev, j)
-                if stream is not main:
-                    stream.wait_stream(main)
-                    used.append(stream)
-                with torch.cuda.stream(stream):
-                    if job_events is not None:
-                        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                        job_events.append((j, (rank_k, rank_v), 2 * (hi - lo), ev0, ev1))
-                        ev0.record()
-                    fs = factorize.factorize_groups(rows_k[lo:hi] + rows_v[lo:hi], [rank_k] * (hi - lo) + [rank_v] * (hi - lo),
-                                                    opts, extra_rows=extra_rows)
-                    if job_events is not None:
-                        job_events[-1][4].record()
-                for i in range(hi - lo):
-                    kf[lo + i], vf[lo + i] = fs[i], fs[hi - lo + i]
-                if stream is not main:
-                    for f in fs:
-                        for t in (f.A_storage, f.Vt, f.V, f.sigma_lead):
-                            if t is not None:
-                                t.record_stream(main)
-            for stream in used:
-                main.wait_stream(stream)
-            ids = layer_ids if layer_ids is not None else [list(range(len(g))) for g in keys]
-            return [GroupFactors(layers=list(ids[g]), key=kf[g], value=vf[g]) for g in range(ng)]
     jobs = []   # (target list, first group, groups, rank)
     per_side = max(1, num_streams // max(len(sides), 1))
     for side in sides:
@@ -145,13 +93,10 @@ def compress_groups(
     # of another.  Measured (bench step, 10 steps, two runs): no priorities, last job on the caller's stream 44.3 / 43.1 ms;
     # all side streams 41.9; priorities -1 / -2 / -3 dealt round-robin 39.2 - 39.8 (8 jobs).  With both sides compressed the
     # chains of the larger rank (the longer ones: wider sketch, more Cholesky block steps) get the top priority -3 and the
-    # others -1, so that all chains end together: 37.9 / 38.1 -> 37.1 / 37.2 ms same box (tools/ab_priorities.py; the
-    # device has four levels, 0 .. -3; the reverse order costs 0.6 ms, distinct levels per chain gain nothing).
-    prev_gram = None   # staggered start: a chain's Gram launch waits for the Gram of the chain enqueued before it
+    # others -1, so that all chains end together: 37.9 / 38.1 -> 37.1 / 37.2 ms same box (profiles/r02_priorities_ab.jsonl;
+    # the device has four levels, 0 .. -3; the reverse order costs 0.6 ms, distinct levels per chain gain nothing).
     for j, (dst, lo, groups, rank) in enumerate(jobs):
-        if priorities:
-            prio = priorities[j % len(priorities)]
-        elif len(sides) == 2 and rank_k != rank_v:
+        if len(sides) == 2 and rank_k != rank_v:
             prio = -3 if rank == max(rank_k, rank_v) else -1   # the longer chains (wider sketch) first
         else:
             prio = -1 - (j % 3)
@@ -159,9 +104,6 @@ def compress_groups(
         if stream is not main:
             stream.wait_stream(main)
             used.append(stream)
-            if prev_gram is not None:
-                stream.wait_event(prev_gram)
-        gram_done = torch.cuda.Event() if (stagger and stream is not main) else None
         with torch.cuda.stream(stream):
             if job_events is not None:
                 ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -171,10 +113,8 @@ def compress_groups(
             # layout goes through the gather kernel first (reference cache:170-171 + :13-14)
             rows = [[factorize.layer_rows(t) for t in grp] for grp in groups] if in_place else None
             if rows is not None and all(r is not None for grp in rows for r in grp) and len(groups[0]) <= 16:
-                fs = factorize.factorize_groups(rows, rank, opts, extra_rows=extra_rows, gram_done=gram_done)
-                prev_gram = gram_done
+                fs = factorize.factorize_groups(rows, rank, opts, extra_rows=extra_rows)
             else:
-                prev_gram = None
                 xs = pack_groups(groups)
                 fs = factorize.factorize_batch(xs, rank, opts, extra_rows=extra_rows)
                 if stream is not main:

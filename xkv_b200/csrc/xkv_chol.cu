@@ -45,8 +45,7 @@ struct CholFusedParams {
   __nv_bfloat16* hi[XKV_MAX_BATCH];
   __nv_bfloat16* mid[XKV_MAX_BATCH];
   __nv_bfloat16* lo[XKV_MAX_BATCH];
-  int l, nblk;                 // uniform size (grid sizing, cluster size)
-  int l_b[XKV_MAX_BATCH];      // per-matrix size (0: the uniform l); see batch_rows_override
+  int l, nblk;                 // matrix size and its number of CB blocks
   long long ld, ld_limb;
   float pivot_floor, shift;
   const int* run_if;   // optional per-matrix device predicate (xkv_set_launch_predicate): the whole cluster exits
@@ -273,8 +272,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chol_cluster_kernel(const __gri
   float* S = p.S[blockIdx.y];
   float* Li = p.Linv[blockIdx.y];
   const long long ld = p.ld;
-  const int lsize = p.l_b[blockIdx.y] > 0 ? p.l_b[blockIdx.y] : p.l;
-  const int nblk = lsize / CB;
+  const int nblk = p.nblk;
   const int tid = threadIdx.x;
   auto blk = [&](float* base, int bi, int bj) -> float* {
     return base + static_cast<long long>(bi) * CB * ld + static_cast<long long>(bj) * CB;
@@ -420,8 +418,8 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chol_cluster_kernel(const __gri
   __nv_bfloat16* hi = p.hi[blockIdx.y];
   __nv_bfloat16* mid = p.mid[blockIdx.y];
   __nv_bfloat16* lo = p.lo[blockIdx.y];
-  const int l4 = lsize >> 2;
-  for (int r = c; r < lsize; r += CL) {
+  const int l4 = p.l >> 2;
+  for (int r = c; r < p.l; r += CL) {
     const int bi = r / CB;
     float* row = Li + static_cast<long long>(r) * ld;
     for (int q = tid; q < l4; q += CH_THREADS) {
@@ -450,9 +448,6 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chol_cluster_kernel(const __gri
 
 using namespace xkv;
 
-static int g_chol_cluster_cap = 0;   // xkv_cholesky_set_cluster_cap
-extern "C" void xkv_cholesky_set_cluster_cap(int cap) { g_chol_cluster_cap = cap; }
-
 extern "C" int xkv_cholesky_inverse_limbs(float* const* S_host, float* const* Linv_host, void* const* hi_host,
                                           void* const* mid_host, void* const* lo_host, int batch, int l, int64_t ld,
                                           int64_t ld_limb, float shift, float pivot_floor, void* stream) {
@@ -472,14 +467,6 @@ extern "C" int xkv_cholesky_inverse_limbs(float* const* S_host, float* const* Li
     p.mid[b] = mid_host ? static_cast<__nv_bfloat16*>(mid_host[b]) : nullptr;
     p.lo[b] = lo_host ? static_cast<__nv_bfloat16*>(lo_host[b]) : nullptr;
   }
-  {
-    const int* ov = batch_rows_override();
-    for (int b = 0; b < XKV_MAX_BATCH; ++b) {
-      p.l_b[b] = (ov != nullptr && b < batch) ? ov[b] : 0;
-      XKV_REQUIRE(p.l_b[b] % CB == 0 && p.l_b[b] <= ld, "cholesky: per-matrix size %d must be a multiple of %d within ld", p.l_b[b], CB);
-      if (p.l_b[b] > l) l = p.l_b[b];
-    }
-  }
   p.l = l;
   p.nblk = l / CB;
   p.ld = ld;
@@ -494,7 +481,6 @@ extern "C" int xkv_cholesky_inverse_limbs(float* const* S_host, float* const* Li
     attr_set() = true;
   }
   int CL = p.nblk >= 6 ? 8 : (p.nblk >= 3 ? 4 : (p.nblk == 2 ? 2 : 1));
-  if (g_chol_cluster_cap > 0 && CL > g_chol_cluster_cap) CL = g_chol_cluster_cap;
   cudaLaunchConfig_t cfg;
   std::memset(&cfg, 0, sizeof(cfg));
   cfg.blockDim = dim3(CH_THREADS, 1, 1);
@@ -521,7 +507,7 @@ extern "C" int xkv_cholesky_inverse_limbs(float* const* S_host, float* const* Li
     (void)cudaGetLastError();
     cl16_probe = 1 + cl16_clusters;
   }
-  if (p.nblk >= 20 && cl16_probe - 1 >= batch && g_chol_cluster_cap == 0) CL = 16;
+  if (p.nblk >= 20 && cl16_probe - 1 >= batch) CL = 16;
   cfg.gridDim = dim3(CL, batch, 1);
   attr[0].val.clusterDim.x = CL;
   XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, chol_cluster_kernel, p));

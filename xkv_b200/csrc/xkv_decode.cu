@@ -49,18 +49,7 @@ struct alignas(64) ScoreParams {
   int S, rk, H, qpk, tiles_n, nkb;
   int stages;   // ring slots of the score-MMA kernel
   float scale;
-#ifdef XKV_PROBE
-  int dbg;   // tools/probe_decode_scores.cu: bisect switches, compiled out of the library
-#endif
 };
-
-#ifdef XKV_PROBE
-static int g_probe_dbg = 0;
-static int g_probe_stages = 0;
-#define XKV_DBG(P, bit) (((P).dbg & (bit)) != 0)
-#else
-#define XKV_DBG(P, bit) false
-#endif
 
 __device__ __forceinline__ float bf16r(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
@@ -577,7 +566,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
     if (elect_one()) {   // the whole producer loop in one lane (see the MMA warp)
       int s = 0;
       uint32_t ph = 0;
-      for (int tile = slot; tile < ntiles && !XKV_DBG(P, 64); tile += nslots) {
+      for (int tile = slot; tile < ntiles; tile += nslots) {
         for (int kb = 0; kb < P.nkb; ++kb) {
           mbar_wait(&empty_bar[s], ph ^ 1u);
           mbar_expect_tx(&full_bar[s], D_A_BYTES);
@@ -608,23 +597,18 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
       int s = 0, acc = 0;
       uint32_t ph = 0, acc_ph = 0u;
       for (int tile = slot; tile < ntiles; tile += nslots) {
-        if (!XKV_DBG(P, 4)) mbar_wait(&tempty_bar[acc], ((acc_ph >> acc) & 1u) ^ 1u);
+        mbar_wait(&tempty_bar[acc], ((acc_ph >> acc) & 1u) ^ 1u);
         tc_fence_after();
         const uint32_t d_addr = tmem_base + static_cast<uint32_t>(acc * D);
         uint64_t b_desc = b_desc0;
         for (int kb = 0; kb < P.nkb; ++kb) {
-          if (!XKV_DBG(P, 64)) mbar_wait(&full_bar[s], ph);
+          mbar_wait(&full_bar[s], ph);
           tc_fence_after();
-          if (!XKV_DBG(P, 1)) {
-            umma_bf16_ss(d_addr, a_desc, b_desc, idesc, kb > 0 ? 1u : 0u);
-            umma_bf16_ss(d_addr, a_desc + kKStep, b_desc + kKStep, idesc, 1u);
-            umma_bf16_ss(d_addr, a_desc + 2 * kKStep, b_desc + 2 * kKStep, idesc, 1u);
-            umma_bf16_ss(d_addr, a_desc + 3 * kKStep, b_desc + 3 * kKStep, idesc, 1u);
-          }
-          if (XKV_DBG(P, 512)) {
-            // probe: no per-stage commit
-          } else
-            umma_commit(&empty_bar[s]);
+          umma_bf16_ss(d_addr, a_desc, b_desc, idesc, kb > 0 ? 1u : 0u);
+          umma_bf16_ss(d_addr, a_desc + kKStep, b_desc + kKStep, idesc, 1u);
+          umma_bf16_ss(d_addr, a_desc + 2 * kKStep, b_desc + 2 * kKStep, idesc, 1u);
+          umma_bf16_ss(d_addr, a_desc + 3 * kKStep, b_desc + 3 * kKStep, idesc, 1u);
+          umma_commit(&empty_bar[s]);
           b_desc += kBlockStep;
           a_desc += kStageStep;
           if (++s == R_STAGES) {
@@ -639,43 +623,39 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
       }
     }
     __syncwarp();
-  } else if (XKV_DBG(P, 4)) {
-    // probe: no epilogue pipeline at all
   } else if (warp == 2) {
-    if (!XKV_DBG(P, 16)) {
-      // scores[128 x 16] = K^rot (TMEM, 64 packed columns) * Q^T (shared memory, K-major)
-      constexpr uint32_t idesc2 = umma_idesc_bf16(DBM, R_QROWS, 0, 0);
-      mbar_wait(q_bar, 0);
-      const uint32_t q_base = smem_u32(sQ);
-      if (elect_one()) {
-        const uint64_t q_desc0 = umma_desc_sw128(q_base, 16, 1024);
-        int b = 0;
-        uint32_t bph = 0u;
-        for (int tile = slot; tile < ntiles; tile += nslots) {
-          mbar_wait(&a2full_bar[b], (bph >> b) & 1u);                 // rotated keys of this tile are in TMEM
-          mbar_wait(&d2empty_bar[b], ((bph >> b) & 1u) ^ 1u);         // score buffer read out
-          tc_fence_after();
-          const uint32_t a2 = tmem_base + R_COL_A2 + static_cast<uint32_t>(b * 64);
-          const uint32_t d2 = tmem_base + R_COL_D2 + static_cast<uint32_t>(b * 32);
+    // scores[128 x 16] = K^rot (TMEM, 64 packed columns) * Q^T (shared memory, K-major)
+    constexpr uint32_t idesc2 = umma_idesc_bf16(DBM, R_QROWS, 0, 0);
+    mbar_wait(q_bar, 0);
+    const uint32_t q_base = smem_u32(sQ);
+    if (elect_one()) {
+      const uint64_t q_desc0 = umma_desc_sw128(q_base, 16, 1024);
+      int b = 0;
+      uint32_t bph = 0u;
+      for (int tile = slot; tile < ntiles; tile += nslots) {
+        mbar_wait(&a2full_bar[b], (bph >> b) & 1u);                 // rotated keys of this tile are in TMEM
+        mbar_wait(&d2empty_bar[b], ((bph >> b) & 1u) ^ 1u);         // score buffer read out
+        tc_fence_after();
+        const uint32_t a2 = tmem_base + R_COL_A2 + static_cast<uint32_t>(b * 64);
+        const uint32_t d2 = tmem_base + R_COL_D2 + static_cast<uint32_t>(b * 32);
 #pragma unroll
-          for (int k = 0; k < D / 16; ++k)
-            umma_bf16_ts(d2, a2 + static_cast<uint32_t>(k * 8),
-                         q_desc0 + static_cast<uint64_t>(((k >> 2) * (R_Q_BYTES / 2) + (k & 3) * 32) >> 4), idesc2, k > 0 ? 1u : 0u);
-          umma_commit(&d2full_bar[b]);
-          umma_commit(&a2empty_bar[b]);
-          bph ^= 1u << b;
-          b ^= 1;
-        }
+        for (int k = 0; k < D / 16; ++k)
+          umma_bf16_ts(d2, a2 + static_cast<uint32_t>(k * 8),
+                       q_desc0 + static_cast<uint64_t>(((k >> 2) * (R_Q_BYTES / 2) + (k & 3) * 32) >> 4), idesc2, k > 0 ? 1u : 0u);
+        umma_commit(&d2full_bar[b]);
+        umma_commit(&a2empty_bar[b]);
+        bph ^= 1u << b;
+        b ^= 1;
       }
-      __syncwarp();
     }
+    __syncwarp();
   } else if (warp >= 4 && warp < 4 + R_EPI_WARPS) {
     // ===== epilogue: K^ row -> bf16 -> RoPE (packed bf16) -> back to TMEM as the A operand of the score MMA =====
     const int qd = warp & 3;
     const int half = (warp - 4) >> 2;
     const int row = qd * 32 + lane;
     const int d0 = half * 32;           // this thread rotates the pairs (d, d + 64), d in [d0, d0 + 32)
-    const bool rope = P.cos != nullptr && !XKV_DBG(P, 8);
+    const bool rope = P.cos != nullptr;
     int acc = 0;
     uint32_t acc_ph = 0u;
     for (int tile = slot; tile < ntiles; tile += nslots) {
@@ -730,11 +710,6 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
           hi_w[j] = *reinterpret_cast<const uint32_t*>(&o2);
         }
       }
-      if (XKV_DBG(P, 16)) {
-        acc_ph ^= 1u << acc;
-        acc ^= 1;
-        continue;
-      }
       // K^rot -> TMEM (column c = dims 2c, 2c+1): wait until the score MMAs of two tiles ago released the buffer
       mbar_wait(&a2empty_bar[acc], ((acc_ph >> acc) & 1u) ^ 1u);
       tc_fence_after();
@@ -749,7 +724,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
       acc_ph ^= 1u << acc;
       acc ^= 1;
     }
-  } else if (warp >= 4 + R_EPI_WARPS && !XKV_DBG(P, 16)) {
+  } else if (warp >= 4 + R_EPI_WARPS) {
     // ===== score read-out: one warp per TMEM lane quarter, thread = token =====
     const int qd = warp & 3;
     const int row = qd * 32 + lane;
@@ -1459,7 +1434,6 @@ static inline int decode_split_k(int S, int rv) {
 static bool g_force_tiled_scores = false;  // test hook: exercise the tile-per-CTA scores kernel
 static int g_scores_variant = 0;           // test hook: 0 automatic, 1 FFMA epilogue, 2 score MMA in single CTAs, 3 CTA pairs
 static bool g_split_reduce_combine = false;   // test hook (variant 4): slab reduction and combine as two launches
-static int g_scores_stages = 0;            // tuning hook: cap on the TMA ring depth of the score-MMA kernels (0: as many slots as fit)
 
 // Launch the single-CTA score-MMA kernel (persistent: one CTA per SM, every head at least one).
 static int launch_scores_mma2(const ScoreParams& sp, int S, int H, cudaStream_t st) {
@@ -1485,10 +1459,6 @@ static int launch_scores_pair(ScoreParams& sp, int S, int H, cudaStream_t st) {
   int& resident = state();
   sp.stages = pair_stages_for(sp.nkb);
   if (sp.stages < 3) return -1;
-  if (g_scores_stages >= 3 && g_scores_stages < sp.stages) sp.stages = g_scores_stages;
-#ifdef XKV_PROBE
-  if (g_probe_stages > 0 && g_probe_stages < sp.stages) sp.stages = g_probe_stages;
-#endif
   cudaLaunchConfig_t cfg;
   std::memset(&cfg, 0, sizeof(cfg));
   cfg.blockDim = dim3(R_THREADS, 1, 1);
@@ -1561,10 +1531,6 @@ static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, i
   sp.nkb = (rk + DBK - 1) / DBK;
   sp.scale = scale;
   sp.stages = r_stages_for(sp.nkb);
-#ifdef XKV_PROBE
-  sp.dbg = g_probe_dbg;
-  if (g_probe_stages > 0 && g_probe_stages < sp.stages) sp.stages = g_probe_stages;
-#endif
   const int grid = ((S + DBM - 1) / DBM) * sp.tiles_n;
   static PerDevice<bool> configured;
   if (!configured()) {
@@ -1829,8 +1795,6 @@ extern "C" void xkv_decode_set_variant(int variant) {
   g_split_reduce_combine = variant == 4;
   g_scores_variant = variant == 4 ? 0 : variant;
 }
-/* tuning hook: cluster size of the score-MMA kernel (0 automatic) */
-extern "C" void xkv_decode_set_stages(int stages) { g_scores_stages = stages; }
 
 extern "C" int xkv_decode_attention(const void* q, int Hq, int H, int D, const void* A_k, int64_t lda_k, int rk,
                                     const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,

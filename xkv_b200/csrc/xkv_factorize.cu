@@ -35,11 +35,10 @@ struct Bump {
 
 struct Plan {
   int B, m, n, W, nw, sk, skw, gs;
-  int lmax;                    // widest sketch of the batch: leading dimension of every l x l matrix
   bool rr;
-  // per matrix: rank, sketch width l = round_up(rank + oversample, 64), Rayleigh-Ritz window [r0, r0 + W) with wl kept
-  // columns on its left of column r and wr = l - r discarded ones on its right
-  int r[XKV_MAX_BATCH], l[XKV_MAX_BATCH], wl[XKV_MAX_BATCH], wr[XKV_MAX_BATCH], r0[XKV_MAX_BATCH];
+  // rank r, sketch width l = round_up(r + oversample, 64), Rayleigh-Ritz window [r0, r0 + W) with wl kept columns on
+  // its left of column r and wr = l - r discarded ones on its right
+  int r, l, wl, wr, r0;
   // per-matrix buffers
   void* g_limb[XKV_MAX_BATCH][3];
   float* f_a[XKV_MAX_BATCH];
@@ -67,7 +66,7 @@ struct Plan {
   size_t bytes;
 };
 
-static int make_plan(Plan& P, Bump& bump, int B, int m, int n, const int* ranks, const xkv_factorize_options& o) {
+static int make_plan(Plan& P, Bump& bump, int B, int m, int n, int rank, const xkv_factorize_options& o) {
   XKV_REQUIRE(B >= 1 && B <= XKV_MAX_BATCH, "factorize: batch %d out of range (1..%d)", B, XKV_MAX_BATCH);
   XKV_REQUIRE(n % 8 == 0, "factorize: n=%d must be a multiple of 8", n);
   P.B = B;
@@ -77,59 +76,42 @@ static int make_plan(Plan& P, Bump& bump, int B, int m, int n, const int* ranks,
   const int nkb = (n + 63) / 64;
   P.sk = o.small_split_k < 1 ? 1 : (o.small_split_k > nkb ? nkb : o.small_split_k);
   P.skw = nkb < 16 ? nkb : 16;
-  P.lmax = 0;
-  int lmin = 1 << 30;
-  for (int b = 0; b < B; ++b) {
-    const int rank = ranks[b];
-    P.r[b] = rank;
-    P.l[b] = round_up_int(rank + o.oversample, 64);
-    XKV_REQUIRE(rank > 0 && rank <= m && P.l[b] <= n, "factorize: rank %d (sketch %d) does not fit a %d x %d matrix", rank,
-                P.l[b], m, n);
-    P.wr[b] = P.l[b] - rank;
-    if (P.l[b] > P.lmax) P.lmax = P.l[b];
-    if (P.l[b] < lmin) lmin = P.l[b];
-  }
-  // Rayleigh-Ritz window [r0, r0 + W) straddling column r: one width W for the whole batch (the Jacobi launch is
-  // uniform); matrix b keeps wl[b] = W - wr[b] columns of it
-  int W = o.window < lmin ? o.window : lmin;
+  P.r = rank;
+  P.l = round_up_int(rank + o.oversample, 64);
+  XKV_REQUIRE(rank > 0 && rank <= m && P.l <= n, "factorize: rank %d (sketch %d) does not fit a %d x %d matrix", rank, P.l, m,
+              n);
+  P.wr = P.l - rank;
+  // Rayleigh-Ritz window [r0, r0 + W) straddling column r: wl = W - wr columns of it are kept
+  int W = o.window < P.l ? o.window : P.l;
   if (W > 160) W = 160;
   W -= W % 2;
   P.rr = o.rayleigh_ritz != 0;
-  bool uniform = true;
-  int W0 = -1;
-  for (int b = 0; b < B; ++b) {
-    int wl = W - P.wr[b];
-    if (wl > P.r[b]) wl = P.r[b];
-    int Wb = wl + P.wr[b];
-    if (wl > 0 && (Wb % 2)) {
-      --wl;
-      --Wb;
-    }
-    if (wl <= 0) P.rr = false;
-    P.wl[b] = wl;
-    P.r0[b] = P.r[b] - wl;
-    if (W0 < 0) W0 = Wb;
-    if (Wb != W0) uniform = false;
+  int wl = W - P.wr;
+  if (wl > rank) wl = rank;
+  int Wb = wl + P.wr;
+  if (wl > 0 && (Wb % 2)) {
+    --wl;
+    --Wb;
   }
-  XKV_REQUIRE(!P.rr || uniform, "factorize: the ranks of one batch must give the same Rayleigh-Ritz window width");
-  P.W = P.rr ? W0 : W;
+  if (wl <= 0) P.rr = false;
+  P.wl = wl;
+  P.r0 = rank - wl;
+  P.W = P.rr ? Wb : W;
   P.nw = P.rr ? (o.want_sigma ? 2 : 1) : 0;
-  const size_t nn = n, lm = P.lmax;
+  const size_t nn = n, l = P.l;
   W = P.W;
   for (int b = 0; b < B; ++b) {
-    const size_t l = P.l[b];
     for (int i = 0; i < 3; ++i) P.g_limb[b][i] = bump.bf16(nn * nn);
     P.f_a[b] = bump.f32(l * nn);
     P.f_b[b] = bump.f32(l * nn);
     P.lh[b] = bump.bf16(l * nn);
     P.lm[b] = bump.bf16(l * nn);
     P.ll[b] = bump.bf16(l * nn);
-    // l x l matrices: leading dimension lmax for every matrix of the batch (the batched kernels take one)
-    P.s_slabs[b] = bump.f32(static_cast<size_t>(P.sk) * lm * lm);
-    P.s_mat[b] = bump.f32(lm * lm);
-    P.linv[b] = bump.f32(lm * lm);
-    P.rdiag[b] = bump.f32(lm);
-    for (int i = 0; i < 3; ++i) P.linv_l[b][i] = bump.bf16(lm * lm);
+    P.s_slabs[b] = bump.f32(static_cast<size_t>(P.sk) * l * l);
+    P.s_mat[b] = bump.f32(l * l);
+    P.linv[b] = bump.f32(l * l);
+    P.rdiag[b] = bump.f32(l);
+    for (int i = 0; i < 3; ++i) P.linv_l[b][i] = bump.bf16(l * l);
     for (int w = 0; w < P.nw; ++w) {
       P.yw[b][w] = bump.f32(static_cast<size_t>(W) * nn);
       for (int i = 0; i < 3; ++i) P.yw_l[b][w][i] = bump.bf16(static_cast<size_t>(W) * nn);
@@ -273,22 +255,7 @@ extern "C" size_t xkv_factorize_workspace_bytes(int batch, int m, int n, int ran
     xkv_factorize_default_options(&o);
   Plan P;
   Bump bump{nullptr, 0, 0, false};
-  int ranks[XKV_MAX_BATCH];
-  for (int b = 0; b < XKV_MAX_BATCH; ++b) ranks[b] = rank;
-  if (batch < 1 || batch > XKV_MAX_BATCH || make_plan(P, bump, batch, m, n, ranks, o)) return 0;
-  return P.bytes;
-}
-
-extern "C" size_t xkv_factorize_workspace_bytes_mixed(int batch, int m, int n, const int32_t* ranks_host,
-                                                      const xkv_factorize_options* opts) {
-  xkv_factorize_options o;
-  if (opts)
-    o = *opts;
-  else
-    xkv_factorize_default_options(&o);
-  Plan P;
-  Bump bump{nullptr, 0, 0, false};
-  if (!ranks_host || batch < 1 || batch > XKV_MAX_BATCH || make_plan(P, bump, batch, m, n, ranks_host, o)) return 0;
+  if (batch < 1 || batch > XKV_MAX_BATCH || make_plan(P, bump, batch, m, n, rank, o)) return 0;
   return P.bytes;
 }
 
@@ -301,13 +268,13 @@ extern "C" int xkv_factorize_sigma_count(int rank, const xkv_factorize_options* 
   Plan P;
   Bump bump{nullptr, 0, 0, false};
   // m, n large enough not to trip the fit check: only the window arithmetic matters here
-  if (make_plan(P, bump, 1, 1 << 20, 1 << 20, &rank, o)) return 0;
+  if (make_plan(P, bump, 1, 1 << 20, 1 << 20, rank, o)) return 0;
   return (P.rr && o.want_sigma) ? P.W : 0;
 }
 
 // X_host: packed matrices (layers == 0) or per-layer pointers [batch][layers] read in place
 static int factorize_impl(const void* const* X_host, int layers, int layer_cols, int batch, int m, int n, int64_t ldx,
-                          const int* ranks, const xkv_factorize_options* opts, void* const* A_host, void* const* Vt_host,
+                          int rank, const xkv_factorize_options* opts, void* const* A_host, void* const* Vt_host,
                           void* const* V_host, float* const* sigma_host, float* const* gram_host, int phase,
                           void* workspace, size_t workspace_bytes, void* const* stage_events_host, void* stream) {
   xkv_factorize_options o;
@@ -323,18 +290,12 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   XKV_REQUIRE(phase == 0 || phase == 4 || gram_host != nullptr, "factorize: phases 1 / 2 / 3 need the per-matrix Gram buffers");
   static thread_local Plan P;
   Bump bump{static_cast<char*>(workspace), 0, workspace_bytes, false};
-  XKV_REQUIRE(ranks != nullptr, "factorize: null ranks");
-  XKV_TRY(make_plan(P, bump, batch, m, n, ranks, o));
+  XKV_TRY(make_plan(P, bump, batch, m, n, rank, o));
   XKV_REQUIRE(!bump.overflow && P.bytes <= workspace_bytes, "factorize: workspace too small (%zu < %zu bytes)",
               workspace_bytes, P.bytes);
   XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "factorize: workspace must be 256-byte aligned");
-  const int B = batch, W = P.W, lmax = P.lmax;
-  const int* const l = P.l;     // per-matrix sketch widths
-  const int* const r = P.r;     // per-matrix ranks
+  const int B = batch, W = P.W, l = P.l, r = P.r;
   const long long nn = n;
-  bool mixed = false;
-  for (int b = 1; b < B; ++b) mixed = mixed || l[b] != l[0];
-  const int* const l_rows = mixed ? P.l : nullptr;   // per-matrix row counts of the batched small kernels (uniform: none)
   cudaStream_t st = as_stream(stream);
   int ev = 0;
   auto mark = [&]() -> int {
@@ -351,7 +312,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   auto project = [&]() -> int {
     for (int b = 0; b < B; ++b) {
       const void* x0 = layers > 0 ? X_host[static_cast<size_t>(b) * layers] : X_host[b];
-      xkv_gemm_problem p = problem(x0, nullptr, nullptr, ldx, 0, Vt_host[b], nullptr, nullptr, nn, 0, A_host[b], r[b], m, r[b], n, 1);
+      xkv_gemm_problem p = problem(x0, nullptr, nullptr, ldx, 0, Vt_host[b], nullptr, nullptr, nn, 0, A_host[b], r, m, r, n, 1);
       if (layers > 0) {
         p.a_layers = layers;
         p.layer_cols = layer_cols;
@@ -434,72 +395,54 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
       const int pp = ip + p0;  // index into the per-pass parameters (shift, limb terms)
       const bool cond = conditional_extra && ip == npass;
       if (cond) {
-        {
-          BatchRowsScope rows(l_rows);
-          XKV_TRY(xkv_pass_flags(P.linv, B, lmax, lmax, o.second_pass_min_pivot, P.pass_flags, stream));
-        }
+        XKV_TRY(xkv_pass_flags(P.linv, B, l, l, o.second_pass_min_pivot, P.pass_flags, stream));
         xkv_set_launch_predicate(P.pass_flags);
       }
       int rc = [&]() -> int {
-        {
-          BatchRowsScope rows(l_rows);
-          XKV_TRY(xkv_shift_normalize_rows(cur, (ip == 0 && shifted) ? nxt : nullptr, P.shift_dev,
-                                           track ? P.rdiag : nullptr, ip == 0, P.lh, P.lm, P.ll, B, lmax, n, nn, nn, stream));
-        }
+        XKV_TRY(xkv_shift_normalize_rows(cur, (ip == 0 && shifted) ? nxt : nullptr, P.shift_dev, track ? P.rdiag : nullptr,
+                                         ip == 0, P.lh, P.lm, P.ll, B, l, n, nn, nn, stream));
         // pass 0 is regularised by a 3e-4 shift; a 3-term product (error ~1e-5 per entry) is accurate enough there
         // only if those errors are incoherent -- see xkv_factorize_options.pass0_terms
         const int nt = (pp == 0 && o.pass0_terms == 3) ? 3 : 6;
         for (int b = 0; b < B; ++b) {
           xkv_gemm_problem p = problem(P.lh[b], P.lm[b], P.ll[b], nn, 0, P.lh[b], P.lm[b], P.ll[b], nn, 0, P.s_slabs[b],
-                                       lmax, l[b], l[b], n, nt);
+                                       l, l, l, n, nt);
           p.sym_upper = 1;
           p.split_k = P.sk;
-          p.split_stride = static_cast<long long>(lmax) * lmax;
+          p.split_stride = static_cast<long long>(l) * l;
           p.run_if = cond ? P.pass_flags + b : nullptr;
           ps.push_back(p);
         }
         XKV_TRY(run_gemms(ps, stream));
-        {
-          BatchRowsScope rows(l_rows);
-          XKV_TRY(xkv_reduce_slabs_batched(P.s_slabs, P.s_mat, B, P.sk, static_cast<long long>(lmax) * lmax, lmax, lmax, lmax, 1,
-                                           lmax, stream));
-        }
+        XKV_TRY(xkv_reduce_slabs_batched(P.s_slabs, P.s_mat, B, P.sk, static_cast<long long>(l) * l, l, l, l, 1, l, stream));
         {
           void *h0[XKV_MAX_BATCH], *h1[XKV_MAX_BATCH], *h2[XKV_MAX_BATCH];
           for (int b = 0; b < B; ++b) h0[b] = P.linv_l[b][0], h1[b] = P.linv_l[b][1], h2[b] = P.linv_l[b][2];
           const float shift = o.shifts[pp < 3 ? pp : 3];
-          {
-            BatchRowsScope rows(l_rows);
-            XKV_TRY(xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, nt > 3 ? h2 : nullptr, B, lmax, lmax, lmax, shift,
-                                               o.pivot_floor, stream));
-          }
+          XKV_TRY(xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, nt > 3 ? h2 : nullptr, B, l, l, l, shift, o.pivot_floor,
+                                             stream));
           if (o.heavy_redo && pp > 0 && shift < o.shifts[0]) {
             // A pivot below twice the shift means the fp32 Gram of the basis was numerically indefinite (the pass before
             // left it too ill-conditioned: extreme outlier channels).  Such matrices redo the Cholesky with the heavy
             // shift of pass 0 -- the slabs still hold S -- which costs orthogonality (later passes restore it) but never
             // produces the overflow -> NaN cascade of a clamped pivot.
-            BatchRowsScope rows(l_rows);
-            XKV_TRY(xkv_pass_flags(P.linv, B, lmax, lmax, 2.f * shift, P.redo_flags, stream));
+            XKV_TRY(xkv_pass_flags(P.linv, B, l, l, 2.f * shift, P.redo_flags, stream));
             xkv_set_launch_predicate(P.redo_flags);
-            int rc2 = xkv_reduce_slabs_batched(P.s_slabs, P.s_mat, B, P.sk, static_cast<long long>(lmax) * lmax, lmax, lmax, lmax,
-                                               1, lmax, stream);
+            int rc2 = xkv_reduce_slabs_batched(P.s_slabs, P.s_mat, B, P.sk, static_cast<long long>(l) * l, l, l, l, 1, l, stream);
             if (!rc2)
-              rc2 = xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, nt > 3 ? h2 : nullptr, B, lmax, lmax, lmax, o.shifts[0],
+              rc2 = xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, nt > 3 ? h2 : nullptr, B, l, l, l, o.shifts[0],
                                                o.pivot_floor, stream);
             xkv_set_launch_predicate(cond ? P.pass_flags : nullptr);
             if (rc2) return rc2;
           }
         }
-        if (track) {
-          BatchRowsScope rows(l_rows);
-          XKV_TRY(xkv_rdiag_update(P.rdiag, P.linv, B, lmax, lmax, stream));
-        }
+        if (track) XKV_TRY(xkv_rdiag_update(P.rdiag, P.linv, B, l, l, stream));
         // Q = Linv Y, computed as Q^T = Y^T Linv^T with the result stored transposed (same memory, same order of products):
         // the long dimension n becomes M, the sketch width l becomes N, which the CTA-pair GEMM tiles without padding
         // (l = 576 as 3 x 192 columns, 832 as 4 x 208)
         for (int b = 0; b < B; ++b) {
-          xkv_gemm_problem p = swap_roles(problem(P.linv_l[b][0], P.linv_l[b][1], P.linv_l[b][2], lmax, 0, P.lh[b], P.lm[b],
-                                                  P.ll[b], nn, 1, cond ? cur[b] : nxt[b], nn, l[b], n, l[b],
+          xkv_gemm_problem p = swap_roles(problem(P.linv_l[b][0], P.linv_l[b][1], P.linv_l[b][2], l, 0, P.lh[b], P.lm[b],
+                                                  P.ll[b], nn, 1, cond ? cur[b] : nxt[b], nn, l, n, l,
                                                   (o.solve_terms == 3 && !final_call) ? 3 : nt));
           p.run_if = cond ? P.pass_flags + b : nullptr;
           ps.push_back(p);
@@ -517,14 +460,14 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   auto apply_gram = [&](int nterms) -> int {
     for (int b = 0; b < B; ++b)   // as (G Q^T)^T: see swap_roles
       ps.push_back(swap_roles(problem(P.lh[b], P.lm[b], P.ll[b], nn, 0, P.g_limb[b][0], P.g_limb[b][1], P.g_limb[b][2], nn, 0,
-                                      nxt[b], nn, l[b], n, n, nterms)));
+                                      nxt[b], nn, l, n, n, nterms)));
     XKV_TRY(run_gemms(ps, stream));
     swap_bufs();
     return 0;
   };
 
   // ---- 2-3. Gaussian range finder ----
-  for (int b = 0; b < B; ++b) XKV_TRY(xkv_fill_gaussian_bf16(P.lh[b], l[b], n, nn, o.seed + 7919ull * b, stream));
+  for (int b = 0; b < B; ++b) XKV_TRY(xkv_fill_gaussian_bf16(P.lh[b], l, n, nn, o.seed + 7919ull * b, stream));
   XKV_TRY(apply_gram(1));
   XKV_TRY(cholqr(o.first_passes, false, false, 0, false, o.power_iters == 0));
   XKV_TRY(mark());  // 3: range finder
@@ -536,20 +479,11 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   if (use_shift) XKV_CHECK_CUDA(cudaMemsetAsync(P.shift_dev, 0, XKV_MAX_BATCH * sizeof(float), st));
   for (int it = 0; it < o.power_iters; ++it) {
     const int pterms = o.power_terms == 6 ? 6 : 3;
-    {
-      BatchRowsScope rows(l_rows);
-      XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, pterms == 6 ? P.ll : nullptr, B, lmax, n, nn, nn, stream));
-    }
+    XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, pterms == 6 ? P.ll : nullptr, B, l, n, nn, nn, stream));
     XKV_TRY(apply_gram(pterms));
     const bool shifted = use_shift && it > 0;
     if (shifted)
-    {
-      int lmin = l[0];
-      for (int b = 1; b < B; ++b) lmin = l[b] < lmin ? l[b] : lmin;
-      BatchRowsScope rows(l_rows);
-      XKV_TRY(xkv_ritz_shift_update(P.rdiag, B, lmax, o.shift_tail < lmin ? o.shift_tail : lmin, o.spectral_shift, P.shift_dev,
-                                    stream));
-    }
+      XKV_TRY(xkv_ritz_shift_update(P.rdiag, B, l, o.shift_tail < l ? o.shift_tail : l, o.spectral_shift, P.shift_dev, stream));
     // From step `single_pass_from` on the basis entering the step is orthonormal to ~1e-5 and ordered by dominance,
     // so the row-normalised product is well conditioned: ONE pass with the second pass's parameters (small shift,
     // 6-term Gram) orthonormalises it; the first, heavily shifted pass is only needed while the sketch is raw.
@@ -563,17 +497,13 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   // ---- 5. windowed Rayleigh-Ritz ----
   if (P.rr) {
     const int nw = P.nw;
-    const int* const r0 = P.r0;
-    const int* const wl = P.wl;
-    auto w0 = [&](int b, int w) { return w == 0 ? r0[b] : 0; };   // first basis row of window w of matrix b
-    {
-      BatchRowsScope rows(l_rows);
-      XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, P.ll, B, lmax, n, nn, nn, stream));
-    }
+    const int r0 = P.r0, wl = P.wl;
+    auto w0 = [&](int w) { return w == 0 ? r0 : 0; };   // first basis row of window w
+    XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, P.ll, B, l, n, nn, nn, stream));
     for (int b = 0; b < B; ++b)
       for (int w = 0; w < nw; ++w)
-        ps.push_back(swap_roles(problem(row_bf16(P.lh[b], w0(b, w), nn), row_bf16(P.lm[b], w0(b, w), nn),
-                                        row_bf16(P.ll[b], w0(b, w), nn), nn, 0, P.g_limb[b][0], P.g_limb[b][1], P.g_limb[b][2],
+        ps.push_back(swap_roles(problem(row_bf16(P.lh[b], w0(w), nn), row_bf16(P.lm[b], w0(w), nn),
+                                        row_bf16(P.ll[b], w0(w), nn), nn, 0, P.g_limb[b][0], P.g_limb[b][1], P.g_limb[b][2],
                                         nn, 0, P.yw[b][w], nn, W, n, n, 6)));   // as (G Qw^T)^T: M = n in CTA pairs, N = W
     XKV_TRY(run_gemms(ps, stream));
     {
@@ -595,7 +525,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
     for (int b = 0; b < B; ++b)
       for (int w = 0; w < nw; ++w) {
         xkv_gemm_problem p =
-            problem(row_bf16(P.lh[b], w0(b, w), nn), row_bf16(P.lm[b], w0(b, w), nn), row_bf16(P.ll[b], w0(b, w), nn), nn, 0,
+            problem(row_bf16(P.lh[b], w0(w), nn), row_bf16(P.lm[b], w0(w), nn), row_bf16(P.ll[b], w0(w), nn), nn, 0,
                     P.yw_l[b][w][0], P.yw_l[b][w][1], P.yw_l[b][w][2], nn, 0, P.t_slabs[b][w], W, W, W, n, 6);
         p.split_k = P.skw;
         p.split_stride = static_cast<long long>(W) * W;
@@ -630,20 +560,12 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
         xs[b] = P.wt[b];
         h0[b] = P.wsel_l[b][0], h1[b] = P.wsel_l[b][1], h2[b] = P.wsel_l[b][2];
       }
-      // the top wl[b] Ritz vectors of matrix b (wl differs with the sketch width: per-matrix row counts)
-      bool wl_mixed = false;
-      int wl_max = wl[0];
-      for (int b = 1; b < B; ++b) {
-        wl_mixed = wl_mixed || wl[b] != wl[0];
-        wl_max = wl[b] > wl_max ? wl[b] : wl_max;
-      }
-      BatchRowsScope rows(wl_mixed ? wl : nullptr);
-      XKV_TRY(xkv_split_bf16_batched(xs, h0, h1, h2, B, wl_max, W, W, W, stream));
+      XKV_TRY(xkv_split_bf16_batched(xs, h0, h1, h2, B, wl, W, W, W, stream));
     }
     for (int b = 0; b < B; ++b)
-      ps.push_back(problem(P.wsel_l[b][0], P.wsel_l[b][1], P.wsel_l[b][2], W, 0, row_bf16(P.lh[b], r0[b], nn),
-                           row_bf16(P.lm[b], r0[b], nn), row_bf16(P.ll[b], r0[b], nn), nn, 1,
-                           cur[b] + static_cast<size_t>(r0[b]) * nn, nn, wl[b], n, W, 6));
+      ps.push_back(problem(P.wsel_l[b][0], P.wsel_l[b][1], P.wsel_l[b][2], W, 0, row_bf16(P.lh[b], r0, nn),
+                           row_bf16(P.lm[b], r0, nn), row_bf16(P.ll[b], r0, nn), nn, 1,
+                           cur[b] + static_cast<size_t>(r0) * nn, nn, wl, n, W, 6));
     XKV_TRY(run_gemms(ps, stream));
     if (o.want_sigma && sigma_host)
       for (int b = 0; b < B; ++b)
@@ -652,15 +574,11 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   XKV_TRY(mark());  // 5: Rayleigh-Ritz
 
   // ---- 6. right factor in bf16, both layouts ----
-  for (int b = 0; b < B; ++b) XKV_TRY(xkv_convert_bf16(cur[b], r[b], n, nn, Vt_host[b], nn, V_host[b], r[b], stream));
+  for (int b = 0; b < B; ++b) XKV_TRY(xkv_convert_bf16(cur[b], r, n, nn, Vt_host[b], nn, V_host[b], r, stream));
   if (phase == 3) return 0;   // the caller projects later (phase 4), possibly on another rank's rows
   XKV_TRY(project());
   XKV_TRY(mark());  // 6: projection
   return 0;
-}
-
-static void uniform_ranks(int* ranks, int rank) {
-  for (int b = 0; b < XKV_MAX_BATCH; ++b) ranks[b] = rank;
 }
 
 extern "C" int xkv_factorize_batch(const void* const* X_host, int batch, int m, int n, int64_t ldx, int rank,
@@ -668,9 +586,7 @@ extern "C" int xkv_factorize_batch(const void* const* X_host, int batch, int m, 
                                    void* const* V_host, float* const* sigma_host, float* const* gram_host,
                                    int phase, void* workspace, size_t workspace_bytes,
                                    void* const* stage_events_host, void* stream) {
-  int ranks[XKV_MAX_BATCH];
-  uniform_ranks(ranks, rank);
-  return factorize_impl(X_host, 0, 0, batch, m, n, ldx, ranks, opts, A_host, Vt_host, V_host, sigma_host, gram_host, phase,
+  return factorize_impl(X_host, 0, 0, batch, m, n, ldx, rank, opts, A_host, Vt_host, V_host, sigma_host, gram_host, phase,
                         workspace, workspace_bytes, stage_events_host, stream);
 }
 
@@ -686,28 +602,6 @@ extern "C" int xkv_factorize_groups(const void* const* layer_ptrs_host, int batc
                                     void* const* Vt_host, void* const* V_host, float* const* sigma_host, void* workspace,
                                     size_t workspace_bytes, void* const* stage_events_host, void* stream) {
   XKV_TRY(check_layers(layers, layer_cols, ld_layer));
-  int ranks[XKV_MAX_BATCH];
-  uniform_ranks(ranks, rank);
-  return factorize_impl(layer_ptrs_host, layers, layer_cols, batch, m, layers * layer_cols, ld_layer, ranks, opts, A_host,
+  return factorize_impl(layer_ptrs_host, layers, layer_cols, batch, m, layers * layer_cols, ld_layer, rank, opts, A_host,
                         Vt_host, V_host, sigma_host, nullptr, 0, workspace, workspace_bytes, stage_events_host, stream);
-}
-
-extern "C" int xkv_factorize_groups_mixed(const void* const* layer_ptrs_host, int batch, int layers, int layer_cols, int m,
-                                          int64_t ld_layer, const int32_t* ranks_host, const xkv_factorize_options* opts,
-                                          void* const* A_host, void* const* Vt_host, void* const* V_host,
-                                          float* const* sigma_host, void* workspace, size_t workspace_bytes,
-                                          void* const* stage_events_host, void* stream) {
-  XKV_TRY(check_layers(layers, layer_cols, ld_layer));
-  XKV_REQUIRE(ranks_host != nullptr && batch >= 1 && batch <= XKV_MAX_BATCH, "factorize: bad batch / ranks");
-  return factorize_impl(layer_ptrs_host, layers, layer_cols, batch, m, layers * layer_cols, ld_layer, ranks_host, opts, A_host,
-                        Vt_host, V_host, sigma_host, nullptr, 0, workspace, workspace_bytes, stage_events_host, stream);
-}
-
-extern "C" int xkv_factorize_batch_mixed(const void* const* X_host, int batch, int m, int n, int64_t ldx,
-                                         const int32_t* ranks_host, const xkv_factorize_options* opts, void* const* A_host,
-                                         void* const* Vt_host, void* const* V_host, float* const* sigma_host, void* workspace,
-                                         size_t workspace_bytes, void* const* stage_events_host, void* stream) {
-  XKV_REQUIRE(ranks_host != nullptr && batch >= 1 && batch <= XKV_MAX_BATCH, "factorize: bad batch / ranks");
-  return factorize_impl(X_host, 0, 0, batch, m, n, ldx, ranks_host, opts, A_host, Vt_host, V_host, sigma_host, nullptr, 0,
-                        workspace, workspace_bytes, stage_events_host, stream);
 }

@@ -69,7 +69,7 @@ struct alignas(64) GemmProb {
 };
 struct GemmParams {
   int nprob;
-  int pair_stages;   // gemm_pair_kernel: ring depth
+  int pair_stages;   // gemm_pair_kernel: ring depth (PG_STAGES)
   GemmProb p[XKV_MAX_GEMM_PROBLEMS];
   CUtensorMap layer_maps[XKV_MAX_LAYER_MAPS];
 };
@@ -429,7 +429,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_kernel(const __grid_cons
 // CTA and are signalled by multicast commits; tmem_empty[2] lives in the even CTA and counts the epilogue warps of both.
 // ---------------------------------------------------------------------------------------------
 constexpr int PG_BM = 256;                              // pair tile rows (128 per CTA)
-constexpr int PG_STAGES = 6;                            // default ring depth (measured 5 / 6 / 7: see xkv_gemm_set_gram_pair)
+constexpr int PG_STAGES = 6;                            // ring depth (5 / 6 / 7 measured equal, 4 slower: DESIGN.md)
 constexpr int PG_MAX_STAGES = 7;
 constexpr int PG_A_BYTES = BM * BK * 2;                 // this CTA's 128 rows of A
 constexpr int PG_B_BYTES = (BN / 2) * BK * 2;           // this CTA's half of the tile's B rows (bn / 2 <= 128)
@@ -768,7 +768,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_pair_kernel(const __grid
 // ---------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------
-static int g_gram_pair = 1;   // xkv_gemm_set_gram_pair: 0 off, 1 default ring depth, 3 .. 7 that many stages
+static bool g_gram_pair = true;   // xkv_gemm_set_gram_pair
 
 // N tile of the problem in the pair kernel, 0 = the problem stays on single-CTA tiles.  Pairs are used where the 256-row
 // tile granularity costs nothing (M large, a multiple of 256, or its last 256 rows more than half used) and the operand
@@ -920,7 +920,7 @@ static int launch_pair_variant(GemmParams& params, int grid, cudaStream_t stream
                                         static_cast<int>(pg_smem_bytes(PG_MAX_STAGES))));
     configured() = true;
   }
-  params.pair_stages = (g_gram_pair >= 3 && g_gram_pair <= PG_MAX_STAGES) ? g_gram_pair : PG_STAGES;
+  params.pair_stages = PG_STAGES;
   for (int i = 0; i < params.nprob; ++i) {   // each problem cuts the launch's ring into stages of its own size
     const int stage = (params.p[i].na + params.p[i].nb) * PG_A_BYTES;
     const int st = params.pair_stages * PG_STAGE_BYTES / stage;
@@ -981,7 +981,7 @@ static int launch_variant(const GemmParams& params, int grid, cudaStream_t strea
 }  // namespace xkv
 
 extern "C" size_t xkv_gemm_problem_size(void) { return sizeof(xkv_gemm_problem); }
-extern "C" void xkv_gemm_set_gram_pair(int on) { xkv::g_gram_pair = on < 0 ? 0 : on; }
+extern "C" void xkv_gemm_set_gram_pair(int on) { xkv::g_gram_pair = on != 0; }
 
 extern "C" int xkv_gemm_grouped(const xkv_gemm_problem* problems, int num_problems, void* stream) {
   using namespace xkv;

@@ -22,17 +22,6 @@ extern std::atomic<long long> g_launch_count;
 // rdiag update): matrix b is skipped when flags[b] == 0.  nullptr (the default) = unconditional.
 const int*& launch_predicate();
 
-// Per-matrix row counts of the calling thread's next batched launches (normalise, limb split, square slab reduction,
-// Cholesky, rdiag / pass-flag / Ritz-shift updates): with a non-null HOST array rows[b] matrix b has rows[b] rows (and
-// columns, where the matrix is square) instead of the call's uniform `rows`, which then only sizes the grid (pass the
-// maximum).  Lets one launch carry matrices of different sketch widths (a group's K and V factorisations).  nullptr
-// (the default) = uniform.  Internal to the library: the factorisation driver sets and clears it around each call.
-const int*& batch_rows_override();
-struct BatchRowsScope {
-  explicit BatchRowsScope(const int* rows) { batch_rows_override() = rows; }
-  ~BatchRowsScope() { batch_rows_override() = nullptr; }
-};
-
 // Launch priority of the calling thread's next GEMM launches: true = the lowest CTA-level priority whatever the stream's.
 // The factorisation driver sets it around the projection A = X V, the last kernel of a chain (thousands of CTAs, nothing
 // waits for its first results): the SMs that free up go to the latency-bound kernels of the other chains first

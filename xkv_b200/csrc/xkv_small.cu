@@ -18,7 +18,6 @@ struct ReduceParams {
   const float* slabs[XKV_MAX_BATCH];
   float* out[XKV_MAX_BATCH];
   const int* run_if;   // optional per-matrix device predicate (xkv_set_launch_predicate)
-  int rows_b[XKV_MAX_BATCH];   // per-matrix size of a SQUARE matrix (0: the launch's uniform rows / cols)
 };
 template <int SYM>
 __global__ void __launch_bounds__(256) reduce_slabs_kernel(const __grid_constant__ ReduceParams rp, int num_slabs,
@@ -28,7 +27,6 @@ __global__ void __launch_bounds__(256) reduce_slabs_kernel(const __grid_constant
   if (rp.run_if != nullptr && rp.run_if[blockIdx.y] == 0) return;
   const float* __restrict__ slabs = rp.slabs[blockIdx.y];
   float* __restrict__ out = rp.out[blockIdx.y];
-  if (rp.rows_b[blockIdx.y] > 0) rows = cols = rp.rows_b[blockIdx.y];
   int bi, bj;
   if (SYM) {
     // linear index over tile pairs bi <= bj
@@ -136,11 +134,9 @@ struct SplitParams {
   __nv_bfloat16* hi[XKV_MAX_BATCH];
   __nv_bfloat16* mid[XKV_MAX_BATCH];
   __nv_bfloat16* lo[XKV_MAX_BATCH];
-  int rows_b[XKV_MAX_BATCH];   // per-matrix row count (0: the launch's uniform rows)
 };
 __global__ void __launch_bounds__(256) split_bf16_kernel(const __grid_constant__ SplitParams sp, int rows, int cols,
                                                          long long ld, long long ldo) {
-  if (sp.rows_b[blockIdx.y] > 0) rows = sp.rows_b[blockIdx.y];
   const float* __restrict__ x = sp.x[blockIdx.y];
   __nv_bfloat16* __restrict__ hi = sp.hi[blockIdx.y];
   __nv_bfloat16* __restrict__ mid = sp.mid[blockIdx.y];
@@ -298,7 +294,6 @@ struct NormParams {
   const float* Linv[XKV_MAX_BATCH];
   float* c;                        // per-matrix spectral shift (device), used when Q != null
   int rows, cols, tail, rdiag_first;
-  int rows_b[XKV_MAX_BATCH];       // per-matrix row count (0: the uniform `rows`)
   float shift_scale;
   long long ld, ldo, ld_linv;
   const int* run_if;               // optional per-matrix device predicate (xkv_set_launch_predicate)
@@ -317,9 +312,8 @@ struct NormParams {
 __global__ void __launch_bounds__(256) ritz_shift_kernel(const __grid_constant__ NormParams p) {
   __shared__ float red[8];
   const float* rd = p.rdiag[blockIdx.x];
-  const int rows = p.rows_b[blockIdx.x] > 0 ? p.rows_b[blockIdx.x] : p.rows;
   float acc = 0.f;
-  for (int j = rows - p.tail + threadIdx.x; j < rows; j += blockDim.x) acc += rd[j];
+  for (int j = p.rows - p.tail + threadIdx.x; j < p.rows; j += blockDim.x) acc += rd[j];
   acc = warp_sum(acc);
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
   __syncthreads();
@@ -335,8 +329,7 @@ __global__ void __launch_bounds__(256) rdiag_update_kernel(const __grid_constant
   float* rd = p.rdiag[blockIdx.y];
   const float* li = p.Linv[blockIdx.y];
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  const int rows = p.rows_b[blockIdx.y] > 0 ? p.rows_b[blockIdx.y] : p.rows;
-  if (j < rows) rd[j] = rd[j] / li[static_cast<long long>(j) * p.ld_linv + j];
+  if (j < p.rows) rd[j] = rd[j] / li[static_cast<long long>(j) * p.ld_linv + j];
 }
 
 // flags[b] = 1 when the Cholesky pass that just finished met a pivot L_jj^2 < min_pivot (S has a unit diagonal, so the
@@ -349,9 +342,8 @@ __global__ void __launch_bounds__(256) pass_flag_kernel(const __grid_constant__ 
     return;
   }
   const float* li = p.Linv[blockIdx.x];
-  const int rows = p.rows_b[blockIdx.x] > 0 ? p.rows_b[blockIdx.x] : p.rows;
   int bad = 0;
-  for (int j = threadIdx.x; j < rows; j += blockDim.x) {
+  for (int j = threadIdx.x; j < p.rows; j += blockDim.x) {
     const float d = li[static_cast<long long>(j) * p.ld_linv + j];   // 1 / L_jj
     if (!(d * d <= p.inv_min_pivot)) bad = 1;
   }
@@ -363,7 +355,6 @@ __global__ void __launch_bounds__(256) normalize_rows_kernel(const __grid_consta
   __shared__ float red[8];
   __shared__ float scale_s;
   if (p.run_if != nullptr && p.run_if[blockIdx.y] == 0) return;
-  if (p.rows_b[blockIdx.y] > 0 && static_cast<int>(blockIdx.x) >= p.rows_b[blockIdx.y]) return;   // uniform per CTA
   float* row = p.Y[blockIdx.y] + static_cast<long long>(blockIdx.x) * p.ld;
   const int cols4 = p.cols >> 2;
   float acc = 0.f;
@@ -580,20 +571,6 @@ const int*& launch_predicate() {
   static thread_local const int* pred = nullptr;
   return pred;
 }
-const int*& batch_rows_override() {
-  static thread_local const int* rows = nullptr;
-  return rows;
-}
-// fills dst[b] from the override (0 = uniform) and returns the grid-sizing row count
-static int take_batch_rows(int* dst, int batch, int uniform_rows) {
-  const int* ov = batch_rows_override();
-  int mx = uniform_rows;
-  for (int b = 0; b < XKV_MAX_BATCH; ++b) {
-    dst[b] = (ov != nullptr && b < batch) ? ov[b] : 0;
-    if (dst[b] > mx) mx = dst[b];
-  }
-  return mx;
-}
 
 }  // namespace xkv
 
@@ -609,7 +586,6 @@ extern "C" int xkv_pass_flags(const float* const* Linv_host, int batch, int rows
   std::memset(&p, 0, sizeof(p));
   for (int b = 0; b < batch; ++b) p.Linv[b] = Linv_host[b];
   p.rows = rows;
-  take_batch_rows(p.rows_b, batch, rows);
   p.ld_linv = ld_linv;
   p.flags = flags_dev;
   p.inv_min_pivot = 1.f / min_pivot;
@@ -631,10 +607,6 @@ extern "C" int xkv_reduce_slabs_batched(const float* const* slabs_host, float* c
     rp.slabs[b] = slabs_host[b];
     rp.out[b] = out_host[b];
   }
-  if (symmetrize)
-    rows = cols = take_batch_rows(rp.rows_b, batch, rows);
-  else
-    std::memset(rp.rows_b, 0, sizeof(rp.rows_b));
   rp.run_if = launch_predicate();
   const int tr = (rows + 31) / 32, tc = (cols + 31) / 32;
   if (symmetrize) {
@@ -712,7 +684,6 @@ extern "C" int xkv_split_bf16_batched(const float* const* x_host, void* const* h
     sp.mid[b] = mid_host ? static_cast<__nv_bfloat16*>(mid_host[b]) : nullptr;
     sp.lo[b] = lo_host ? static_cast<__nv_bfloat16*>(lo_host[b]) : nullptr;
   }
-  rows = take_batch_rows(sp.rows_b, batch, rows);
   const long long total = static_cast<long long>(rows) * (cols / 4);
   long long grid = (total + 255) / 256;
   const long long cap = static_cast<long long>(sm_count()) * 16 / batch + 1;
@@ -755,7 +726,6 @@ extern "C" int xkv_normalize_rows(float* const* Y_host, void* const* hi_host, vo
     p.lo[b] = lo_host ? static_cast<__nv_bfloat16*>(lo_host[b]) : nullptr;
   }
   p.rows = rows;
-  rows = take_batch_rows(p.rows_b, batch, rows);
   p.cols = cols;
   p.ld = ld;
   p.ldo = ld_out;
@@ -785,7 +755,6 @@ extern "C" int xkv_shift_normalize_rows(float* const* Y_host, const float* const
   }
   p.c = shift_dev;
   p.rows = rows;
-  rows = take_batch_rows(p.rows_b, batch, rows);
   p.cols = cols;
   p.rdiag_first = rdiag_first;
   p.ld = ld;
@@ -805,7 +774,6 @@ extern "C" int xkv_ritz_shift_update(float* const* rdiag_host, int batch, int ro
   for (int b = 0; b < batch; ++b) p.rdiag[b] = rdiag_host[b];
   p.c = shift_dev;
   p.rows = rows;
-  take_batch_rows(p.rows_b, batch, rows);
   p.tail = tail_rows;
   p.shift_scale = shift_scale;
   ritz_shift_kernel<<<batch, 256, 0, as_stream(stream)>>>(p);
@@ -823,7 +791,6 @@ extern "C" int xkv_rdiag_update(float* const* rdiag_host, const float* const* Li
     p.Linv[b] = Linv_host[b];
   }
   p.rows = rows;
-  rows = take_batch_rows(p.rows_b, batch, rows);
   p.ld_linv = ld_linv;
   p.run_if = launch_predicate();
   rdiag_update_kernel<<<dim3((rows + 255) / 256, batch), 256, 0, as_stream(stream)>>>(p);

@@ -142,90 +142,44 @@ def layer_rows(t: torch.Tensor) -> Optional[torch.Tensor]:
     return t.as_strided((s, h * d), (ss, 1))
 
 
-def mixed_ranks_ok(ranks: Sequence[int], opts: Optional[FactorizeOptions] = None) -> bool:
-    """Can matrices of these ranks share one driver call?  Their sketches must share a Rayleigh-Ritz window width: true when
-    every sketch is at least `window` wide and leaves room for at least one kept column in it."""
-    o = opts or FactorizeOptions()
-    ls = [sketch_width(int(r), o.oversample) for r in ranks]
-    w = min(o.window, 160) // 2 * 2
-    return all(l >= w and 0 < w - (l - int(r)) <= int(r) and (w - (l - int(r)) + (l - int(r))) % 2 == 0 for l, r in zip(ls, ranks))
-
-
-_STAGGER_MARK = 1   # stage mark of the driver the `gram_done` event is recorded at (1: behind the Gram launch)
-
-
-def factorize_groups(groups: Sequence[Sequence[torch.Tensor]], rank, opts: Optional[FactorizeOptions] = None,
-                     workspace: Optional[torch.Tensor] = None, extra_rows: int = 0,
-                     gram_done: Optional[torch.cuda.Event] = None) -> List[Factors]:
-    """Factorise layer groups IN PLACE: groups[g][i] is the (S, H*D) row-major matrix of layer i of group g
-    (:func:`layer_rows`); the group matrix is their column-wise concatenation — the reference's ``torch.cat(dim=1)`` +
-    ``transpose(1, 2).reshape`` (cache:170-171, :13-14) — and is never materialised: the Gram pass and the projection pass
-    read the layer tensors through per-layer tensor maps (xkv_factorize_groups).  `rank`: one rank for all, or one per group
-    matrix — a group's K and V matrices (different ranks, hence different sketch widths) then share every launch of the
-    latency-bound stages (xkv_factorize_groups_mixed).  `gram_done`: an event the driver records on the current stream
-    right behind the (last) Gram launch — what a concurrent chain on another stream waits for when the chains' Gram launches
-    are staggered (compress.compress_groups)."""
-    opts = opts or FactorizeOptions()
-    if len(groups) == 0:
-        return []
-    ranks = [int(rank)] * len(groups) if isinstance(rank, int) else [int(x) for x in rank]
-    if len(ranks) != len(groups):
-        raise XkvError("factorize_groups: one rank per group matrix required")
+def _factorize_chunks(items: Sequence, chunk: int, m: int, n: int, rank: int, opts: FactorizeOptions,
+                      workspace: Optional[torch.Tensor], extra_rows: int, dev, run) -> List[Factors]:
+    """What factorize_groups and factorize_batch share: sizes (and if needed allocates) the workspace for `chunk` matrices,
+    then per chunk of `items` allocates A (with `extra_rows` spare token rows behind it, for tokens appended later by
+    xkv_append_project), Vt, V and sigma, and makes the driver call ``run(part, co, outs, tail)`` — outs: the A / Vt / V /
+    sigma pointer arrays, tail: the workspace, its size, the stage events and the stream, in the C argument order.  With
+    `opts.profile` the 7 stage events of every call are recorded and their intervals summed into each Factors.timings."""
     lib = _lib.load()
-    nl = len(groups[0])
-    m, lc = groups[0][0].shape
-    ld = groups[0][0].stride(0)
-    dev = groups[0][0].device
-    for grp in groups:
-        if len(grp) != nl:
-            raise XkvError("factorize_groups: equally sized groups required")
-        for t in grp:
-            if (not t.is_cuda or t.dtype != torch.bfloat16 or tuple(t.shape) != (m, lc) or t.stride() != (ld, 1)
-                    or t.data_ptr() & 15):
-                raise XkvError("factorize_groups: layers must be equally shaped row-major bf16 CUDA matrices, 16-byte aligned")
-    n = nl * lc
     co = _c_options(opts)
-    per_call = max(1, min(_lib.MAX_BATCH, 64 // nl))     # XKV_MAX_LAYER_MAPS layer matrices per launch
-    chunk = min(len(groups), per_call)
-    need = 0
-    for lo in range(0, len(groups), chunk):
-        rk = (C.c_int32 * len(ranks[lo:lo + chunk]))(*ranks[lo:lo + chunk])
-        nb_ = int(lib.xkv_factorize_workspace_bytes_mixed(len(rk), m, n, rk, C.byref(co)))
-        if nb_ == 0:
-            raise XkvError(lib.xkv_last_error().decode() or "factorize: invalid problem")
-        need = max(need, nb_)
+    need = int(lib.xkv_factorize_workspace_bytes(chunk, m, n, rank, C.byref(co)))
+    if need == 0:
+        raise XkvError(lib.xkv_last_error().decode() or "factorize: invalid problem")
     if workspace is None or workspace.numel() * workspace.element_size() < need:
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
-    nsig = int(lib.xkv_factorize_sigma_count(ranks[0], C.byref(co)))
+    nsig = int(lib.xkv_factorize_sigma_count(rank, C.byref(co)))
     stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
     out: List[Factors] = []
     all_events = []
-    for lo in range(0, len(groups), chunk):
-        part = groups[lo:lo + chunk]
-        rs = ranks[lo:lo + chunk]
+    for lo in range(0, len(items), chunk):
+        part = items[lo:lo + chunk]
         nb = len(part)
-        a_store = [torch.empty(m + extra_rows, r, dtype=torch.bfloat16, device=dev) for r in rs]
+        a_store = [torch.empty(m + extra_rows, rank, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
         a = [t[:m] for t in a_store]
-        vt = [torch.empty(r, n, dtype=torch.bfloat16, device=dev) for r in rs]
-        v = [torch.empty(n, r, dtype=torch.bfloat16, device=dev) for r in rs]
+        vt = [torch.empty(rank, n, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
+        v = [torch.empty(n, rank, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
         sig = [torch.empty(nsig, dtype=torch.float32, device=dev) if nsig else None for _ in range(nb)]
         ev_arr = None
         if opts.profile:
             events = [torch.cuda.Event(enable_timing=True) for _ in range(7)]
             for e in events:
-                e.record()
+                e.record()  # torch creates the cudaEvent lazily; recording materialises the handle
             ev_arr = (C.c_void_p * 7)(*[e.cuda_event for e in events])
             all_events.append(events)
-        elif gram_done is not None and lo + chunk >= len(groups):
-            gram_done.record()   # materialises the handle; the driver records it again behind the Gram launch (stage mark 1)
-            ev_arr = (C.c_void_p * 7)(*[gram_done.cuda_event if i == _STAGGER_MARK else None for i in range(7)])
-        flat = [t for grp in part for t in grp]
-        _lib.check(lib.xkv_factorize_groups_mixed(
-            ops._ptr_array(flat), nb, nl, lc, m, ld, (C.c_int32 * nb)(*rs), C.byref(co), ops._ptr_array(a),
-            ops._ptr_array(vt), ops._ptr_array(v), ops._ptr_array(sig) if nsig else None,
-            C.c_void_p(workspace.data_ptr()), workspace.numel() * workspace.element_size(), ev_arr, stream))
+        outs = (ops._ptr_array(a), ops._ptr_array(vt), ops._ptr_array(v), ops._ptr_array(sig) if nsig else None)
+        tail = (C.c_void_p(workspace.data_ptr()), workspace.numel() * workspace.element_size(), ev_arr, stream)
+        run(part, co, outs, tail)
         for b in range(nb):
-            out.append(Factors(A=a[b], Vt=vt[b], V=v[b], rank=rs[b], sigma_lead=sig[b], A_storage=a_store[b]))
+            out.append(Factors(A=a[b], Vt=vt[b], V=v[b], rank=rank, sigma_lead=sig[b], A_storage=a_store[b]))
     if opts.profile:
         torch.cuda.synchronize()
         timings: Dict[str, float] = {}
@@ -235,6 +189,37 @@ def factorize_groups(groups: Sequence[Sequence[torch.Tensor]], rank, opts: Optio
         for f in out:
             f.timings = timings
     return out
+
+
+def factorize_groups(groups: Sequence[Sequence[torch.Tensor]], rank: int, opts: Optional[FactorizeOptions] = None,
+                     workspace: Optional[torch.Tensor] = None, extra_rows: int = 0) -> List[Factors]:
+    """Factorise layer groups IN PLACE at rank `rank`: groups[g][i] is the (S, H*D) row-major matrix of layer i of group g
+    (:func:`layer_rows`); the group matrix is their column-wise concatenation — the reference's ``torch.cat(dim=1)`` +
+    ``transpose(1, 2).reshape`` (cache:170-171, :13-14) — and is never materialised: the Gram pass and the projection pass
+    read the layer tensors through per-layer tensor maps (xkv_factorize_groups)."""
+    opts = opts or FactorizeOptions()
+    if len(groups) == 0:
+        return []
+    lib = _lib.load()
+    nl = len(groups[0])
+    m, lc = groups[0][0].shape
+    ld = groups[0][0].stride(0)
+    for grp in groups:
+        if len(grp) != nl:
+            raise XkvError("factorize_groups: equally sized groups required")
+        for t in grp:
+            if (not t.is_cuda or t.dtype != torch.bfloat16 or tuple(t.shape) != (m, lc) or t.stride() != (ld, 1)
+                    or t.data_ptr() & 15):
+                raise XkvError("factorize_groups: layers must be equally shaped row-major bf16 CUDA matrices, 16-byte aligned")
+    r = int(rank)
+    per_call = max(1, min(_lib.MAX_BATCH, 64 // nl))     # XKV_MAX_LAYER_MAPS layer matrices per launch
+
+    def run(part, co, outs, tail):
+        flat = [t for grp in part for t in grp]
+        _lib.check(lib.xkv_factorize_groups(ops._ptr_array(flat), len(part), nl, lc, m, ld, r, C.byref(co), *outs, *tail))
+
+    return _factorize_chunks(groups, min(len(groups), per_call), m, nl * lc, r, opts, workspace, extra_rows,
+                             groups[0][0].device, run)
 
 
 def factorize_batch(xs: Sequence[torch.Tensor], rank: int, opts: Optional[FactorizeOptions] = None,
@@ -261,73 +246,38 @@ def factorize_batch(xs: Sequence[torch.Tensor], rank: int, opts: Optional[Factor
         if x.dtype != torch.bfloat16 or tuple(x.shape) != (m, n) or x.stride(1) != 1 or x.stride(0) != xs[0].stride(0):
             raise XkvError("factorize: inputs must be equally-shaped row-major bf16 matrices")
     r = int(rank)
-    co = _c_options(opts)
-    chunk = min(len(xs), _lib.MAX_BATCH)
-    need = int(lib.xkv_factorize_workspace_bytes(chunk, m, n, r, C.byref(co)))
-    if need == 0:
-        raise XkvError(lib.xkv_last_error().decode() or "factorize: invalid problem")
-    if workspace is None or workspace.numel() * workspace.element_size() < need:
-        workspace = torch.empty(need, dtype=torch.uint8, device=dev)
-    nsig = int(lib.xkv_factorize_sigma_count(r, C.byref(co)))
-    out: List[Factors] = []
-    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
-    all_events = []
-    for lo in range(0, len(xs), chunk):
-        part = xs[lo:lo + chunk]
+
+    def run(part, co, outs, tail):
         nb = len(part)
-        # `extra_rows` spare token rows behind A (for tokens appended later by xkv_append_project)
-        a_store = [torch.empty(m + extra_rows, r, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
-        a = [t[:m] for t in a_store]
-        vt = [torch.empty(r, n, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
-        v = [torch.empty(n, r, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
-        sig = [torch.empty(nsig, dtype=torch.float32, device=dev) if nsig else None for _ in range(nb)]
-        events = [torch.cuda.Event(enable_timing=True) for _ in range(7)] if opts.profile else None
-        ev_arr = None
-        if events is not None:
-            for e in events:
-                e.record()  # torch creates the cudaEvent lazily; recording materialises the handle
-            ev_arr = (C.c_void_p * 7)(*[e.cuda_event for e in events])
-            all_events.append(events)
+
         def call(phase, grams):
-            _lib.check(lib.xkv_factorize_batch(
-                ops._ptr_array(part), nb, m, n, part[0].stride(0), r, C.byref(co), ops._ptr_array(a),
-                ops._ptr_array(vt), ops._ptr_array(v), ops._ptr_array(sig) if nsig else None,
-                ops._ptr_array(grams) if grams is not None else None, phase, C.c_void_p(workspace.data_ptr()),
-                workspace.numel() * workspace.element_size(), ev_arr, stream))
+            _lib.check(lib.xkv_factorize_batch(ops._ptr_array(part), nb, m, n, part[0].stride(0), r, C.byref(co), *outs,
+                                               ops._ptr_array(grams) if grams is not None else None, phase, *tail))
 
         if process_group is None:
             call(0, None)
-        else:
-            import torch.distributed as dist
+            return
+        import torch.distributed as dist
 
-            # the only data-path collective: all-reduce(sum) of the local Gram matrices, upper triangles only
-            # (n^2 / 2 + 16 n floats per matrix instead of n^2: the Gram is symmetric)
-            grams = torch.empty(nb, n, n, dtype=torch.float32, device=dev)
-            call(1, list(grams))
-            per = ops.gram_packed_elems(n)
-            packed = torch.empty(nb, per, dtype=torch.float32, device=dev)
-            for b in range(nb):
-                ops.gram_pack_upper(grams[b], packed[b])
-            if comm_events is not None:
-                comm_events[0].record()
-            dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=process_group)
-            if comm_events is not None:
-                comm_events[1].record()
-                comm_events.append(packed.numel() * packed.element_size())
-            for b in range(nb):
-                ops.gram_unpack_upper(packed[b], grams[b])
-            call(2, list(grams))
+        # the only data-path collective: all-reduce(sum) of the local Gram matrices, upper triangles only
+        # (n^2 / 2 + 16 n floats per matrix instead of n^2: the Gram is symmetric)
+        grams = torch.empty(nb, n, n, dtype=torch.float32, device=dev)
+        call(1, list(grams))
+        per = ops.gram_packed_elems(n)
+        packed = torch.empty(nb, per, dtype=torch.float32, device=dev)
         for b in range(nb):
-            out.append(Factors(A=a[b], Vt=vt[b], V=v[b], rank=r, sigma_lead=sig[b], A_storage=a_store[b]))
-    if opts.profile:
-        torch.cuda.synchronize()
-        timings: Dict[str, float] = {}
-        for events in all_events:
-            for i, name in enumerate(_STAGES):
-                timings[name] = timings.get(name, 0.0) + events[i].elapsed_time(events[i + 1])
-        for f in out:
-            f.timings = timings
-    return out
+            ops.gram_pack_upper(grams[b], packed[b])
+        if comm_events is not None:
+            comm_events[0].record()
+        dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=process_group)
+        if comm_events is not None:
+            comm_events[1].record()
+            comm_events.append(packed.numel() * packed.element_size())
+        for b in range(nb):
+            ops.gram_unpack_upper(packed[b], grams[b])
+        call(2, list(grams))
+
+    return _factorize_chunks(xs, min(len(xs), _lib.MAX_BATCH), m, n, r, opts, workspace, extra_rows, dev, run)
 
 
 _chain_streams = {}
