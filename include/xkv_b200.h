@@ -278,6 +278,20 @@ XKV_API int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, const 
                                      int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
                                      int64_t tail_stride_t, float scale, void* out, void* workspace,
                                      size_t workspace_bytes, void* stream, float* lse_out);
+/* Multi-token step (speculative verification, a continuation chunk): Tq query tokens per q head in one call.
+ *   q, out     (Hq*Tq, D) bf16, row hq*Tq + t = query token t of q head hq (HF's query[0] (Hq, Tq, D) made contiguous)
+ *   k_tail, v_tail  (H, T, D): the LAST Tq tail tokens are the queries' own (T >= Tq); query token t sees the whole
+ *              compressed prefix and tail tokens [0, T - Tq + t] (causal among the new tokens)
+ *   lse_out    Hq*Tq floats (may be NULL), one per row
+ * Bounds: (Hq/H)*Tq <= 64 and Hq*Tq <= 512 (XKV_ERR otherwise: callers take a dense path).  Workspace:
+ * xkv_decode_workspace_bytes(Hq*Tq, S, T, rv).  Four launches whatever Tq is; the prefix keys are rebuilt once per call on
+ * the head_dim 128 path (CTA pairs), once per 8 rows of a kv head on the others.  Tq = 1 is xkv_decode_attention_lse. */
+XKV_API int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                                       const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,
+                                       const void* Vv_layer, int64_t ldv_v, int S, const void* cos, const void* sin,
+                                       int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
+                                       int64_t tail_stride_t, float scale, void* out, void* workspace,
+                                       size_t workspace_bytes, void* stream, float* lse_out);
 /* test hook: 1 forces the tile-per-CTA scores kernel (otherwise chosen only when one head's slice of the right
  * factor exceeds 128 KiB of shared memory), 0 restores the automatic choice */
 XKV_API void xkv_decode_force_tiled(int on);

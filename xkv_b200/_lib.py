@@ -132,6 +132,8 @@ SIGNATURES = {
                                   _vp, _vp, _i, _i64, _i64, _f, _vp, _vp, _sz, _vp]),
     "xkv_decode_attention_lse": (_i, [_vp, _i, _i, _i, _vp, _i64, _i, _vp, _i64, _vp, _i64, _i, _vp, _i64, _i, _vp, _vp,
                                       _i64, _vp, _vp, _i, _i64, _i64, _f, _vp, _vp, _sz, _vp, _vp]),
+    "xkv_decode_attention_multi": (_i, [_vp, _i, _i, _i, _i, _vp, _i64, _i, _vp, _i64, _vp, _i64, _i, _vp, _i64, _i, _vp,
+                                        _vp, _i64, _vp, _vp, _i, _i64, _i64, _f, _vp, _vp, _sz, _vp, _vp]),
     "xkv_decode_absorbed_workspace_bytes": (_sz, [_i, _i, _i]),
     "xkv_decode_absorbed": (_i, [_vp, _i, _vp, _i64, _i, _i, _vp, _vp, _vp, _i64, _i, _f, _vp, _vp, _vp, _sz, _vp]),
     "xkv_decode_force_tiled": (None, [_i]),

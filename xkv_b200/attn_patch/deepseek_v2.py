@@ -35,7 +35,7 @@ from transformers.cache_utils import Cache
 from transformers.modeling_utils import ALL_ATTENTION_FUNCTIONS
 from transformers.models.deepseek_v2.modeling_deepseek_v2 import DeepseekV2Attention, apply_rotary_emb
 
-from ..customized_cache.fake_layer_merge_dynamic_cache import FakeLayerMergingCache
+from ..customized_cache.fake_layer_merge_dynamic_cache import FakeLayerMergingCache, is_prefill_step
 
 
 def xKV_mla_forward(  # noqa: N802
@@ -49,7 +49,9 @@ def xKV_mla_forward(  # noqa: N802
 ):
     cache = past_key_values if past_key_values is not None else past_key_value
     bsz, q_len = hidden_states.shape[:-1]
-    is_prefill = q_len > 1  # auto-regressive use, as in the reference
+    # the first forward of a layer; later multi-token forwards are decode steps and take the dense path below
+    # (latent_slot declines q_len > 1)
+    is_prefill = is_prefill_step(cache, self.layer_idx, q_len)
 
     if self.q_lora_rank is None:
         q = self.q_proj(hidden_states)

@@ -2,13 +2,17 @@
 
 Semantics kept from the reference:
 * RoPE is applied to Q only before the cache is touched (llama.py:39-40);
-* prefill (q_len > 1) hands the PRE-RoPE keys plus cos/sin to ``cache.update(..., mode='prefill')`` and then
+* prefill hands the PRE-RoPE keys plus cos/sin to ``cache.update(..., mode='prefill')`` and then
   attends on the ORIGINAL keys/values (llama.py:45-50) — compression only affects later decode steps;
-* decode appends the post-RoPE key (llama.py:51-53) and attends over the cache;
+* decode appends the post-RoPE keys (llama.py:51-53) and attends over the cache;
 * only the sdpa attention implementation is accepted (llama.py:55-56);
 * a sliding-window layer whose context exceeds the window attends through SDPA with transformers' mask
   (mistral.py:69): the fused kernel has no window, so it is bypassed there.
-What differs: the decode step calls ``cache.attend`` — the fused reconstruct + RoPE + GQA-softmax kernel over
+What differs: the reference calls every q_len > 1 forward a prefill; here only the first forward of a layer is
+(``is_prefill_step``: several tokens, empty layer).  A later multi-token forward (assisted decoding verifying a
+draft, a second chunk of a prompt) is a decode step of q_len tokens, causal among themselves: the fused kernel takes
+it within its bounds, past them ``cache.attend`` declines and the dense path runs with transformers' causal mask.
+Also: the decode step calls ``cache.attend`` — the fused reconstruct + RoPE + GQA-softmax kernel over
 the stored factors — instead of SDPA over dense reconstructed tensors.  Written against the installed
 transformers (``past_key_values`` kwarg; the reference's ``past_key_value`` spelling is accepted too).
 """
@@ -22,7 +26,7 @@ from transformers.cache_utils import Cache
 from transformers.modeling_utils import ALL_ATTENTION_FUNCTIONS
 from transformers.models.llama.modeling_llama import LlamaAttention, apply_rotary_pos_emb
 
-from ..customized_cache.fake_layer_merge_dynamic_cache import FakeLayerMergingCache
+from ..customized_cache.fake_layer_merge_dynamic_cache import FakeLayerMergingCache, is_prefill_step
 
 
 def _heads(proj, hidden_states: torch.Tensor, head_dim: int) -> torch.Tensor:
@@ -60,7 +64,7 @@ def xKV_llama_forward(  # noqa: N802
     v = _heads(self.v_proj, hidden_states, self.head_dim)
     k = _rope(k_pre, cos, sin)
 
-    if cache is not None and hidden_states.shape[1] > 1:
+    if cache is not None and is_prefill_step(cache, self.layer_idx, hidden_states.shape[1]):
         # prefill: the cache gets the pre-RoPE keys and the tables; attention below runs on the ORIGINAL K / V
         assert isinstance(cache, FakeLayerMergingCache)
         cache.update(k_pre, v, self.layer_idx, mode="prefill", cos=cos, sin=sin, return_dense=False)

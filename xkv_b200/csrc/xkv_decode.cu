@@ -38,20 +38,26 @@ struct alignas(64) ScoreParams {
   CUtensorMap a_map;  // A_k  (S x r_k), box {64, 128}
   CUtensorMap b_map;  // Bk_l (H*D x r_k), box {64, 256}
   CUtensorMap b_head_map;  // Bk_l, box {64, D}: one kv head (persistent kernel)
-  CUtensorMap q_map;       // q (Hq x D), box {64, 16}: the q rows of one kv head (score MMA)
+  CUtensorMap q_map;       // q (rows x D), box {64, 16}: the q rows of one pass of a kv head (score MMA)
   CUtensorMap b_half_map;  // Bk_l, box {64, 64}: half a kv head's dims (pair kernel)
-  CUtensorMap q_half_map;  // q, box {64, 8}: the q rows one CTA of a pair supplies to the score MMA
-  const __nv_bfloat16* q;    // (Hq, D)
+  CUtensorMap q_half_map;  // q, box {64, nq16 / 2}: the q rows one CTA of a pair supplies to the score MMA
+  const __nv_bfloat16* q;    // (rows, D): row r = hq * Tq + t, query token t of q head hq
   const __nv_bfloat16* cos;  // (S, D) or null
   const __nv_bfloat16* sin;
-  float* scores;             // (Hq, ld_scores)
+  float* scores;             // (rows, ld_scores)
   long long ld_cs, ld_scores;
-  int S, rk, H, qpk, tiles_n, nkb;
+  // qpk: q rows per kv head (q heads per kv head x query tokens), contiguous from h * qpk.  The kernels other than the
+  // pair kernel take at most D_MAX_QPK of them per CTA: kv head h is worked in npass passes of <= 8 rows (pass_rows).
+  int S, rk, H, qpk, tiles_n, nkb, npass;
   int stages;   // ring slots of the score-MMA kernel
   float scale;
 };
 
 __device__ __forceinline__ float bf16r(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
+
+// first q row and row count of pass p of kv head h (npass == 1, the single-token case: rows h * qpk, qpk of them)
+__device__ __forceinline__ int pass_row0(const ScoreParams& P, int h, int p) { return h * P.qpk + p * D_MAX_QPK; }
+__device__ __forceinline__ int pass_rows(const ScoreParams& P, int p) { return min(D_MAX_QPK, P.qpk - p * D_MAX_QPK); }
 
 template <int D>
 __global__ void __launch_bounds__(D_THREADS, 2) decode_scores_kernel(const __grid_constant__ ScoreParams P) {
@@ -69,6 +75,7 @@ __global__ void __launch_bounds__(D_THREADS, 2) decode_scores_kernel(const __gri
   const int tm = blockIdx.x / P.tiles_n, tn = blockIdx.x - tm * P.tiles_n;
   const int m0 = tm * DBM, n0 = tn * DBN;
   const int h0 = n0 / D;  // first kv head of this tile
+  const int pass = blockIdx.y, nrow = pass_rows(P, pass);
 
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < DSTAGES; ++i) {
@@ -82,13 +89,13 @@ __global__ void __launch_bounds__(D_THREADS, 2) decode_scores_kernel(const __gri
   }
   if (warp == 1) tmem_alloc(tmem_slot, D_TMEM_COLS);
   if (warp >= 2) {
-    // stage this tile's query heads as fp32: q_s[(hh * qpk + g) * D + d]
-    const int nq = HPT * P.qpk * D;
+    // stage this tile's q rows of this pass as fp32: q_s[(hh * nrow + g) * D + d]
+    const int nq = HPT * nrow * D;
     for (int e = threadIdx.x - 64; e < nq; e += 128) {
       const int d = e % D, hg = e / D;
-      const int hh = hg / P.qpk, g = hg - hh * P.qpk;
+      const int hh = hg / nrow, g = hg - hh * nrow;
       const int h = h0 + hh;
-      q_s[e] = (h < P.H) ? __bfloat162float(P.q[static_cast<long long>(h * P.qpk + g) * D + d]) : 0.f;
+      q_s[e] = (h < P.H) ? __bfloat162float(P.q[static_cast<long long>(pass_row0(P, h, pass) + g) * D + d]) : 0.f;
     }
   }
   tc_fence_before();
@@ -176,7 +183,7 @@ __global__ void __launch_bounds__(D_THREADS, 2) decode_scores_kernel(const __gri
         tmem_ld_32x32(lane_addr + static_cast<uint32_t>(hh * D + c * 32), x1);
         tmem_ld_32x32(lane_addr + static_cast<uint32_t>(hh * D + (c + NCH / 2) * 32), x2);
         tmem_ld_wait();
-        const float* qh = q_s + (hh * P.qpk) * D;
+        const float* qh = q_s + (hh * nrow) * D;
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const float k1 = bf16r(__uint_as_float(x1[j]));
@@ -193,7 +200,7 @@ __global__ void __launch_bounds__(D_THREADS, 2) decode_scores_kernel(const __gri
           const int d1 = c * 32 + j, d2 = d1 + D / 2;
 #pragma unroll
           for (int g = 0; g < D_MAX_QPK; ++g)
-            if (g < P.qpk) acc[hh][g] = fmaf(qh[g * D + d1], o1, fmaf(qh[g * D + d2], o2, acc[hh][g]));
+            if (g < nrow) acc[hh][g] = fmaf(qh[g * D + d1], o1, fmaf(qh[g * D + d2], o2, acc[hh][g]));
         }
       }
     }
@@ -204,7 +211,7 @@ __global__ void __launch_bounds__(D_THREADS, 2) decode_scores_kernel(const __gri
         if (h < P.H) {
 #pragma unroll
           for (int g = 0; g < D_MAX_QPK; ++g)
-            if (g < P.qpk) P.scores[static_cast<long long>(h * P.qpk + g) * P.ld_scores + tok] = acc[hh][g] * P.scale;
+            if (g < nrow) P.scores[static_cast<long long>(pass_row0(P, h, pass) + g) * P.ld_scores + tok] = acc[hh][g] * P.scale;
         }
       }
     }
@@ -250,9 +257,13 @@ __global__ void __launch_bounds__(P_THREADS, 1) decode_scores_persistent_kernel(
   float* part = q_s + 128 * D_MAX_QPK;                                      // [2][128 tokens][8] partial scores
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int h = blockIdx.x % P.H;
-  const int slot = blockIdx.x / P.H;
-  const int nslots = (gridDim.x - h + P.H - 1) / P.H;   // CTAs that share this head
+  // CTA -> (kv head h, pass) of one of the H * npass row sets, and the token tiles slot, slot + nslots, ...
+  const int nv = P.H * P.npass;
+  const int vh = blockIdx.x % nv;
+  const int h = vh / P.npass, pass = vh - h * P.npass;
+  const int row0 = pass_row0(P, h, pass), nrow = pass_rows(P, pass);
+  const int slot = blockIdx.x / nv;
+  const int nslots = (gridDim.x - vh + nv - 1) / nv;   // CTAs that share this row set
   const int ntiles = (P.S + DBM - 1) / DBM;
 
   if (warp == 0 && lane == 0) {
@@ -273,7 +284,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) decode_scores_persistent_kernel(
   if (warp >= 2) {
     for (int e = threadIdx.x - 64; e < D * D_MAX_QPK; e += 32 * P_EPI_WARPS) {
       const int d = e / D_MAX_QPK, g = e - d * D_MAX_QPK;
-      q_s[e] = g < P.qpk ? __bfloat162float(P.q[static_cast<long long>(h * P.qpk + g) * D + d]) : 0.f;
+      q_s[e] = g < nrow ? __bfloat162float(P.q[static_cast<long long>(row0 + g) * D + d]) : 0.f;
     }
   }
   tc_fence_before();
@@ -417,7 +428,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) decode_scores_persistent_kernel(
           const float4 qb = *reinterpret_cast<const float4*>(q_s + d2 * D_MAX_QPK);
           sc01 = __ffma2_rn(make_float2(qa.x, qa.y), a, __ffma2_rn(make_float2(qb.x, qb.y), b, sc01));
           sc23 = __ffma2_rn(make_float2(qa.z, qa.w), a, __ffma2_rn(make_float2(qb.z, qb.w), b, sc23));
-          if (P.qpk > 4) {
+          if (nrow > 4) {
             const float4 qc = *reinterpret_cast<const float4*>(q_s + d1 * D_MAX_QPK + 4);
             const float4 qe = *reinterpret_cast<const float4*>(q_s + d2 * D_MAX_QPK + 4);
             sc45 = __ffma2_rn(make_float2(qc.x, qc.y), a, __ffma2_rn(make_float2(qe.x, qe.y), b, sc45));
@@ -430,7 +441,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) decode_scores_persistent_kernel(
       if (prt > 0) {
         float* pt = part + (((prt - 1) * 2 + pb) * DBM + row) * D_MAX_QPK;
         *reinterpret_cast<float4*>(pt) = make_float4(sc[0], sc[1], sc[2], sc[3]);
-        if (P.qpk > 4) *reinterpret_cast<float4*>(pt + 4) = make_float4(sc[4], sc[5], sc[6], sc[7]);
+        if (nrow > 4) *reinterpret_cast<float4*>(pt + 4) = make_float4(sc[4], sc[5], sc[6], sc[7]);
       }
       asm volatile("bar.sync 1, %0;" ::"n"(32 * P_EPI_WARPS) : "memory");   // epilogue warps only
       if (prt == 0 && tok_ok) {
@@ -442,14 +453,14 @@ __global__ void __launch_bounds__(P_THREADS, 1) decode_scores_persistent_kernel(
           const float* pt = part + ((o * 2 + pb) * DBM + row) * D_MAX_QPK;
           const float4 lo4 = *reinterpret_cast<const float4*>(pt);
           tot[0] += lo4.x, tot[1] += lo4.y, tot[2] += lo4.z, tot[3] += lo4.w;
-          if (P.qpk > 4) {
+          if (nrow > 4) {
             const float4 hi4 = *reinterpret_cast<const float4*>(pt + 4);
             tot[4] += hi4.x, tot[5] += hi4.y, tot[6] += hi4.z, tot[7] += hi4.w;
           }
         }
 #pragma unroll
         for (int g = 0; g < D_MAX_QPK; ++g)
-          if (g < P.qpk) P.scores[static_cast<long long>(h * P.qpk + g) * P.ld_scores + tok] = tot[g] * P.scale;
+          if (g < nrow) P.scores[static_cast<long long>(row0 + g) * P.ld_scores + tok] = tot[g] * P.scale;
       }
       acc = (acc + 1) % P_NACC;
       pb ^= 1;
@@ -520,11 +531,15 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // CTA `cid` works on kv head h and on the token tiles slot, slot + nslots, ...
+  // (kv head, pass) as in decode_scores_persistent_kernel
   const int cid = static_cast<int>(blockIdx.x);
   const int ncta = static_cast<int>(gridDim.x);
-  const int h = cid % P.H;
-  const int slot = cid / P.H;
-  const int nslots = (ncta - h + P.H - 1) / P.H;
+  const int nv = P.H * P.npass;
+  const int vh = cid % nv;
+  const int h = vh / P.npass, pass = vh - h * P.npass;
+  const int row0 = pass_row0(P, h, pass), nrow = pass_rows(P, pass);
+  const int slot = cid / nv;
+  const int nslots = (ncta - vh + nv - 1) / nv;
   const int ntiles = (P.S + DBM - 1) / DBM;
 
   if (warp == 0 && lane == 0) {
@@ -557,8 +572,8 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
   if (warp == 0) {
     if (elect_one()) {
       mbar_expect_tx(q_bar, R_Q_BYTES);
-      tma_load_2d(sQ, &P.q_map, q_bar, 0, h * P.qpk);            // dims 0..63 of q rows [h qpk, h qpk + 16)
-      tma_load_2d(sQ + R_Q_BYTES / 2, &P.q_map, q_bar, 64, h * P.qpk);
+      tma_load_2d(sQ, &P.q_map, q_bar, 0, row0);            // dims 0..63 of q rows [row0, row0 + 16)
+      tma_load_2d(sQ + R_Q_BYTES / 2, &P.q_map, q_bar, 64, row0);
       mbar_expect_tx(b_bar, static_cast<uint32_t>(P.nkb) * B_KB_BYTES);
       for (int kb = 0; kb < P.nkb; ++kb) tma_load_2d(sB + kb * B_KB_BYTES, &P.b_head_map, b_bar, kb * DBK, h * D);
     }
@@ -744,7 +759,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
       if (tok < P.S) {
 #pragma unroll
         for (int g = 0; g < D_MAX_QPK; ++g)
-          if (g < P.qpk) P.scores[static_cast<long long>(h * P.qpk + g) * P.ld_scores + tok] = __uint_as_float(v[g]) * P.scale;
+          if (g < nrow) P.scores[static_cast<long long>(row0 + g) * P.ld_scores + tok] = __uint_as_float(v[g]) * P.scale;
       }
       bph ^= 1u << b;
       b ^= 1;
@@ -767,23 +782,34 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_mma2_kernel(const 
 // 66 / 61 us per layer): a slot is held from the TMA issue until the MMAs that read it RETIRE, so at most ~2-3 loads
 // were in flight against an L2 round trip of ~0.6 us.  Half a slice leaves room for 9 slots (7 are used; 7 at r_k 768,
 // 5 at 1024 -- ranks whose whole slice does not fit at all).  The epilogue is the single-CTA kernel's, run by both
-// CTAs on their own tokens; the score MMA (M = 256, N = 16: 8 q rows from each CTA) is issued by the even CTA once
-// BOTH epilogues have written their rotated keys (remote mbarrier arrivals), commits are multicast to both CTAs.
+// CTAs on their own tokens; the score MMA (M = 256, N = nq16: nq16 / 2 q rows from each CTA) is issued by the even CTA
+// once BOTH epilogues have written their rotated keys (remote mbarrier arrivals), commits are multicast to both CTAs.
+// Multi-token steps: the qpk = (q heads per kv head) x (query tokens) <= 64 rows of a kv head all go through ONE score MMA
+// per tile, N = nq16 = qpk rounded up to 16; the 64 score columns of tensor memory hold 64 / nq16 buffers of nq16 columns
+// (4 x 16 up to 16 rows: the single-token layout, 2 x 32, then 1 x 48 or 1 x 64).  The reconstruction, the epilogue and
+// the 3 rotated-key buffers do not change with the row count.
 // ---------------------------------------------------------------------------------------------
 constexpr int PR_B_KB_BYTES = 64 * DBK * 2;        // one rank block of a half slice: 64 dims x 128 B
-constexpr int PR_Q_BYTES = 2 * 8 * 128;            // 8 q rows per CTA, two 64-dim chunks
-constexpr size_t PR_FIXED_BYTES = PR_Q_BYTES + 1024 /*align*/ + 512 /*barriers*/;
-constexpr int PR_A2 = 3, PR_D2 = 4;         // rotated-key / score buffers in tensor memory
-constexpr uint32_t PR_COL_A2 = 256, PR_COL_D2 = 256 + PR_A2 * 64;   // 256 accumulator columns, then 3 x 64, then 4 x 16 = 512
-static inline int pair_stages_for(int nkb) {
+constexpr int PR_A2 = 3, PR_D2 = 4;         // rotated-key / score buffers in tensor memory (score buffers: at most 4)
+constexpr uint32_t PR_COL_A2 = 256, PR_COL_D2 = 256 + PR_A2 * 64;   // 256 accumulator columns, then 3 x 64, then 64 score columns
+constexpr int PR_SCORE_COLS = 64;
+__host__ __device__ constexpr int pair_nq16(int qpk) { return (qpk + 15) & ~15; }
+// q rows of one CTA (nq16 / 2), two 64-dim chunks of 128 B per row: 2 KiB up to 16 rows per kv head
+__host__ __device__ constexpr int pair_q_bytes(int qpk) { return pair_nq16(qpk) * 128; }
+static inline size_t pair_fixed_bytes(int qpk) { return pair_q_bytes(qpk) + 1024 /*align*/ + 512 /*barriers*/; }
+static inline int pair_stages_for(int nkb, int qpk) {
   const size_t b = static_cast<size_t>(nkb) * PR_B_KB_BYTES;
-  if (b + PR_FIXED_BYTES + 3 * D_A_BYTES > R_SMEM_LIMIT) return 0;
-  int st = static_cast<int>((R_SMEM_LIMIT - PR_FIXED_BYTES - b) / D_A_BYTES);
+  const size_t fixed = pair_fixed_bytes(qpk);
+  if (b + fixed + 3 * D_A_BYTES > R_SMEM_LIMIT) return 0;
+  int st = static_cast<int>((R_SMEM_LIMIT - fixed - b) / D_A_BYTES);
   // measured (config 2, one layer): 3 / 5 / 6 / 7 / 8 / 9 slots -> 75.6 / 53.8 / 49.9 / 49.5 / 51.4 / 53.0 us: past 7 the extra
   // loads in flight only add L2 contention
   return st > 7 ? 7 : st;
 }
 
+// NQ16: the score MMA's N = q rows per kv head rounded up to 16 (a template parameter so that the single-token form,
+// NQ16 = 16, keeps its instruction descriptor, buffer ring and read-out as compile-time constants)
+template <int NQ16>
 __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const __grid_constant__ ScoreParams P) {
   constexpr int D = 128;
   extern __shared__ uint8_t smem_raw[];
@@ -792,7 +818,9 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
   uint8_t* sB = smem;                              // nkb x 8 KiB: this CTA's half of the head's right-factor slice
   uint8_t* sA = smem + P.nkb * PR_B_KB_BYTES;
   uint8_t* sQ = sA + R_STAGES * D_A_BYTES;
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(sQ + PR_Q_BYTES);   // used in the even CTA: both CTAs' loads land
+  constexpr int nq16 = NQ16, q_bytes = NQ16 * 128;
+  constexpr int nd2 = PR_SCORE_COLS / NQ16;        // score buffers
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(sQ + q_bytes);   // used in the even CTA: both CTAs' loads land
   uint64_t* empty_bar = full_bar + R_MAX_STAGES;   // in each CTA: multicast commit
   uint64_t* tfull_bar = empty_bar + R_MAX_STAGES;  // [2] in each CTA: multicast commit
   uint64_t* tempty_bar = tfull_bar + 2;            // [2] even CTA: the epilogue warps of BOTH CTAs
@@ -853,11 +881,11 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
       // both CTAs load their halves; every completion is counted on the even CTA's barriers
       const uint32_t qb = cluster_map_shared(smem_u32(q_bar), 0), bb = cluster_map_shared(smem_u32(b_bar), 0);
       if (leader) {
-        mbar_expect_tx(q_bar, 2 * PR_Q_BYTES);
+        mbar_expect_tx(q_bar, 2 * q_bytes);
         mbar_expect_tx(b_bar, 2u * static_cast<uint32_t>(P.nkb) * PR_B_KB_BYTES);
       }
-      tma_load_2d_pair(sQ, &P.q_half_map, qb, 0, h * P.qpk + crank * 8);
-      tma_load_2d_pair(sQ + PR_Q_BYTES / 2, &P.q_half_map, qb, 64, h * P.qpk + crank * 8);
+      tma_load_2d_pair(sQ, &P.q_half_map, qb, 0, h * P.qpk + crank * (nq16 / 2));
+      tma_load_2d_pair(sQ + q_bytes / 2, &P.q_half_map, qb, 64, h * P.qpk + crank * (nq16 / 2));
       for (int kb = 0; kb < P.nkb; ++kb)
         tma_load_2d_pair(sB + kb * PR_B_KB_BYTES, &P.b_half_map, bb, kb * DBK, h * D + crank * 64);
       int s = 0;
@@ -917,8 +945,8 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
     }
   } else if (warp == 2) {
     if (leader) {
-      // scores[256 x 16] = K^rot (each CTA's tensor memory) * Q^T (8 q rows from each CTA's shared memory)
-      constexpr uint32_t idesc2 = umma_idesc_bf16(2 * DBM, R_QROWS, 0, 0);
+      // scores[256 x nq16] = K^rot (each CTA's tensor memory) * Q^T (nq16 / 2 q rows from each CTA's shared memory)
+      constexpr uint32_t idesc2 = umma_idesc_bf16(2 * DBM, nq16, 0, 0);
       if (elect_one()) {
         mbar_wait_cluster(q_bar, 0);
         const uint64_t q_desc0 = umma_desc_sw128(smem_u32(sQ), 16, 1024);
@@ -929,18 +957,18 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
           mbar_wait_cluster(&d2empty_bar[bd], ((pd >> bd) & 1u) ^ 1u);
           tc_fence_after();
           const uint32_t a2 = tmem_base + PR_COL_A2 + static_cast<uint32_t>(ba * 64);
-          const uint32_t d2 = tmem_base + PR_COL_D2 + static_cast<uint32_t>(bd * 16);
+          const uint32_t d2 = tmem_base + PR_COL_D2 + static_cast<uint32_t>(bd * nq16);
 #pragma unroll
           for (int k = 0; k < D / 16; ++k)
             umma_bf16_ts_pair(d2, a2 + static_cast<uint32_t>(k * 8),
-                              q_desc0 + static_cast<uint64_t>(((k >> 2) * (PR_Q_BYTES / 2) + (k & 3) * 32) >> 4), idesc2,
+                              q_desc0 + static_cast<uint64_t>(((k >> 2) * (q_bytes / 2) + (k & 3) * 32) >> 4), idesc2,
                               k > 0 ? 1u : 0u);
           umma_commit_pair(&d2full_bar[bd]);
           umma_commit_pair(&a2empty_bar[ba]);
           pa ^= 1u << ba;
           pd ^= 1u << bd;
           ba = ba + 1 == PR_A2 ? 0 : ba + 1;
-          bd = bd + 1 == PR_D2 ? 0 : bd + 1;
+          bd = bd + 1 == nd2 ? 0 : bd + 1;
         }
       }
       __syncwarp();
@@ -1021,7 +1049,7 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
       ba = ba + 1 == PR_A2 ? 0 : ba + 1;
     }
   } else if (warp >= 4 + R_EPI_WARPS) {
-    // ===== score read-out: one warp per TMEM lane quarter, thread = token =====
+    // ===== score read-out: one warp per TMEM lane quarter, thread = token; the qpk score columns in groups of 8 =====
     const int qd = warp & 3;
     const int row = qd * 32 + lane;
     const uint32_t d2empty0 = cluster_map_shared(smem_u32(&d2empty_bar[0]), 0);
@@ -1031,20 +1059,26 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
       const int tok = (2 * tile + crank) * DBM + row;
       mbar_wait(&d2full_bar[b], (bph >> b) & 1u);
       tc_fence_after();
-      uint32_t v[8];
+      uint32_t v[NQ16 / 8][8];
+      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(qd * 32) << 16) + PR_COL_D2 + static_cast<uint32_t>(b * nq16);
       __syncwarp();
-      tmem_ld_32x8(tmem_base + (static_cast<uint32_t>(qd * 32) << 16) + PR_COL_D2 + static_cast<uint32_t>(b * 16), v);
+#pragma unroll
+      for (int c = 0; c < NQ16 / 8; ++c)
+        if (c == 0 || c * 8 < P.qpk) tmem_ld_32x8(taddr + static_cast<uint32_t>(c * 8), v[c]);
       tmem_ld_wait();
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(d2empty0 + static_cast<uint32_t>(b * 8));
       if (tok < P.S) {
 #pragma unroll
-        for (int g = 0; g < D_MAX_QPK; ++g)
-          if (g < P.qpk) P.scores[static_cast<long long>(h * P.qpk + g) * P.ld_scores + tok] = __uint_as_float(v[g]) * P.scale;
+        for (int c = 0; c < NQ16 / 8; ++c)
+#pragma unroll
+          for (int g = 0; g < 8; ++g)
+            if (c * 8 + g < P.qpk)
+              P.scores[static_cast<long long>(h * P.qpk + c * 8 + g) * P.ld_scores + tok] = __uint_as_float(v[c][g]) * P.scale;
       }
       bph ^= 1u << b;
-      b = b + 1 == PR_D2 ? 0 : b + 1;
+      b = b + 1 == nd2 ? 0 : b + 1;
     }
   }
   tc_fence_before();
@@ -1062,12 +1096,17 @@ __global__ void __launch_bounds__(R_THREADS, 1) decode_scores_pair_kernel(const 
 // operand) and the fp32 sum l_c; the slab reduction and the combine kernel rescale by exp(m_c - m).  One pass over
 // the scores instead of a max launch and an exp launch, and p keeps full bf16 precision inside every chunk.
 // The tail chunk's CTA first scores its tokens (scale * q . k_tail): nobody else reads those scores.
+// Rows: row r = hq * Tq + t is query token t of q head hq; qpk counts the rows of one kv head (q heads x Tq).  The last Tq
+// tail tokens are the queries' own, so row r sees the tail tokens [0, T - Tq + t] (causal); the tail chunk stops there and
+// the later tail tokens get no score and no probability (nothing downstream reads past tail_visible).
 constexpr int SM_MAX_CHUNKS = 72;   // >= 64 split-K slabs + the tail chunk
 
 // One (q head, chunk) unit, worked by NT threads (NT = 32: one warp, shuffles only -- the prefix chunks, a few KB each;
 // NT = 256: the whole block -- the dense tail chunk, which first has to score its tokens).
+__device__ __forceinline__ int tail_visible(int T, int Tq, int row) { return T - Tq + row % Tq + 1; }
+
 template <int NT>
-__device__ __forceinline__ void softmax_unit(float* __restrict__ scores, long long ld, int S, int T, int kps, int nchunk_s,
+__device__ __forceinline__ void softmax_unit(float* __restrict__ scores, long long ld, int S, int T, int Tq, int kps, int nchunk_s,
                                              const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k_tail,
                                              long long sh, long long st, int qpk, int D, float scale,
                                              __nv_bfloat16* __restrict__ prob, long long ldp, float* __restrict__ chunk_max,
@@ -1108,10 +1147,11 @@ __device__ __forceinline__ void softmax_unit(float* __restrict__ scores, long lo
     i0 = min(S, ch * kps * 64);
     i1 = min(S, (ch + 1) * kps * 64);
   } else {
+    const int tv = T > 0 ? tail_visible(T, Tq, hq) : 0;
     i0 = S;
-    i1 = S + T;
+    i1 = S + tv;
     const int h = hq / qpk;
-    for (int t = warp; t < T; t += NT / 32) {
+    for (int t = warp; t < tv; t += NT / 32) {
       const __nv_bfloat16* kr = k_tail + h * sh + t * st;
       float acc = 0.f;
       for (int d = lane; d < D; d += 32) acc += __bfloat162float(q[hq * D + d]) * __bfloat162float(kr[d]);
@@ -1178,7 +1218,7 @@ __device__ __forceinline__ void softmax_unit(float* __restrict__ scores, long lo
 // grid: ceil(Hq * nchunk_s / 8) blocks whose eight warps take one prefix (q head, chunk) unit each -- no block barrier, the
 // whole unit is one L2 round trip, a shuffle reduction, the exps and another shuffle reduction (the one-block-per-unit form
 // with its six block barriers took 7-8 us per layer) -- followed by Hq blocks for the tail chunks.
-__global__ void __launch_bounds__(256) softmax_chunk_kernel(float* __restrict__ scores, long long ld, int S, int T,
+__global__ void __launch_bounds__(256) softmax_chunk_kernel(float* __restrict__ scores, long long ld, int S, int T, int Tq,
                                                             int kps, int nchunk_s, int Hq, const __nv_bfloat16* __restrict__ q,
                                                             const __nv_bfloat16* __restrict__ k_tail, long long sh,
                                                             long long st, int qpk, int D, float scale,
@@ -1192,10 +1232,10 @@ __global__ void __launch_bounds__(256) softmax_chunk_kernel(float* __restrict__ 
   if (static_cast<int>(blockIdx.x) < nprefix_blocks) {
     const int unit = static_cast<int>(blockIdx.x) * 8 + static_cast<int>(threadIdx.x >> 5);
     if (unit >= Hq * nchunk_s) return;
-    softmax_unit<32>(scores, ld, S, T, kps, nchunk_s, q, k_tail, sh, st, qpk, D, scale, prob, ldp, chunk_max, chunk_sum, raw_bias,
+    softmax_unit<32>(scores, ld, S, T, Tq, kps, nchunk_s, q, k_tail, sh, st, qpk, D, scale, prob, ldp, chunk_max, chunk_sum, raw_bias,
                      row_scale, raw_scale, unit / nchunk_s, unit % nchunk_s, red, &bcast);
   } else {
-    softmax_unit<256>(scores, ld, S, T, kps, nchunk_s, q, k_tail, sh, st, qpk, D, scale, prob, ldp, chunk_max, chunk_sum, raw_bias,
+    softmax_unit<256>(scores, ld, S, T, Tq, kps, nchunk_s, q, k_tail, sh, st, qpk, D, scale, prob, ldp, chunk_max, chunk_sum, raw_bias,
                       row_scale, raw_scale, static_cast<int>(blockIdx.x) - nprefix_blocks, nchunk_s, red, &bcast);
   }
 }
@@ -1271,11 +1311,12 @@ __global__ void __launch_bounds__(256) reduce_u_kernel(const float* __restrict__
 }
 
 // o[hq][d] = ( sum_j U[hq][j] * Bv[(h*D + d)][j]  +  sum_t p_tail[hq][t] * v_tail[h][t][d] ) / rowsum[hq]
-// grid (Hq, D / 8), 8 warps x 1 output dim (a short dependency chain per warp; U is re-read by the D / 8 blocks of a head).
+// (hq: a q row as in softmax_unit, h = hq / qpk its kv head; qpk counts the rows of a kv head)
+// grid (rows, D / 8), 8 warps x 1 output dim (a short dependency chain per warp; U is re-read by the D / 8 blocks of a head).
 __global__ void __launch_bounds__(256) combine_kernel(const float* __restrict__ slabs, int nslabs, long long slab_stride,
                                                       int rv, const __nv_bfloat16* __restrict__ Bv, long long ldb,
                                                       const __nv_bfloat16* __restrict__ prob, long long ldp, int S, int T,
-                                                      const __nv_bfloat16* __restrict__ v_tail, long long sh, long long st,
+                                                      int Tq, const __nv_bfloat16* __restrict__ v_tail, long long sh, long long st,
                                                       const float* __restrict__ rowsum, int qpk, int D,
                                                       __nv_bfloat16* __restrict__ out,
                                                       const float* __restrict__ chunk_max, int nchunks,
@@ -1294,6 +1335,7 @@ __global__ void __launch_bounds__(256) combine_kernel(const float* __restrict__ 
   const float m = stats[0], rs = stats[1];
   const float inv = 1.f / rs;
   const float w_tail = T > 0 ? w_s[nchunks - 1] : 0.f;
+  const int tv = T > 0 ? tail_visible(T, Tq, hq) : 0;   // causal: the tail tokens this row sees
   if (lse_out != nullptr && blockIdx.y == 0 && threadIdx.x == 0) {
     // log-sum-exp of this head's scaled scores over the tokens of THIS call: what a flash-decoding style merge of
     // token shards needs besides the normalised output
@@ -1307,7 +1349,7 @@ __global__ void __launch_bounds__(256) combine_kernel(const float* __restrict__ 
       acc = fmaf(u_s[j], __bfloat162float(b2.x), fmaf(u_s[j + 1], __bfloat162float(b2.y), acc));
     }
     float acc_t = 0.f;
-    for (int t = lane; t < T; t += 32)
+    for (int t = lane; t < tv; t += 32)
       acc_t = fmaf(__bfloat162float(prob[hq * ldp + S + t]), __bfloat162float(v_tail[h * sh + t * st + d]), acc_t);
     acc = warp_sum(fmaf(w_tail, acc_t, acc));
     if (lane == 0) out[hq * D + d] = __float2bfloat16_rn(acc * inv);
@@ -1323,7 +1365,7 @@ constexpr int RC_CL = 8;
 __global__ void __launch_bounds__(256) reduce_combine_kernel(const float* __restrict__ slabs, int nslabs, long long slab_stride,
                                                              int rv, const __nv_bfloat16* __restrict__ Bv, long long ldb,
                                                              const __nv_bfloat16* __restrict__ prob, long long ldp, int S, int T,
-                                                             const __nv_bfloat16* __restrict__ v_tail, long long sh, long long st,
+                                                             int Tq, const __nv_bfloat16* __restrict__ v_tail, long long sh, long long st,
                                                              const float* __restrict__ rowsum, int qpk, int D,
                                                              __nv_bfloat16* __restrict__ out,
                                                              const float* __restrict__ chunk_max, int nchunks,
@@ -1375,8 +1417,9 @@ __global__ void __launch_bounds__(256) reduce_combine_kernel(const float* __rest
       const __nv_bfloat162 b2 = *reinterpret_cast<const __nv_bfloat162*>(row + jj);
       acc = fmaf(u_s[jj], __bfloat162float(b2.x), fmaf(u_s[jj + 1], __bfloat162float(b2.y), acc));
     }
+    const int tv = T > 0 ? tail_visible(T, Tq, hq) : 0;   // causal: the tail tokens this row sees
     float acc_t = 0.f;
-    for (int t = lane; t < T; t += 32)
+    for (int t = lane; t < tv; t += 32)
       acc_t = fmaf(__bfloat162float(prob[hq * ldp + S + t]), __bfloat162float(v_tail[h * sh + t * st + d]), acc_t);
     acc = warp_sum(fmaf(w_tail, acc_t, acc));
     if (lane == 0) out[hq * D + d] = __float2bfloat16_rn(acc * inv);
@@ -1417,13 +1460,14 @@ __global__ void __launch_bounds__(256) rope_bf16_kernel(__nv_bfloat16* __restric
 }
 
 static inline size_t al(size_t x) { return (x + 1023) / 1024 * 1024; }
-// Split-K factor of U = P A_v: as many K slices as make tiles_n x split CTAs fill the SMs ONCE (a 64-way split of
-// 3 column tiles is 192 CTAs = 1.3 waves on 148 SMs: the second wave runs at a third of the machine).
-static inline int decode_split_k(int S, int rv) {
+// Split-K factor of U = P A_v (M rows): as many K slices as make tiles_m x tiles_n x split CTAs fill the SMs ONCE (a
+// 64-way split of 3 column tiles is 192 CTAs = 1.3 waves on 148 SMs: the second wave runs at a third of the machine).
+static inline int decode_split_k(int S, int rv, int M) {
   const int nkb = (S + 63) / 64;
   const int tiles_n = (rv + 255) / 256;
+  const int tiles_m = (M + 127) / 128;
   const int sms = device_sm_count();
-  int split = sms / (tiles_n < 1 ? 1 : tiles_n);
+  int split = sms / (tiles_n * tiles_m < 1 ? 1 : tiles_n * tiles_m);
   if (split > nkb) split = nkb;
   if (split > 64) split = 64;
   if (split < 1) split = 1;
@@ -1436,7 +1480,7 @@ static int g_scores_variant = 0;           // test hook: 0 automatic, 1 FFMA epi
 static bool g_split_reduce_combine = false;   // test hook (variant 4): slab reduction and combine as two launches
 
 // Launch the single-CTA score-MMA kernel (persistent: one CTA per SM, every head at least one).
-static int launch_scores_mma2(const ScoreParams& sp, int S, int H, cudaStream_t st) {
+static int launch_scores_mma2(const ScoreParams& sp, int S, int H, cudaStream_t st) {   // H: row sets (kv heads x passes)
   static PerDevice<bool> configured;
   if (!configured()) {
     XKV_CHECK_CUDA(cudaFuncSetAttribute(decode_scores_mma2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -1457,12 +1501,12 @@ static int launch_scores_mma2(const ScoreParams& sp, int S, int H, cudaStream_t 
 static int launch_scores_pair(ScoreParams& sp, int S, int H, cudaStream_t st) {
   static PerDevice<int> state;   // 0: not probed, -1: not launchable, > 0: resident pairs
   int& resident = state();
-  sp.stages = pair_stages_for(sp.nkb);
+  sp.stages = pair_stages_for(sp.nkb, sp.qpk);
   if (sp.stages < 3) return -1;
   cudaLaunchConfig_t cfg;
   std::memset(&cfg, 0, sizeof(cfg));
   cfg.blockDim = dim3(R_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = PR_FIXED_BYTES + static_cast<size_t>(sp.nkb) * PR_B_KB_BYTES + static_cast<size_t>(sp.stages) * D_A_BYTES;
+  cfg.dynamicSmemBytes = pair_fixed_bytes(sp.qpk) + static_cast<size_t>(sp.nkb) * PR_B_KB_BYTES + static_cast<size_t>(sp.stages) * D_A_BYTES;
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -1473,13 +1517,16 @@ static int launch_scores_pair(ScoreParams& sp, int S, int H, cudaStream_t st) {
   cfg.numAttrs = 1;
   if (resident == 0) {
     resident = -1;
-    if (cudaFuncSetAttribute(decode_scores_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             static_cast<int>(R_SMEM_LIMIT)) == cudaSuccess) {
+    const int lim = static_cast<int>(R_SMEM_LIMIT);
+    if (cudaFuncSetAttribute(decode_scores_pair_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim) == cudaSuccess &&
+        cudaFuncSetAttribute(decode_scores_pair_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim) == cudaSuccess &&
+        cudaFuncSetAttribute(decode_scores_pair_kernel<48>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim) == cudaSuccess &&
+        cudaFuncSetAttribute(decode_scores_pair_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim) == cudaSuccess) {
       int n = 0;
       cfg.gridDim = dim3(2, 1, 1);
       const size_t launch_smem = cfg.dynamicSmemBytes;
-      cfg.dynamicSmemBytes = R_SMEM_LIMIT;   // one CTA per SM whatever the rank
-      if (cudaOccupancyMaxActiveClusters(&n, decode_scores_pair_kernel, &cfg) == cudaSuccess && n >= 1) resident = n;
+      cfg.dynamicSmemBytes = R_SMEM_LIMIT;   // one CTA per SM whatever the rank (the same for every instantiation)
+      if (cudaOccupancyMaxActiveClusters(&n, decode_scores_pair_kernel<16>, &cfg) == cudaSuccess && n >= 1) resident = n;
       cfg.dynamicSmemBytes = launch_smem;
     }
     (void)cudaGetLastError();
@@ -1489,16 +1536,24 @@ static int launch_scores_pair(ScoreParams& sp, int S, int H, cudaStream_t st) {
   int npairs = resident < ptiles * H ? resident : ptiles * H;
   if (npairs < H) npairs = H;   // every head needs at least one pair
   cfg.gridDim = dim3(2 * npairs, 1, 1);
-  XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, decode_scores_pair_kernel, sp));
+  switch (pair_nq16(sp.qpk)) {
+    case 16: XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, decode_scores_pair_kernel<16>, sp)); break;
+    case 32: XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, decode_scores_pair_kernel<32>, sp)); break;
+    case 48: XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, decode_scores_pair_kernel<48>, sp)); break;
+    default: XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, decode_scores_pair_kernel<64>, sp)); break;
+  }
   return 0;
 }
 
-// scores[hq][t] = scale * q_hq . rope(bf16(A_k[t] Bk_l^T)) for the S tokens of the compressed prefix: fused reconstruct +
-// RoPE + q.K, one launch (kernel chosen by head_dim, rank and the test hooks)
-static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, int64_t lda_k, int rk, const void* Vk_layer,
+// scores[r][t] = scale * q_r . rope(bf16(A_k[t] Bk_l^T)) for the S tokens of the compressed prefix and the `rows` q rows
+// (rows / H contiguous rows per kv head): fused reconstruct + RoPE + q.K, one launch (kernel chosen by head_dim, rank and
+// the test hooks).  The pair kernel takes all rows of a kv head at once; the others work rows / H > 8 in passes of <= 8
+// rows, one CTA set per pass (each pass rebuilds the keys of the whole prefix).
+static int launch_scores(const void* q, int rows, int H, int D, const void* A_k, int64_t lda_k, int rk, const void* Vk_layer,
                          int64_t ldv_k, int S, const void* cos, const void* sin, int64_t ld_cs, float scale, float* scores,
                          long long ldl, cudaStream_t st) {
-  const int qpk = Hq / H;
+  const int qpk = rows / H;
+  const int npass = (qpk + D_MAX_QPK - 1) / D_MAX_QPK;
   int rc;
   static thread_local ScoreParams sp;
   std::memset(&sp, 0, sizeof(sp));
@@ -1510,9 +1565,9 @@ static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, i
   if (rc) return rc;
   const bool q_tma_ok = D == 128 && (reinterpret_cast<uintptr_t>(q) & 15) == 0;
   if (q_tma_ok) {
-    rc = encode_tmap_2d_bf16(&sp.q_map, q, D, Hq, D, 64, R_QROWS);
+    rc = encode_tmap_2d_bf16(&sp.q_map, q, D, rows, D, 64, R_QROWS);
     if (rc) return rc;
-    rc = encode_tmap_2d_bf16(&sp.q_half_map, q, D, Hq, D, 64, 8);
+    rc = encode_tmap_2d_bf16(&sp.q_half_map, q, D, rows, D, 64, pair_nq16(qpk) / 2);
     if (rc) return rc;
     rc = encode_tmap_2d_bf16(&sp.b_half_map, Vk_layer, rk, static_cast<uint64_t>(H) * D, ldv_k, DBK, 64);
     if (rc) return rc;
@@ -1527,6 +1582,7 @@ static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, i
   sp.rk = rk;
   sp.H = H;
   sp.qpk = qpk;
+  sp.npass = 1;
   sp.tiles_n = (H * D + DBN - 1) / DBN;
   sp.nkb = (rk + DBK - 1) / DBK;
   sp.scale = scale;
@@ -1545,7 +1601,7 @@ static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, i
     configured() = true;
   }
   // CTA pairs (half a slice per CTA, deep ring) when the head layout allows the score MMA: the default for head_dim 128
-  if (D == 128 && q_tma_ok && qpk <= 8 && !g_force_tiled_scores && (g_scores_variant == 0 || g_scores_variant == 3)) {
+  if (D == 128 && q_tma_ok && qpk <= PR_SCORE_COLS && !g_force_tiled_scores && (g_scores_variant == 0 || g_scores_variant == 3)) {
     const int prc = launch_scores_pair(sp, S, H, st);
     if (prc > 0) return prc;
     if (prc == 0) {
@@ -1554,24 +1610,26 @@ static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, i
     }
     sp.stages = r_stages_for(sp.nkb);
   }
+  sp.npass = npass;
+  const int nv = H * npass;   // row sets: (kv head, pass)
   // persistent kernel when one head's slice of the right factor fits in shared memory
   const bool persistent = static_cast<size_t>(sp.nkb) * D * DBK * 2 <= PB_MAX_BYTES && !g_force_tiled_scores;
   if (persistent) {
     const int sms = device_sm_count();
     const int ntiles = (S + DBM - 1) / DBM;
-    int pgrid = sms < ntiles * H ? sms : ntiles * H;
-    if (pgrid < H) pgrid = H;   // every head needs at least one CTA
-    if (D == 128 && q_tma_ok && qpk <= 8 && g_scores_variant != 1) {
-      rc = launch_scores_mma2(sp, S, H, st);
+    int pgrid = sms < ntiles * nv ? sms : ntiles * nv;
+    if (pgrid < nv) pgrid = nv;   // every row set needs at least one CTA
+    if (D == 128 && q_tma_ok && g_scores_variant != 1) {
+      rc = launch_scores_mma2(sp, S, nv, st);
       if (rc) return rc;
     } else if (D == 128)
       decode_scores_persistent_kernel<128><<<pgrid, P_THREADS, P_SMEM_BYTES, st>>>(sp);
     else
       decode_scores_persistent_kernel<64><<<pgrid, P_THREADS, P_SMEM_BYTES, st>>>(sp);
   } else if (D == 128) {
-    decode_scores_kernel<128><<<grid, D_THREADS, D_SMEM_BYTES, st>>>(sp);
+    decode_scores_kernel<128><<<dim3(grid, npass), D_THREADS, D_SMEM_BYTES, st>>>(sp);
   } else {
-    decode_scores_kernel<64><<<grid, D_THREADS, D_SMEM_BYTES, st>>>(sp);
+    decode_scores_kernel<64><<<dim3(grid, npass), D_THREADS, D_SMEM_BYTES, st>>>(sp);
   }
   XKV_LAUNCHED();
   return 0;
@@ -1581,62 +1639,74 @@ static int launch_scores(const void* q, int Hq, int H, int D, const void* A_k, i
 
 using namespace xkv;
 
+// Hq: q rows (q heads x query tokens of a multi-token step)
 extern "C" size_t xkv_decode_workspace_bytes(int Hq, int S, int T, int rv) {
   const size_t L = static_cast<size_t>(S) + T;
   const size_t ldl = (L + 63) / 64 * 64;
   const int nkb = (S + 63) / 64;
   (void)nkb;
   const int split = 64;   // upper bound of decode_split_k
+  const size_t prob_rows = (static_cast<size_t>(Hq) + 127) / 128 * 128;
   size_t b = 0;
   b += al(Hq * ldl * 4);            // scores
-  b += al(128 * ldl * 2);           // probabilities (bf16), padded to a full 128-row tile
+  b += al(prob_rows * ldl * 2);     // probabilities (bf16), padded to full 128-row tiles
   b += al(2 * Hq * SM_MAX_CHUNKS * 4);   // per-chunk max / sum of the softmax
   b += al(static_cast<size_t>(split + 1) * Hq * rv * 4);  // split-K slabs of U, then U itself
   return b + 1024;
 }
 
-extern "C" int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, const void* A_k, int64_t lda_k, int rk,
-                                    const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,
-                                    const void* Vv_layer, int64_t ldv_v, int S, const void* cos, const void* sin,
-                                    int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
-                                    int64_t tail_stride_t, float scale, void* out, void* workspace,
-                                    size_t workspace_bytes, void* stream, float* lse_out) {
+// Multi-token step: q / out (Hq * Tq, D), row hq * Tq + t = query token t of q head hq; the last Tq of the T tail tokens
+// are the queries' own and attention among them is causal.  Internally every per-head quantity is per ROW (rows = Hq Tq,
+// qpk below = rows per kv head).
+extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                                          const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,
+                                          const void* Vv_layer, int64_t ldv_v, int S, const void* cos, const void* sin,
+                                          int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
+                                          int64_t tail_stride_t, float scale, void* out, void* workspace,
+                                          size_t workspace_bytes, void* stream, float* lse_out) {
   XKV_REQUIRE(q && A_k && Vk_layer && A_v && Vv_layer && out && workspace, "decode: null argument");
   XKV_REQUIRE(D == 64 || D == 128, "decode: head_dim %d not supported (64 or 128)", D);
-  XKV_REQUIRE(H >= 1 && Hq % H == 0 && Hq / H <= D_MAX_QPK && Hq <= 128, "decode: unsupported head counts Hq=%d H=%d", Hq, H);
+  XKV_REQUIRE(Tq >= 1, "decode: Tq=%d query tokens (at least 1)", Tq);
+  XKV_REQUIRE(H >= 1 && Hq >= 1 && Hq % H == 0, "decode: unsupported head counts Hq=%d H=%d", Hq, H);
+  XKV_REQUIRE((Hq / H) * Tq <= 64 && Hq * Tq <= 512,
+              "decode: %d q heads per kv head x %d query tokens (at most 64 rows per kv head) and %d q heads (at most 512 "
+              "rows in all) is past the fused kernel's bounds", Hq / H, Tq, Hq);
   XKV_REQUIRE(S >= 1 && T >= 0 && rk >= 1 && rv >= 1 && rv % 2 == 0, "decode: bad sizes");
+  // a single query may come without a tail (xkv_decode_attention); several queries attend to their own tokens
+  XKV_REQUIRE(Tq == 1 || T >= Tq, "decode: the tail (T=%d) must hold the Tq=%d query tokens", T, Tq);
   XKV_REQUIRE(T == 0 || (k_tail && v_tail), "decode: tail pointers missing");
   XKV_REQUIRE((cos == nullptr) == (sin == nullptr), "decode: cos and sin must both be given or both be null");
   XKV_REQUIRE(cos == nullptr || ld_cs % 8 == 0, "decode: cos/sin row stride must be a multiple of 8");
-  XKV_REQUIRE(workspace_bytes >= xkv_decode_workspace_bytes(Hq, S, T, rv), "decode: workspace too small");
+  const int rows = Hq * Tq;
+  XKV_REQUIRE(workspace_bytes >= xkv_decode_workspace_bytes(rows, S, T, rv), "decode: workspace too small");
   XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "decode: workspace must be 256-byte aligned");
   cudaStream_t st = as_stream(stream);
-  const int qpk = Hq / H;
+  const int qpk = rows / H;
   const size_t L = static_cast<size_t>(S) + T;
   const long long ldl = static_cast<long long>((L + 63) / 64 * 64);
   const int nkb_s = (S + 63) / 64;
   (void)nkb_s;
-  const int split = decode_split_k(S, rv);
+  const int split = decode_split_k(S, rv, rows);
   char* w = static_cast<char*>(workspace);
   float* scores = reinterpret_cast<float*>(w);
-  w += al(Hq * ldl * 4);
+  w += al(rows * ldl * 4);
   __nv_bfloat16* prob = reinterpret_cast<__nv_bfloat16*>(w);
-  w += al(128 * ldl * 2);
+  w += al((static_cast<size_t>(rows) + 127) / 128 * 128 * ldl * 2);
   float* rowsum = reinterpret_cast<float*>(w);        // per-chunk sums of p
-  float* chunk_max = rowsum + Hq * SM_MAX_CHUNKS;
-  w += al(2 * Hq * SM_MAX_CHUNKS * 4);
+  float* chunk_max = rowsum + rows * SM_MAX_CHUNKS;
+  w += al(2 * rows * SM_MAX_CHUNKS * 4);
   float* u_slabs = reinterpret_cast<float*>(w);
-  w += al(static_cast<size_t>(split + 1) * Hq * rv * 4);
+  w += al(static_cast<size_t>(split + 1) * rows * rv * 4);
 
   // ---- scores of the compressed prefix: fused reconstruct + RoPE + q.K ----
-  int rc = launch_scores(q, Hq, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, S, cos, sin, ld_cs, scale, scores, ldl, st);
+  int rc = launch_scores(q, rows, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, S, cos, sin, ld_cs, scale, scores, ldl, st);
   if (rc) return rc;
   // ---- softmax with chunk-local maxima: chunk c = token range of split-K slab c, last chunk = the dense tail ----
   const int nkb_p = (S + 63) / 64;
   const int kps = (nkb_p + split - 1) / split;          // k-blocks per slab, as xkv_gemm_grouped cuts them
   const int nchunks = split + 1;
   XKV_REQUIRE(nchunks <= SM_MAX_CHUNKS, "decode: too many softmax chunks");
-  softmax_chunk_kernel<<<(Hq * split + 7) / 8 + Hq, 256, 0, st>>>(scores, ldl, S, T, kps, split, Hq, static_cast<const __nv_bfloat16*>(q),
+  softmax_chunk_kernel<<<(rows * split + 7) / 8 + rows, 256, 0, st>>>(scores, ldl, S, T, Tq, kps, split, rows, static_cast<const __nv_bfloat16*>(q),
                                                           static_cast<const __nv_bfloat16*>(k_tail), tail_stride_h,
                                                           tail_stride_t, qpk, D, scale, prob, ldl, chunk_max, rowsum, nullptr, nullptr,
                                                           0.f);
@@ -1644,7 +1714,7 @@ extern "C" int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, con
   // ---- U = P[:, :S] * A_v  (tokens are the contraction: P K-major, A_v MN-major) ----
   xkv_gemm_problem gp;
   std::memset(&gp, 0, sizeof(gp));
-  gp.M = Hq;
+  gp.M = rows;
   gp.N = rv;
   gp.K = S;
   gp.num_terms = 1;
@@ -1657,14 +1727,14 @@ extern "C" int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, con
   gp.D = u_slabs;
   gp.ldd = rv;
   gp.split_k = split;
-  gp.split_stride = static_cast<long long>(Hq) * rv;
+  gp.split_stride = static_cast<long long>(rows) * rv;
   rc = xkv_gemm_grouped(&gp, 1, stream);
   if (rc) return rc;
   // ---- o = (U Bv_l^T + P_tail V_tail) / rowsum, U reduced over the split-K slabs by the same launch ----
   if (rv <= 128 * RC_CL && split <= 64 && !g_split_reduce_combine) {
     cudaLaunchConfig_t cfg;
     std::memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(Hq, RC_CL, 1);
+    cfg.gridDim = dim3(rows, RC_CL, 1);
     cfg.blockDim = dim3(256, 1, 1);
     cfg.dynamicSmemBytes = rv * sizeof(float);
     cfg.stream = st;
@@ -1676,24 +1746,36 @@ extern "C" int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, con
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, reduce_combine_kernel, static_cast<const float*>(u_slabs), split,
-                                      static_cast<long long>(Hq) * rv, rv, static_cast<const __nv_bfloat16*>(Vv_layer),
-                                      static_cast<long long>(ldv_v), static_cast<const __nv_bfloat16*>(prob), ldl, S, T,
+                                      static_cast<long long>(rows) * rv, rv, static_cast<const __nv_bfloat16*>(Vv_layer),
+                                      static_cast<long long>(ldv_v), static_cast<const __nv_bfloat16*>(prob), ldl, S, T, Tq,
                                       static_cast<const __nv_bfloat16*>(v_tail), static_cast<long long>(tail_stride_h),
                                       static_cast<long long>(tail_stride_t), static_cast<const float*>(rowsum), qpk, D,
                                       static_cast<__nv_bfloat16*>(out), static_cast<const float*>(chunk_max), nchunks, lse_out));
     XKV_LAUNCHED();
     return 0;
   }
-  float* U = u_slabs + static_cast<size_t>(split) * Hq * rv;
-  reduce_u_kernel<<<dim3((rv + 63) / 64, Hq), 256, 0, st>>>(u_slabs, split, static_cast<long long>(Hq) * rv, rv, chunk_max,
-                                                            rowsum, nchunks, U, 0, nullptr);
+  float* U = u_slabs + static_cast<size_t>(split) * rows * rv;
+  reduce_u_kernel<<<dim3((rv + 63) / 64, rows), 256, 0, st>>>(u_slabs, split, static_cast<long long>(rows) * rv, rv, chunk_max,
+                                                              rowsum, nchunks, U, 0, nullptr);
   XKV_LAUNCHED();
-  combine_kernel<<<dim3(Hq, (D + 7) / 8), 256, rv * sizeof(float), st>>>(
+  combine_kernel<<<dim3(rows, (D + 7) / 8), 256, rv * sizeof(float), st>>>(
       U, 1, 0, rv, static_cast<const __nv_bfloat16*>(Vv_layer), ldv_v, prob, ldl, S,
-      T, static_cast<const __nv_bfloat16*>(v_tail), tail_stride_h, tail_stride_t, rowsum, qpk, D,
+      T, Tq, static_cast<const __nv_bfloat16*>(v_tail), tail_stride_h, tail_stride_t, rowsum, qpk, D,
       static_cast<__nv_bfloat16*>(out), chunk_max, nchunks, lse_out);
   XKV_LAUNCHED();
   return 0;
+}
+
+extern "C" int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                                        const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,
+                                        const void* Vv_layer, int64_t ldv_v, int S, const void* cos, const void* sin,
+                                        int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
+                                        int64_t tail_stride_t, float scale, void* out, void* workspace,
+                                        size_t workspace_bytes, void* stream, float* lse_out) {
+  XKV_REQUIRE(H >= 1 && Hq % H == 0 && Hq / H <= D_MAX_QPK && Hq <= 128, "decode: unsupported head counts Hq=%d H=%d", Hq, H);
+  return xkv_decode_attention_multi(q, Hq, 1, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, A_v, lda_v, rv, Vv_layer, ldv_v, S, cos,
+                                    sin, ld_cs, k_tail, v_tail, T, tail_stride_h, tail_stride_t, scale, out, workspace,
+                                    workspace_bytes, stream, lse_out);
 }
 
 extern "C" size_t xkv_decode_absorbed_workspace_bytes(int Hq, int S, int r) {
@@ -1719,7 +1801,7 @@ extern "C" int xkv_decode_absorbed(const void* q_hat, int Hq, const void* A, int
   XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "absorbed decode: workspace must be 256-byte aligned");
   cudaStream_t st = as_stream(stream);
   const long long ldl = static_cast<long long>((static_cast<size_t>(S) + 63) / 64 * 64);
-  const int split = decode_split_k(S, r);
+  const int split = decode_split_k(S, r, Hq);
   char* w = static_cast<char*>(workspace);
   float* scores = reinterpret_cast<float*>(w);
   w += al(Hq * ldl * 4);
@@ -1755,7 +1837,7 @@ extern "C" int xkv_decode_absorbed(const void* q_hat, int Hq, const void* A, int
   XKV_REQUIRE(nchunks <= SM_MAX_CHUNKS, "absorbed decode: too many softmax chunks");
   XKV_REQUIRE(scale != 0.f, "absorbed decode: the softmax scale must not be zero");
   XKV_REQUIRE(row_scale == nullptr || (reinterpret_cast<uintptr_t>(row_scale) & 15) == 0, "absorbed decode: row_scale must be 16-byte aligned");
-  softmax_chunk_kernel<<<(Hq * split + 7) / 8 + Hq, 256, 0, st>>>(scores, ldl, S, 0, kps, split, Hq, nullptr, nullptr, 0, 0, 1, 0, scale,
+  softmax_chunk_kernel<<<(Hq * split + 7) / 8 + Hq, 256, 0, st>>>(scores, ldl, S, 0, 1, kps, split, Hq, nullptr, nullptr, 0, 0, 1, 0, scale,
                                                           prob, ldl, chunk_max, rowsum, bias_q != nullptr ? bias : nullptr,
                                                           row_scale, scale);
   XKV_LAUNCHED();

@@ -32,6 +32,13 @@ from .._lib import XkvError
 from ..configurations import LayerGroup, xKVConfig
 
 
+def is_prefill_step(cache, layer_idx: int, q_len: int) -> bool:
+    """The routing rule of the patched attention forwards: a forward is the prefill only when it brings several tokens
+    to a layer that holds none yet.  Every later forward is a decode step of q_len tokens (one token, a speculative
+    draft being verified, or a continuation chunk), appended exact to the dense tail."""
+    return q_len > 1 and (cache is None or cache.get_seq_length(layer_idx) == 0)
+
+
 class _XkvLayer(DynamicLayer):
     """One layer's slot: dense prefill K/V until its group is compressed, then (group factors, dense tail)."""
 
@@ -82,6 +89,37 @@ class _XkvLayer(DynamicLayer):
             self.kpre_from = need                    # a token without a pre-RoPE copy: nothing up to here can be folded
         self.tail_len = need
 
+    def check_crop(self, max_length: int) -> int:
+        """Tokens a compressed layer keeps after crop(max_length); XkvError when that cuts into the compressed prefix.
+        One exception: right after the prefill (no decode token yet, nothing folded), the prefill's own last tokens
+        may be dropped -- assisted decoding verifies its first drafts in the prefill forward.  Their token-factor rows
+        are cut; the group's basis, fitted with them, stays."""
+        current = self.get_seq_length()
+        keep = current - abs(max_length) if max_length < 0 else max_length
+        fresh = self.tail_len == 0 and self.group.length == self.group.prefill_tokens
+        if keep < current and keep < self.prefill_len and not (fresh and keep >= 1):
+            raise XkvError(f"FakeLayerMergingCache.crop: cannot crop to {keep} tokens, below the {self.prefill_len} "
+                           "tokens already compressed into the layer group's factors")
+        return keep
+
+    def crop(self, max_length: int) -> None:
+        """Keep the first ``max_length`` tokens (negative: drop ``-max_length``), as ``DynamicLayer.crop``.  A compressed
+        layer loses tokens of its dense tail; its compressed prefix is cut only in the case check_crop allows."""
+        if self.group is None:
+            return super().crop(max_length)
+        keep = self.check_crop(max_length)
+        if keep >= self.get_seq_length():
+            return
+        if keep < self.prefill_len:                  # the prefill's last tokens (check_crop allowed it)
+            self.prefill_len = self.group.length = keep
+            self.group.prefill_tokens = keep
+            for name in ("dense_k", "dense_v"):
+                if getattr(self, name) is not None:
+                    setattr(self, name, getattr(self, name)[..., :keep, :])
+        self.tail_len = keep - self.prefill_len
+        # RoPE rows waiting for the fold belong to the tail tokens: the rejected ones leave with them
+        del self.group.tail_rope[self.tail_len:]
+
 
 class _GroupState:
     """Factors of one compressed group and the RoPE tables of its prefill positions."""
@@ -95,8 +133,10 @@ class _GroupState:
         self.cos = cos      # (S, D) bf16 or None
         self.sin = sin
         self.re_apply_rope = re_apply_rope
-        # RoPE rows (cos, sin) of the decode tokens waiting in the dense tails, one per decode step (recorded when the
-        # group's first layer sees the token); consumed when the tokens are folded into the factors
+        self.length = 0            # tokens in the factors (prefill, then folded decode tokens)
+        self.prefill_tokens = 0    # of which the prefill compressed
+        # RoPE rows (cos, sin) of the decode tokens waiting in the dense tails, one per token (recorded when the group's
+        # first layer sees the token); consumed when the tokens are folded into the factors, trimmed by crop()
         self.tail_rope: List[Tuple[torch.Tensor, torch.Tensor]] = []
 
 
@@ -139,8 +179,10 @@ class FakeLayerMergingCache(DynamicCache):
 
     def update(self, key, value, layer_idx, mode="prefill", cos=None, sin=None, re_apply_rope=True,
                return_dense=True):
-        """Reference cache:127-153.  Prefill: stash the layer's (pre-RoPE) K and V; when the last layer of a
-        group arrives, compress the group; keys of un-grouped layers get RoPE immediately.  Decode: append
+        """Reference cache:127-153.  Prefill happens once, on an empty layer; every later forward is a decode step
+        whatever its token count (speculative verification, a continuation chunk): the tokens are appended to the dense
+        tail, exact, and nothing is re-compressed (the reference assumes a single prefill, SURVEY 9.7; this extends it).
+        Prefill: stash the layer's (pre-RoPE) K and V; when the last layer of a group arrives, compress the group; keys of un-grouped layers get RoPE immediately.  Decode: append
         the (post-RoPE) token to the dense tail.  Returns dense (K_l, V_l) as the reference does;
         ``return_dense=False`` (an extension used by callers that ignore the return, llama.py:46-49) skips
         the materialisation."""
@@ -221,6 +263,7 @@ class FakeLayerMergingCache(DynamicCache):
             sn[:seq] = sin[0]
         state = _GroupState(info, gf, self.num_heads, self.head_dim, cs, sn, bool(re_rope))
         state.length = seq
+        state.prefill_tokens = seq                   # compressed by the prefill itself (crop may still cut those)
         state.layer_ids = ids
         self._groups[first] = state
         for pos, l in enumerate(layers):
@@ -310,34 +353,40 @@ class FakeLayerMergingCache(DynamicCache):
     def attend(self, query: torch.Tensor, key: torch.Tensor, value: torch.Tensor, layer_idx: int,
                scaling: float, key_pre_rope: Optional[torch.Tensor] = None, cos: Optional[torch.Tensor] = None,
                sin: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
-        """Decode step of one layer: append the new (post-RoPE) token and attend over the factored cache with
-        the fused kernel.  query (1, Hq, 1, D) -> (1, Hq, 1, D).  Returns None when the layer is not factored on
-        both sides (the caller then uses the dense path).  key_pre_rope / cos / sin of the new position are
-        only needed when decode tokens are folded into the factors (compress_decode_tokens)."""
+        """Decode step of one layer: append the Tq new (post-RoPE) tokens and attend over the factored cache with
+        the fused kernel, causally among the new tokens.  query (1, Hq, Tq, D) -> (1, Hq, Tq, D).  Returns None, having
+        appended nothing, when the layer is not factored on both sides or the step is past the fused kernel's bounds
+        ((Hq / H) * Tq > 64 or Hq * Tq > 512); the caller then uses the dense path.  key_pre_rope / cos / sin of the new
+        positions are only needed when decode tokens are folded into the factors (compress_decode_tokens); the fold
+        runs at single-token steps only, since the tokens of a multi-token step may still be rejected (crop)."""
         layer = self._layer(layer_idx)
         st = layer.group
-        if st is None or st.factors.key is None or st.factors.value is None or query.shape[2] != 1:
+        if st is None or st.factors.key is None or st.factors.value is None:
+            return None
+        hq, tq = query.shape[1], query.shape[2]
+        h, d = st.heads, st.head_dim
+        if (hq // h) * tq > 64 or hq * tq > 512:
             return None
         fold = self.compress_decode_tokens and key_pre_rope is not None
         layer.append_tail(key, value, key_pre_rope if fold else None)
         if fold and layer_idx == st.layer_ids[0] and st.re_apply_rope and cos is not None:
-            st.tail_rope.append((cos.reshape(-1, cos.shape[-1])[-1].to(torch.bfloat16),
-                                 sin.reshape(-1, sin.shape[-1])[-1].to(torch.bfloat16)))
-        h, d = st.heads, st.head_dim
+            cs = cos.reshape(-1, cos.shape[-1])[-tq:].to(torch.bfloat16)
+            sn = sin.reshape(-1, sin.shape[-1])[-tq:].to(torch.bfloat16)
+            st.tail_rope.extend(zip(cs, sn))
         rows = slice(layer.index_in_group * h * d, (layer.index_in_group + 1) * h * d)
         fk, fv = st.factors.key, st.factors.value
-        need = ops.decode_workspace_bytes(query.shape[1], layer.prefill_len, layer.tail_len, fv.rank)
+        need = ops.decode_workspace_bytes(hq * tq, layer.prefill_len, layer.tail_len, fv.rank)
         if self._workspace is None or self._workspace.numel() < need:
             self._workspace = torch.empty(int(need * 1.25) + 4096, dtype=torch.uint8, device=query.device)
         n_tok = layer.prefill_len
         out = ops.decode_attention(
-            query[0, :, 0, :], fk.A_storage[:n_tok], fk.V[rows], fv.A_storage[:n_tok], fv.V[rows], h,
-            st.cos[:n_tok] if st.re_apply_rope else None, st.sin[:n_tok] if st.re_apply_rope else None,
+            query[0, :, 0, :] if tq == 1 else query[0], fk.A_storage[:n_tok], fk.V[rows], fv.A_storage[:n_tok], fv.V[rows],
+            h, st.cos[:n_tok] if st.re_apply_rope else None, st.sin[:n_tok] if st.re_apply_rope else None,
             layer.tail_k[0, :, : layer.tail_len], layer.tail_v[0, :, : layer.tail_len], scaling,
             workspace=self._workspace)
-        if fold and layer_idx == st.layer_ids[-1]:
+        if fold and tq == 1 and layer_idx == st.layer_ids[-1]:
             self._fold_tail(st)
-        return out[None, :, None, :]
+        return out[None, :, None, :] if tq == 1 else out[None]
 
     @torch.no_grad()
     def latent_slot(self, key: torch.Tensor, value: torch.Tensor, layer_idx: int) -> Optional[dict]:
@@ -392,15 +441,21 @@ class FakeLayerMergingCache(DynamicCache):
             l.tail_len = 0
             l.kpre_from = 0
 
-    # ------------------------------------------------------------------ unsupported cache surgery
+    # ------------------------------------------------------------------ cache surgery
+    def crop(self, max_length: int):
+        """Drop tokens from the end (assisted / speculative decoding rejects drafted tokens this way).  Compressed layers
+        lose tokens of their dense tail; cropping into a group's compressed tokens raises ``XkvError`` and leaves the
+        cache as it was, except right after the prefill (``_XkvLayer.check_crop``).  Un-grouped layers crop as
+        ``DynamicLayer`` does."""
+        for l in self.layers:
+            if getattr(l, "group", None) is not None:
+                l.check_crop(max_length)
+        return super().crop(max_length)
+
     def _refuse_if_compressed(self, what: str) -> None:
         if any(getattr(l, "group", None) is not None for l in self.layers):
-            raise XkvError(f"FakeLayerMergingCache.{what}: not supported once layer groups are factorised (the dense "
-                           "per-layer tensors no longer exist; beam search / cache cropping need the dense cache)")
-
-    def crop(self, max_length: int):
-        self._refuse_if_compressed("crop")
-        return super().crop(max_length)
+            raise XkvError(f"FakeLayerMergingCache.{what}: not supported once layer groups are factorised (beam search "
+                           "and batch > 1 need per-sample caches)")
 
     def batch_repeat_interleave(self, repeats: int):
         self._refuse_if_compressed("batch_repeat_interleave")

@@ -347,20 +347,28 @@ def decode_attention(q: torch.Tensor, a_k: torch.Tensor, vk_layer: torch.Tensor,
     V^ = A_v Vv_l^T never materialised.  q (Hq, D); a_k (S, rk); vk_layer (H*D, rk); a_v (S, rv);
     vv_layer (H*D, rv); cos/sin (S, D) or None; k_tail/v_tail (H, T, D) or None.  Returns (Hq, D) bf16.
     lse_out: optional (Hq,) fp32 tensor that receives log sum exp of the scaled scores over THIS call's tokens
-    (token-sharded contexts: see parallel.merge_token_shards)."""
+    (token-sharded contexts: see parallel.merge_token_shards).
+
+    Multi-token step: q (Hq, Tq, D) returns (Hq, Tq, D) and lse_out is (Hq, Tq).  The last Tq tail tokens are the
+    queries' own (T >= Tq) and query token t sees the prefix and tail tokens [0, T - Tq + t].  Bounds:
+    (Hq / H) * Tq <= 64 and Hq * Tq <= 512 (XkvError past them)."""
     _require_cuda(q, a_k, vk_layer, a_v, vv_layer, cos, sin, k_tail, v_tail, out, workspace)
-    if lse_out is not None and (not lse_out.is_cuda or lse_out.dtype != torch.float32 or lse_out.numel() < q.shape[0]
+    if q.dim() not in (2, 3):
+        raise _lib.XkvError("decode_attention: q must be (Hq, D) or (Hq, Tq, D)")
+    multi = q.dim() == 3
+    hq, d = q.shape[0], q.shape[-1]
+    tq = q.shape[1] if multi else 1
+    if lse_out is not None and (not lse_out.is_cuda or lse_out.dtype != torch.float32 or lse_out.numel() < hq * tq
                                 or not lse_out.is_contiguous()):
-        raise _lib.XkvError("decode_attention: lse_out must be a contiguous CUDA fp32 tensor of Hq elements")
-    hq, d = q.shape
+        raise _lib.XkvError("decode_attention: lse_out must be a contiguous CUDA fp32 tensor of Hq * Tq elements")
     s, rk = a_k.shape
     rv = a_v.shape[1]
     t = 0 if k_tail is None else k_tail.shape[1]
-    need = decode_workspace_bytes(hq, s, t, rv)
+    need = decode_workspace_bytes(hq * tq, s, t, rv)
     if workspace is None or workspace.numel() < need:
         workspace = torch.empty(need, dtype=torch.uint8, device=q.device)
     if out is None:
-        out = torch.empty(hq, d, dtype=torch.bfloat16, device=q.device)
+        out = torch.empty(*q.shape, dtype=torch.bfloat16, device=q.device)
     for name, x in (("q", q), ("a_k", a_k), ("vk_layer", vk_layer), ("a_v", a_v), ("vv_layer", vv_layer)):
         if x.dtype != torch.bfloat16 or x.stride(-1) != 1:
             raise _lib.XkvError(f"decode_attention: {name} must be bf16 with unit inner stride")
@@ -373,11 +381,15 @@ def decode_attention(q: torch.Tensor, a_k: torch.Tensor, vk_layer: torch.Tensor,
         if k_tail.stride() != v_tail.stride() or k_tail.stride(-1) != 1:
             raise _lib.XkvError("decode_attention: k_tail / v_tail must share strides, unit inner stride")
         sh, st = k_tail.stride(0), k_tail.stride(1)
-    check(_lib.load().xkv_decode_attention_lse(
-        _ptr(q), hq, num_kv_heads, d, _ptr(a_k), a_k.stride(0), rk, _ptr(vk_layer), vk_layer.stride(0),
-        _ptr(a_v), a_v.stride(0), rv, _ptr(vv_layer), vv_layer.stride(0), s, _ptr(cos), _ptr(sin),
-        cos.stride(0) if cos is not None else 0, _ptr(k_tail if t else None), _ptr(v_tail if t else None), t, sh, st,
-        C.c_float(scale), _ptr(out), C.c_void_p(workspace.data_ptr()), workspace.numel(), _stream(), _ptr(lse_out)))
+    lib = _lib.load()
+    args = (_ptr(a_k), a_k.stride(0), rk, _ptr(vk_layer), vk_layer.stride(0), _ptr(a_v), a_v.stride(0), rv,
+            _ptr(vv_layer), vv_layer.stride(0), s, _ptr(cos), _ptr(sin), cos.stride(0) if cos is not None else 0,
+            _ptr(k_tail if t else None), _ptr(v_tail if t else None), t, sh, st, C.c_float(scale), _ptr(out),
+            C.c_void_p(workspace.data_ptr()), workspace.numel(), _stream(), _ptr(lse_out))
+    if multi:
+        check(lib.xkv_decode_attention_multi(_ptr(q), hq, tq, num_kv_heads, d, *args))
+    else:
+        check(lib.xkv_decode_attention_lse(_ptr(q), hq, num_kv_heads, d, *args))
     return out
 
 

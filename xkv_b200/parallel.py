@@ -71,7 +71,8 @@ def merge_token_shards(out_local: torch.Tensor, lse_local: torch.Tensor, group=N
     """Decode over a token-sharded factored cache (SURVEY §8e): every rank has run
     ``ops.decode_attention(..., lse_out=lse_local)`` over ITS token rows of A_k / A_v (the decode tail lives on one rank,
     the others pass none); one all-gather of (Hq x (D + 1)) floats per layer and a local merge give every rank the
-    attention output over the whole context.  Returns (Hq, D) in out_local's dtype."""
+    attention output over the whole context.  Returns (Hq, D) in out_local's dtype.  The merge is per row, so a
+    multi-token step (q (Hq, Tq, D)) merges unchanged: pass its output and log-sum-exp as (Hq * Tq, D) and (Hq * Tq,)."""
     import torch.distributed as dist
 
     world = dist.get_world_size(group)
