@@ -182,73 +182,31 @@ XKV_API int xkv_sqrt_clamp(const float* in, float* out, int count, void* stream)
 
 /* ---- (2) the factorisation driver: replaces fake_svd (cache:11-29) for a batch ------------------
  * X[b] (m x n bf16, row stride ldx)  ~=  A[b] (m x rank bf16) * Vt[b] (rank x n bf16); V[b] (n x rank) is
- * Vt transposed (the layout the decode kernel reads). sigma[b] (optional) receives
- * xkv_factorize_sigma_count() leading singular-value estimates. Pure host code: enqueues the kernels
- * above on `stream`. stage_events_host (optional): 7 cudaEvent_t recorded at start / after the Gram
- * GEMM / Gram reduce+split / range finder / power iterations / Rayleigh-Ritz / projection.
- * Token-sharded use (rows of X split over GPUs): phase 1 writes each matrix's LOCAL Gram X_p^T X_p (n x n fp32,
- * symmetric) to gram_host[b] and returns; the caller all-reduces those buffers (NCCL) and calls again with
- * phase 2, which resumes from the reduced Gram and projects the local rows A_p = X_p V. phase 0 (gram_host may
- * be NULL) does everything on one device.  Phases 3 and 4 split phase 2 so that the small-matrix stages of different
- * matrices can run on different ranks: phase 3 derives Vt / V from gram_host[b] and stops (X_host / A_host may be NULL);
- * phase 4 only projects, A = X V, with the Vt the caller supplies (e.g. received from the rank that ran phase 3). */
-typedef struct xkv_factorize_options {
-  int32_t power_iters;    /* power steps on G after the range finder (default 4) */
-  int32_t oversample;     /* extra sketch columns; sketch width l = round_up(rank + oversample, 64) */
-  int32_t first_passes;   /* CholeskyQR passes after the range finder (2) */
-  int32_t passes;         /* CholeskyQR passes after a power step (2) */
-  int32_t final_passes;   /* CholeskyQR passes after the last power step (2) */
-  int32_t window;         /* Rayleigh-Ritz window width, <= 160 (default 128) */
-  int32_t jacobi_sweeps;
-  int32_t rayleigh_ritz;  /* 0: keep the first `rank` basis vectors as they are */
-  int32_t want_sigma;     /* also diagonalise the leading window to report singular values */
-  int32_t gram_split_k;
-  int32_t gram_chunk_tokens; /* the Gram is accumulated on the tensor core over pieces of this many tokens which are summed
-                              * in fp32 by the epilogue (xkv_gemm_problem.accum_phases); 0 = one piece (default 16384) */
-  int32_t small_split_k;
-  float shifts[4];        /* diagonal shift of CholeskyQR pass 0,1,2,3+ */
-  float pivot_floor;
-  float spectral_shift;   /* power steps after the first iterate with G - c I, c = spectral_shift * (estimate of lambda_l); 0 = off (0.5) */
-  int32_t shift_tail;     /* trailing entries of diag(R) of the previous step that estimate lambda_l (8) */
-  int32_t single_pass_from; /* power steps with index >= this (> 0) orthonormalise with ONE CholeskyQR pass (small shift, 6-term Gram); 0 = never */
-  int32_t single_pass_last; /* 1: the last power step may use the single pass too */
-  int32_t pass0_terms;      /* bf16-limb terms (3 or 6) of S = Y Y^T and Q = L^-1 Y in the heavily shifted first pass.  3 is only safe
-                             * when the rounding errors of the limbs are incoherent (energy spread over many columns); with a few
-                             * dominant channels they add up coherently to ~l * 2^-16 > the shift and the Cholesky breaks down
-                             * (default 6) */
-  int32_t heavy_redo;       /* 1 (default): a lightly shifted pass whose Cholesky met a pivot below twice its shift (the Gram of the
-                             * basis was numerically indefinite: extreme outlier channels) is redone ON DEVICE DECISION with the
-                             * heavy shift of pass 0 instead of producing NaN */
-  int32_t power_terms;      /* bf16-limb terms (3 or 6) of the power-step product Y = Q G (default 3) */
-  float second_pass_min_pivot; /* a single-pass step runs a second pass ON DEVICE DECISION for every matrix whose first
-                                * pass met a Cholesky pivot below this (ill-conditioned: steep spectrum at high rank);
-                                * 0 = never (default 0.05) */
-  int32_t solve_terms;      /* bf16-limb terms (3 or 6) of the triangular solve Q = L^-1 Y in every CholeskyQR pass whose result a
-                             * later pass or power step orthonormalises again (range finder, all power steps but the last); the
-                             * last power step always uses 6.  Unlike the Gram of the basis (pass0_terms) the solve cannot break
-                             * down: 3 terms (default) leave the intermediate bases orthonormal to ~1e-5 instead of ~1e-7 */
-  uint64_t seed;
-} xkv_factorize_options;
-XKV_API void xkv_factorize_default_options(xkv_factorize_options* opts);
-/* sizeof(xkv_factorize_options) of this build: foreign-language bindings can hold the options as an opaque, zeroed blob
- * of this many bytes filled in by xkv_factorize_default_options instead of mirroring the struct */
-XKV_API size_t xkv_factorize_options_size(void);
-XKV_API size_t xkv_factorize_workspace_bytes(int batch, int m, int n, int rank, const xkv_factorize_options* opts);
-XKV_API int xkv_factorize_sigma_count(int rank, const xkv_factorize_options* opts);
+ * Vt transposed (the layout the decode kernel reads). sigma[b] (optional) receives XKV_FACTORIZE_SIGMA_COUNT
+ * leading singular-value estimates. The sketch is round_up(rank + 64, 64) columns wide and must fit: 0 < rank <= m and
+ * round_up(rank + 64, 64) <= n. Pure host code: enqueues the kernels above on `stream`. stage_events_host (optional):
+ * 7 cudaEvent_t recorded at start / after the Gram GEMM / Gram reduce+split / range finder / power iterations /
+ * Rayleigh-Ritz / projection.
+ * phase 0 (gram_host may be NULL) does everything on one device.  Token-sharded use (rows of X split over GPUs) splits it
+ * in three: phase 1 writes each matrix's LOCAL Gram X_p^T X_p (n x n fp32, symmetric) to gram_host[b] and returns; the
+ * caller all-reduces those buffers; phase 3 derives Vt / V from the reduced gram_host[b] and stops (X_host / A_host may
+ * be NULL), so that the small-matrix stages of different matrices can run on different ranks; phase 4 only projects,
+ * A = X V, with the Vt the caller supplies (e.g. received from the rank that ran phase 3). */
+#define XKV_FACTORIZE_SIGMA_COUNT 128
+XKV_API size_t xkv_factorize_workspace_bytes(int batch, int m, int n, int rank);
 /* Same on a layer group's K (or V) tensors IN PLACE: matrix b is the column-wise concatenation of `layers` row-major
  * bf16 matrices layer_ptrs_host[b * layers + i] (m x layer_cols, row stride ld_layer) -- the reference's
  * torch.cat(dim=1) + transpose(1,2).reshape (cache:170-171, :13-14) when every layer tensor is a (1, H, S, D) view of
  * token-major memory (layer_cols = H * D).  The Gram pass and the projection pass read the layer tensors through
  * per-layer tensor maps: no gather kernel, no packed copy (1 GiB per group at config 2).  n = layers * layer_cols. */
 XKV_API int xkv_factorize_groups(const void* const* layer_ptrs_host, int batch, int layers, int layer_cols, int m,
-                                 int64_t ld_layer, int rank, const xkv_factorize_options* opts, void* const* A_host,
-                                 void* const* Vt_host, void* const* V_host, float* const* sigma_host, void* workspace,
-                                 size_t workspace_bytes, void* const* stage_events_host, void* stream);
+                                 int64_t ld_layer, int rank, void* const* A_host, void* const* Vt_host,
+                                 void* const* V_host, float* const* sigma_host, void* workspace, size_t workspace_bytes,
+                                 void* const* stage_events_host, void* stream);
 XKV_API int xkv_factorize_batch(const void* const* X_host, int batch, int m, int n, int64_t ldx, int rank,
-                                const xkv_factorize_options* opts, void* const* A_host, void* const* Vt_host,
-                                void* const* V_host, float* const* sigma_host, float* const* gram_host,
-                                int phase, void* workspace, size_t workspace_bytes,
-                                void* const* stage_events_host, void* stream);
+                                void* const* A_host, void* const* Vt_host, void* const* V_host,
+                                float* const* sigma_host, float* const* gram_host, int phase, void* workspace,
+                                size_t workspace_bytes, void* const* stage_events_host, void* stream);
 
 /* ---- (3) decode-time attention over the factored cache: replaces the SDPA call over dense K^/V^ --------
  * llama.py:58-69 with the reconstruction of cache:26-27 and the RoPE of cache:142-148 fused in.

@@ -82,7 +82,7 @@ def _worker(rank, world, port, ret):
         x = torch.randn(512, 64).bfloat16().float()        # the full matrix, identical on every rank
         b, e = parallel.token_shard(512, world, rank)
         g_local = x[b:e].t() @ x[b:e]                        # stand-in for the Gram kernel on the local rows
-        # as factorize_batch(process_group=...) does: only the packed upper triangle is reduced, then mirrored back
+        # as factorize_token_sharded does: only the packed upper triangle is reduced, then mirrored back
         packed = _pack_upper(g_local)
         dist.all_reduce(packed, op=dist.ReduceOp.SUM)
         g_local = _unpack_upper(packed, 64)

@@ -15,8 +15,7 @@ def main():
     rank = int(sys.argv[3]) if len(sys.argv) > 3 else 512
     n = 4096
     xs = [synthetic.group_matrix(S, n, 1.0, seed=b, device="cuda") for b in range(B)]
-    extra = json.loads(os.environ.get("XKV_OPTS", "{}"))   # e.g. XKV_OPTS='{"gram_chunk_tokens": 0}'
-    opts = factorize.FactorizeOptions(profile=True, **extra)
+    opts = factorize.FactorizeOptions(profile=True)
     for rep in range(2):
         torch.cuda.synchronize()
         l0 = ops.launch_count()
@@ -29,11 +28,10 @@ def main():
                           "launches": ops.launch_count() - l0, "stages_ms": fs[0].timings,
                           "sum_ms": sum(fs[0].timings.values())}))
     # un-profiled wall time with events around the whole call
-    opts = factorize.FactorizeOptions(**extra)
     for rep in range(3):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        fs = factorize.factorize_batch(xs, rank, opts)
+        fs = factorize.factorize_batch(xs, rank)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1)

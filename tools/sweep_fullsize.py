@@ -1,6 +1,5 @@
-"""Accuracy sweep of factorisation options at FULL size (64K x 4096 etc.) against the Eckart-Young optimum from the
-fp64 Gram (tests/test_fullsize_gpu.py).  Design aid, not a bench line.
-usage: python tools/sweep_fullsize.py '[{"power_iters": 5}, {"gram_split_k": 8}]'"""
+"""Accuracy of the factorisation at FULL size (64K x 4096 etc.) against the Eckart-Young optimum from the fp64 Gram
+(tests/test_fullsize_gpu.py).  Design aid, not a bench line."""
 import json
 import math
 import os
@@ -36,20 +35,17 @@ def rel_err(x, f):
 
 
 def main():
-    variants = json.loads(sys.argv[1]) if len(sys.argv) > 1 else [{}]
     data = []
     for (t, c, r, a) in CASES:
         x = synthetic.group_matrix(t, c, a, seed=4321, device="cuda")
         data.append((x, r, optimum(x, r)))
-    for v in variants:
-        opts = factorize.FactorizeOptions(**v)
-        row = []
-        for x, r, e_opt in data:
-            (f,) = factorize.factorize_batch([x], r, opts)
-            e = rel_err(x, f)
-            alg = math.sqrt(max(e * e - STORAGE ** 2, 0.0))
-            row.append((round(e / e_opt, 5), round(alg / e_opt, 5)))
-        print(json.dumps({"opts": v, "ratio_raw_and_algorithmic": row}), flush=True)
+    row = []
+    for x, r, e_opt in data:
+        (f,) = factorize.factorize_batch([x], r)
+        e = rel_err(x, f)
+        alg = math.sqrt(max(e * e - STORAGE ** 2, 0.0))
+        row.append((round(e / e_opt, 5), round(alg / e_opt, 5)))
+    print(json.dumps({"ratio_raw_and_algorithmic": row}), flush=True)
 
 
 if __name__ == "__main__":

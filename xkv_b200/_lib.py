@@ -16,6 +16,7 @@ _lib: Optional[C.CDLL] = None
 MAX_GROUP_LAYERS = 16
 MAX_GEMM_PROBLEMS = 16
 MAX_BATCH = 16
+FACTORIZE_SIGMA_COUNT = 128
 
 
 class XkvError(RuntimeError):
@@ -62,37 +63,6 @@ class AppendProblem(C.Structure):
                 ("lda", C.c_int64), ("n", C.c_int32), ("r", C.c_int32)]
 
 
-class FactorizeOptions(C.Structure):
-    """Mirror of ``xkv_factorize_options`` (include/xkv_b200.h)."""
-
-    _fields_ = [
-        ("power_iters", C.c_int32),
-        ("oversample", C.c_int32),
-        ("first_passes", C.c_int32),
-        ("passes", C.c_int32),
-        ("final_passes", C.c_int32),
-        ("window", C.c_int32),
-        ("jacobi_sweeps", C.c_int32),
-        ("rayleigh_ritz", C.c_int32),
-        ("want_sigma", C.c_int32),
-        ("gram_split_k", C.c_int32),
-        ("gram_chunk_tokens", C.c_int32),
-        ("small_split_k", C.c_int32),
-        ("shifts", C.c_float * 4),
-        ("pivot_floor", C.c_float),
-        ("spectral_shift", C.c_float),
-        ("shift_tail", C.c_int32),
-        ("single_pass_from", C.c_int32),
-        ("single_pass_last", C.c_int32),
-        ("pass0_terms", C.c_int32),
-        ("heavy_redo", C.c_int32),
-        ("power_terms", C.c_int32),
-        ("second_pass_min_pivot", C.c_float),
-        ("solve_terms", C.c_int32),
-        ("seed", C.c_uint64),
-    ]
-
-
 # name -> (restype, argtypes); every symbol include/xkv_b200.h declares must appear here
 _vp, _i, _i64, _f, _sz = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t
 _pp = C.POINTER(C.c_void_p)
@@ -116,7 +86,6 @@ SIGNATURES = {
     "xkv_shift_normalize_rows": (_i, [_pp, _pp, _vp, _pp, _i, _pp, _pp, _pp, _i, _i, _i, _i64, _i64, _vp]),
     "xkv_ritz_shift_update": (_i, [_pp, _i, _i, _i, _f, _vp, _vp]),
     "xkv_rdiag_update": (_i, [_pp, _pp, _i, _i, _i64, _vp]),
-    "xkv_factorize_options_size": (C.c_size_t, []),
     "xkv_pass_flags": (_i, [_pp, _i, _i, _i64, C.c_float, _vp, _vp]),
     "xkv_set_launch_predicate": (None, [_vp]),
     "xkv_cholesky_inverse": (_i, [_pp, _pp, _i, _i, _i64, _f, _f, _vp]),
@@ -124,9 +93,7 @@ SIGNATURES = {
     "xkv_jacobi_eigh": (_i, [_pp, _pp, _pp, _i, _i, _i64, _i64, _i, _vp]),
     "xkv_convert_bf16": (_i, [_vp, _i, _i, _i64, _vp, _i64, _vp, _i64, _vp]),
     "xkv_sqrt_clamp": (_i, [_vp, _vp, _i, _vp]),
-    "xkv_factorize_default_options": (None, [C.POINTER(FactorizeOptions)]),
-    "xkv_factorize_workspace_bytes": (_sz, [_i, _i, _i, _i, C.POINTER(FactorizeOptions)]),
-    "xkv_factorize_sigma_count": (_i, [_i, C.POINTER(FactorizeOptions)]),
+    "xkv_factorize_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "xkv_decode_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "xkv_decode_attention": (_i, [_vp, _i, _i, _i, _vp, _i64, _i, _vp, _i64, _vp, _i64, _i, _vp, _i64, _i, _vp, _vp, _i64,
                                   _vp, _vp, _i, _i64, _i64, _f, _vp, _vp, _sz, _vp]),
@@ -146,10 +113,8 @@ SIGNATURES = {
     "xkv_slerp_merge": (_i, [_vp, _vp, _i64, _i, _i64, _f, _f, _vp, _vp, _i64, _vp, _sz, _vp]),
     "xkv_gemm_problem_size": (C.c_size_t, []),
     "xkv_gemm_set_gram_pair": (None, [_i]),
-    "xkv_factorize_groups": (_i, [_pp, _i, _i, _i, _i, _i64, _i, C.POINTER(FactorizeOptions), _pp, _pp, _pp, _pp, _vp, _sz,
-                                  _pp, _vp]),
-    "xkv_factorize_batch": (_i, [_pp, _i, _i, _i, _i64, _i, C.POINTER(FactorizeOptions), _pp, _pp, _pp, _pp, _pp, _i,
-                                 _vp, _sz, _pp, _vp]),
+    "xkv_factorize_groups": (_i, [_pp, _i, _i, _i, _i, _i64, _i, _pp, _pp, _pp, _pp, _vp, _sz, _pp, _vp]),
+    "xkv_factorize_batch": (_i, [_pp, _i, _i, _i, _i64, _i, _pp, _pp, _pp, _pp, _pp, _i, _vp, _sz, _pp, _vp]),
 }
 
 

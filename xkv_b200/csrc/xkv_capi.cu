@@ -67,5 +67,5 @@ int encode_tmap_2d_bf16(CUtensorMap* map, const void* base, uint64_t inner, uint
 }  // namespace xkv
 
 extern "C" const char* xkv_last_error(void) { return xkv::error_buffer(); }
-extern "C" int xkv_version(void) { return 201; }
+extern "C" int xkv_version(void) { return 202; }
 extern "C" int64_t xkv_launch_count(void) { return xkv::g_launch_count.load(); }

@@ -33,13 +33,29 @@ struct Bump {
   void* bf16(size_t n) { return take(n * 2); }
 };
 
+// The schedule (DESIGN.md section 2, measured choices in section 8): sketch width l = round_up(rank + 64, 64); a Gaussian
+// range finder and 4 power steps on G; 2 CholeskyQR passes after the range finder and after the first step, one pass
+// plus a device-decided one after the spectrally shifted steps 1-3; then the Rayleigh-Ritz windows.
+constexpr int kOversample = 64;
+constexpr int kPowerSteps = 4;
+constexpr int kGramPieceTokens = 16384;   // tensor-core accumulation length of the Gram (xkv_gemm_problem.accum_phases)
+constexpr int kSmallSplitK = 8;
+constexpr int kWindow = 128;              // Rayleigh-Ritz window width (shared-memory Jacobi: even, <= 160)
+constexpr int kJacobiSweeps = 3;
+constexpr float kSpectralShift = 0.5f;    // c = 0.5 x (mean of the last kShiftTail entries of diag(R)) ~ lambda_l / 2
+constexpr int kShiftTail = 8;
+constexpr float kCholShift[3] = {3e-4f, 1e-6f, 1e-7f};   // diagonal shift of CholeskyQR pass index 0 / 1 / 2
+constexpr float kPivotFloor = 1e-12f;
+constexpr float kSecondPassMinPivot = 0.05f;
+constexpr uint64_t kSeed = 1234;
+static_assert(kWindow == XKV_FACTORIZE_SIGMA_COUNT, "the leading window gives the singular values");
+
 struct Plan {
-  int B, m, n, W, nw, sk, skw, gs;
-  bool rr;
-  // rank r, sketch width l = round_up(r + oversample, 64), Rayleigh-Ritz window [r0, r0 + W) with wl kept columns on
-  // its left of column r and wr = l - r discarded ones on its right
-  int r, l, wl, wr, r0;
-  // per-matrix buffers
+  int B, m, n, sk, skw;
+  // rank r and sketch width l; the Rayleigh-Ritz window is rows [l - kWindow, l) of the basis, of which the
+  // r - (l - kWindow) rows left of row r are kept
+  int r, l;
+  // per-matrix buffers; window 0 straddles row r, window 1 is rows [0, kWindow) (the leading singular values)
   void* g_limb[XKV_MAX_BATCH][3];
   float* f_a[XKV_MAX_BATCH];
   float* f_b[XKV_MAX_BATCH];
@@ -59,47 +75,27 @@ struct Plan {
   float* wt[XKV_MAX_BATCH];
   void* wsel_l[XKV_MAX_BATCH][3];
   // shared
-  float* gram_slabs;  // [B][gs][n][n]
+  float* gram_slabs;  // [B][n][n]
   float* shift_dev;   // [B] spectral shifts of the current power step
   int* pass_flags;    // [B] device decision: this matrix needs a second CholeskyQR pass in the current step
   int* redo_flags;    // [B] device decision: the lightly shifted Cholesky of this matrix broke down, redo it heavily shifted
   size_t bytes;
 };
 
-static int make_plan(Plan& P, Bump& bump, int B, int m, int n, int rank, const xkv_factorize_options& o) {
+static int make_plan(Plan& P, Bump& bump, int B, int m, int n, int rank) {
   XKV_REQUIRE(B >= 1 && B <= XKV_MAX_BATCH, "factorize: batch %d out of range (1..%d)", B, XKV_MAX_BATCH);
   XKV_REQUIRE(n % 8 == 0, "factorize: n=%d must be a multiple of 8", n);
   P.B = B;
   P.m = m;
   P.n = n;
-  P.gs = o.gram_split_k < 1 ? 1 : o.gram_split_k;
   const int nkb = (n + 63) / 64;
-  P.sk = o.small_split_k < 1 ? 1 : (o.small_split_k > nkb ? nkb : o.small_split_k);
+  P.sk = nkb < kSmallSplitK ? nkb : kSmallSplitK;
   P.skw = nkb < 16 ? nkb : 16;
   P.r = rank;
-  P.l = round_up_int(rank + o.oversample, 64);
+  P.l = round_up_int(rank + kOversample, 64);   // >= 128 = kWindow for every rank >= 1
   XKV_REQUIRE(rank > 0 && rank <= m && P.l <= n, "factorize: rank %d (sketch %d) does not fit a %d x %d matrix", rank, P.l, m,
               n);
-  P.wr = P.l - rank;
-  // Rayleigh-Ritz window [r0, r0 + W) straddling column r: wl = W - wr columns of it are kept
-  int W = o.window < P.l ? o.window : P.l;
-  if (W > 160) W = 160;
-  W -= W % 2;
-  P.rr = o.rayleigh_ritz != 0;
-  int wl = W - P.wr;
-  if (wl > rank) wl = rank;
-  int Wb = wl + P.wr;
-  if (wl > 0 && (Wb % 2)) {
-    --wl;
-    --Wb;
-  }
-  if (wl <= 0) P.rr = false;
-  P.wl = wl;
-  P.r0 = rank - wl;
-  P.W = P.rr ? Wb : W;
-  P.nw = P.rr ? (o.want_sigma ? 2 : 1) : 0;
-  const size_t nn = n, l = P.l;
-  W = P.W;
+  const size_t nn = n, l = P.l, W = kWindow;
   for (int b = 0; b < B; ++b) {
     for (int i = 0; i < 3; ++i) P.g_limb[b][i] = bump.bf16(nn * nn);
     P.f_a[b] = bump.f32(l * nn);
@@ -112,19 +108,17 @@ static int make_plan(Plan& P, Bump& bump, int B, int m, int n, int rank, const x
     P.linv[b] = bump.f32(l * l);
     P.rdiag[b] = bump.f32(l);
     for (int i = 0; i < 3; ++i) P.linv_l[b][i] = bump.bf16(l * l);
-    for (int w = 0; w < P.nw; ++w) {
-      P.yw[b][w] = bump.f32(static_cast<size_t>(W) * nn);
-      for (int i = 0; i < 3; ++i) P.yw_l[b][w][i] = bump.bf16(static_cast<size_t>(W) * nn);
+    for (int w = 0; w < 2; ++w) {
+      P.yw[b][w] = bump.f32(W * nn);
+      for (int i = 0; i < 3; ++i) P.yw_l[b][w][i] = bump.bf16(W * nn);
       P.t_slabs[b][w] = bump.f32(static_cast<size_t>(P.skw) * W * W);
-      P.t_mat[b][w] = bump.f32(static_cast<size_t>(W) * W);
+      P.t_mat[b][w] = bump.f32(W * W);
       P.evals[b][w] = bump.f32(W);
     }
-    if (P.rr) {
-      P.wt[b] = bump.f32(static_cast<size_t>(W) * W);
-      for (int i = 0; i < 3; ++i) P.wsel_l[b][i] = bump.bf16(static_cast<size_t>(W) * W);
-    }
+    P.wt[b] = bump.f32(W * W);
+    for (int i = 0; i < 3; ++i) P.wsel_l[b][i] = bump.bf16(W * W);
   }
-  P.gram_slabs = bump.f32(static_cast<size_t>(B) * P.gs * nn * nn);
+  P.gram_slabs = bump.f32(static_cast<size_t>(B) * nn * nn);
   P.shift_dev = bump.f32(XKV_MAX_BATCH);
   P.pass_flags = reinterpret_cast<int*>(bump.f32(XKV_MAX_BATCH));
   P.redo_flags = reinterpret_cast<int*>(bump.f32(XKV_MAX_BATCH));
@@ -213,88 +207,31 @@ static inline const __nv_bfloat16* row_bf16(const void* base, long long row, lon
 
 using namespace xkv;
 
-extern "C" void xkv_factorize_default_options(xkv_factorize_options* o) {
-  if (!o) return;
-  std::memset(o, 0, sizeof(*o));
-  o->power_iters = 4;
-  o->spectral_shift = 0.5f;
-  o->shift_tail = 8;
-  o->single_pass_from = 1;
-  o->single_pass_last = 1;
-  o->second_pass_min_pivot = 0.05f;
-  o->pass0_terms = 6;
-  o->power_terms = 3;
-  o->heavy_redo = 1;
-  o->solve_terms = 3;
-  o->oversample = 64;
-  o->first_passes = 2;
-  o->passes = 2;
-  o->final_passes = 2;
-  o->window = 128;
-  o->jacobi_sweeps = 3;
-  o->rayleigh_ritz = 1;
-  o->want_sigma = 1;
-  o->gram_split_k = 1;
-  o->gram_chunk_tokens = 16384;
-  o->small_split_k = 8;
-  o->shifts[0] = 3e-4f;
-  o->shifts[1] = 1e-6f;
-  o->shifts[2] = 1e-7f;
-  o->shifts[3] = 1e-7f;
-  o->pivot_floor = 1e-12f;
-  o->seed = 1234;
-}
-
-extern "C" size_t xkv_factorize_options_size(void) { return sizeof(xkv_factorize_options); }
-
-extern "C" size_t xkv_factorize_workspace_bytes(int batch, int m, int n, int rank, const xkv_factorize_options* opts) {
-  xkv_factorize_options o;
-  if (opts)
-    o = *opts;
-  else
-    xkv_factorize_default_options(&o);
+extern "C" size_t xkv_factorize_workspace_bytes(int batch, int m, int n, int rank) {
   Plan P;
   Bump bump{nullptr, 0, 0, false};
-  if (batch < 1 || batch > XKV_MAX_BATCH || make_plan(P, bump, batch, m, n, rank, o)) return 0;
+  if (batch < 1 || batch > XKV_MAX_BATCH || make_plan(P, bump, batch, m, n, rank)) return 0;
   return P.bytes;
-}
-
-extern "C" int xkv_factorize_sigma_count(int rank, const xkv_factorize_options* opts) {
-  xkv_factorize_options o;
-  if (opts)
-    o = *opts;
-  else
-    xkv_factorize_default_options(&o);
-  Plan P;
-  Bump bump{nullptr, 0, 0, false};
-  // m, n large enough not to trip the fit check: only the window arithmetic matters here
-  if (make_plan(P, bump, 1, 1 << 20, 1 << 20, rank, o)) return 0;
-  return (P.rr && o.want_sigma) ? P.W : 0;
 }
 
 // X_host: packed matrices (layers == 0) or per-layer pointers [batch][layers] read in place
 static int factorize_impl(const void* const* X_host, int layers, int layer_cols, int batch, int m, int n, int64_t ldx,
-                          int rank, const xkv_factorize_options* opts, void* const* A_host, void* const* Vt_host,
-                          void* const* V_host, float* const* sigma_host, float* const* gram_host, int phase,
-                          void* workspace, size_t workspace_bytes, void* const* stage_events_host, void* stream) {
-  xkv_factorize_options o;
-  if (opts)
-    o = *opts;
-  else
-    xkv_factorize_default_options(&o);
-  XKV_REQUIRE(phase >= 0 && phase <= 4,
-              "factorize: phase must be 0 (all), 1 (Gram only), 2 (resume from Gram), 3 (right factor from Gram) or 4 (projection)");
+                          int rank, void* const* A_host, void* const* Vt_host, void* const* V_host,
+                          float* const* sigma_host, float* const* gram_host, int phase, void* workspace,
+                          size_t workspace_bytes, void* const* stage_events_host, void* stream) {
+  XKV_REQUIRE(phase == 0 || phase == 1 || phase == 3 || phase == 4,
+              "factorize: phase must be 0 (all), 1 (Gram only), 3 (right factor from Gram) or 4 (projection)");
   XKV_REQUIRE(workspace && Vt_host && (phase == 1 || phase == 4 || V_host) && (phase == 3 || X_host) &&
                   (phase == 1 || phase == 3 || A_host),
               "factorize: null argument");
-  XKV_REQUIRE(phase == 0 || phase == 4 || gram_host != nullptr, "factorize: phases 1 / 2 / 3 need the per-matrix Gram buffers");
+  XKV_REQUIRE(phase == 0 || phase == 4 || gram_host != nullptr, "factorize: phases 1 / 3 need the per-matrix Gram buffers");
   static thread_local Plan P;
   Bump bump{static_cast<char*>(workspace), 0, workspace_bytes, false};
-  XKV_TRY(make_plan(P, bump, batch, m, n, rank, o));
+  XKV_TRY(make_plan(P, bump, batch, m, n, rank));
   XKV_REQUIRE(!bump.overflow && P.bytes <= workspace_bytes, "factorize: workspace too small (%zu < %zu bytes)",
               workspace_bytes, P.bytes);
   XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "factorize: workspace must be 256-byte aligned");
-  const int B = batch, W = P.W, l = P.l, r = P.r;
+  const int B = batch, W = kWindow, l = P.l, r = P.r;
   const long long nn = n;
   cudaStream_t st = as_stream(stream);
   int ev = 0;
@@ -327,48 +264,43 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   if (phase == 4) return project();
 
   // ---- 1. Gram matrices and their bf16 limbs ----
-  // phase 1 stops after the (local) Gram so that token-sharded callers can all-reduce it; phase 2 resumes
+  // phase 1 stops after the (local) Gram so that token-sharded callers can all-reduce it; phase 3 resumes
   // from the caller's reduced Gram.
-  if (phase != 2 && phase != 3) {
+  if (phase != 3) {
     for (int b = 0; b < B; ++b) {
       const void* x0 = layers > 0 ? X_host[static_cast<size_t>(b) * layers] : X_host[b];
       xkv_gemm_problem p = problem(x0, nullptr, nullptr, ldx, 1, x0, nullptr, nullptr, ldx, 1,
-                                   P.gram_slabs + static_cast<size_t>(b) * P.gs * nn * nn, nn, n, n, m, 1);
+                                   P.gram_slabs + static_cast<size_t>(b) * nn * nn, nn, n, n, m, 1);
       if (layers > 0) {   // both operands are the group's layer tensors, read in place
         p.a_layers = p.b_layers = layers;
         p.layer_cols = layer_cols;
         for (int i = 0; i < layers; ++i) p.A_layer[i] = p.B_layer[i] = X_host[static_cast<size_t>(b) * layers + i];
       }
       p.sym_upper = 1;
-      p.split_k = P.gs;
-      p.split_stride = nn * nn;
-      if (o.gram_chunk_tokens > 0) {
-        const int per_split = (m + P.gs - 1) / P.gs;
-        const int ph = (per_split + o.gram_chunk_tokens - 1) / o.gram_chunk_tokens;
-        p.accum_phases = ph > 64 ? 64 : ph;
-      }
+      const int ph = (m + kGramPieceTokens - 1) / kGramPieceTokens;
+      p.accum_phases = ph > 64 ? 64 : ph;
       ps.push_back(p);
     }
     XKV_TRY(run_gemms(ps, stream, layers > 0 ? XKV_MAX_LAYER_MAPS / layers : XKV_MAX_GEMM_PROBLEMS));
   }
   XKV_TRY(mark());  // 1: Gram GEMM (the dominant kernel, timed on its own for the roofline)
   if (phase == 0) {
-    // slabs -> symmetric bf16 limbs in one pass (no fp32 Gram round trip)
+    // upper-triangle tiles -> symmetric bf16 limbs in one pass (no fp32 Gram round trip)
     const float* sl[XKV_MAX_BATCH];
     void *h0[XKV_MAX_BATCH], *h1[XKV_MAX_BATCH], *h2[XKV_MAX_BATCH];
     for (int b = 0; b < B; ++b) {
-      sl[b] = P.gram_slabs + static_cast<size_t>(b) * P.gs * nn * nn;
+      sl[b] = P.gram_slabs + static_cast<size_t>(b) * nn * nn;
       h0[b] = P.g_limb[b][0], h1[b] = P.g_limb[b][1], h2[b] = P.g_limb[b][2];
     }
-    XKV_TRY(xkv_symmetrize_split_bf16(sl, B, P.gs, nn * nn, n, nn, h0, h1, h2, nn, stream));
+    XKV_TRY(xkv_symmetrize_split_bf16(sl, B, 1, nn * nn, n, nn, h0, h1, h2, nn, stream));
   } else {
     for (int b = 0; b < B; ++b) {
       float* g = gram_host[b];
       XKV_REQUIRE(g != nullptr, "factorize: null Gram buffer %d", b);
-      if (phase != 2 && phase != 3)
-        XKV_TRY(xkv_reduce_slabs(P.gram_slabs + static_cast<size_t>(b) * P.gs * nn * nn, P.gs, nn * nn, n, n, nn, 1, g, nn,
-                                 stream));
-      if (phase != 1) XKV_TRY(xkv_split_bf16(g, n, n, nn, P.g_limb[b][0], P.g_limb[b][1], P.g_limb[b][2], nn, stream));
+      if (phase == 1)
+        XKV_TRY(xkv_reduce_slabs(P.gram_slabs + static_cast<size_t>(b) * nn * nn, 1, nn * nn, n, n, nn, 1, g, nn, stream));
+      else
+        XKV_TRY(xkv_split_bf16(g, n, n, nn, P.g_limb[b][0], P.g_limb[b][1], P.g_limb[b][2], nn, stream));
     }
   }
   XKV_TRY(mark());  // 2: Gram reduce + limb split
@@ -381,32 +313,33 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
     cur = nxt;
     nxt = t;
   };
-  // cur <- orth(cur): row-normalised, shifted CholeskyQR
-  // With `shifted`, cur = Q_prev G and nxt still holds Q_prev: the first pass first forms Q_prev (G - c I).
+  // cur <- orth(cur): row-normalised, shifted CholeskyQR in two passes.  The pass index selects the diagonal shift of
+  // the Cholesky (kCholShift); every pass with index > 0 redoes a broken-down Cholesky heavily shifted (device decision).
+  // Not `shifted` (range finder, first power step): passes 0 and 1, the first one heavily shifted for the raw sketch.
+  // `shifted` (power steps 1-3): cur = Q_prev G and nxt still holds Q_prev, so the first pass (index 1) first forms
+  // Q_prev (G - c I).  The basis entering such a step is orthonormal and ordered by dominance, so this one pass is enough
+  // unless its Cholesky met a pivot below kSecondPassMinPivot: the device decides per matrix (xkv_pass_flags) whether
+  // the second pass (index 2) runs; its kernels are always enqueued and exit at once for the matrices that do not need
+  // it.  That pass writes its result over `cur` (its operands are the limb copies), so the buffers are where the
+  // following stages expect them either way.
   // With `track`, diag(R) of the step is accumulated in P.rdiag (row norms x Cholesky diagonals).
-  // `conditional_extra`: after the npass passes the device decides per matrix (xkv_pass_flags on the last pass's
-  // Cholesky pivots) whether one more pass runs; its kernels are always enqueued and exit at once for the matrices
-  // that do not need it.  That pass writes its result over `cur` (its operands are the limb copies), so the
-  // buffers are where the following stages expect them either way.
   // `final_call`: nothing orthonormalises the result again (the last power step): the solve keeps all 6 limb terms
-  auto cholqr = [&](int npass, bool shifted, bool track, int p0, bool conditional_extra, bool final_call) -> int {
-    const int total = npass + (conditional_extra ? 1 : 0);
-    for (int ip = 0; ip < total; ++ip) {
-      const int pp = ip + p0;  // index into the per-pass parameters (shift, limb terms)
-      const bool cond = conditional_extra && ip == npass;
+  auto cholqr = [&](bool shifted, bool track, bool final_call) -> int {
+    const int first = shifted ? 1 : 0;
+    for (int pp = first; pp <= first + 1; ++pp) {
+      const bool cond = shifted && pp == 2;
       if (cond) {
-        XKV_TRY(xkv_pass_flags(P.linv, B, l, l, o.second_pass_min_pivot, P.pass_flags, stream));
+        XKV_TRY(xkv_pass_flags(P.linv, B, l, l, kSecondPassMinPivot, P.pass_flags, stream));
         xkv_set_launch_predicate(P.pass_flags);
       }
       int rc = [&]() -> int {
-        XKV_TRY(xkv_shift_normalize_rows(cur, (ip == 0 && shifted) ? nxt : nullptr, P.shift_dev, track ? P.rdiag : nullptr,
-                                         ip == 0, P.lh, P.lm, P.ll, B, l, n, nn, nn, stream));
-        // pass 0 is regularised by a 3e-4 shift; a 3-term product (error ~1e-5 per entry) is accurate enough there
-        // only if those errors are incoherent -- see xkv_factorize_options.pass0_terms
-        const int nt = (pp == 0 && o.pass0_terms == 3) ? 3 : 6;
+        XKV_TRY(xkv_shift_normalize_rows(cur, (pp == first && shifted) ? nxt : nullptr, P.shift_dev,
+                                         track ? P.rdiag : nullptr, pp == first, P.lh, P.lm, P.ll, B, l, n, nn, nn, stream));
+        // S = Y Y^T with all 6 limb terms: with a few dominant channels the rounding errors of 3 terms add up
+        // coherently above the shift and the Cholesky breaks down (DESIGN.md section 2)
         for (int b = 0; b < B; ++b) {
           xkv_gemm_problem p = problem(P.lh[b], P.lm[b], P.ll[b], nn, 0, P.lh[b], P.lm[b], P.ll[b], nn, 0, P.s_slabs[b],
-                                       l, l, l, n, nt);
+                                       l, l, l, n, 6);
           p.sym_upper = 1;
           p.split_k = P.sk;
           p.split_stride = static_cast<long long>(l) * l;
@@ -418,10 +351,9 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
         {
           void *h0[XKV_MAX_BATCH], *h1[XKV_MAX_BATCH], *h2[XKV_MAX_BATCH];
           for (int b = 0; b < B; ++b) h0[b] = P.linv_l[b][0], h1[b] = P.linv_l[b][1], h2[b] = P.linv_l[b][2];
-          const float shift = o.shifts[pp < 3 ? pp : 3];
-          XKV_TRY(xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, nt > 3 ? h2 : nullptr, B, l, l, l, shift, o.pivot_floor,
-                                             stream));
-          if (o.heavy_redo && pp > 0 && shift < o.shifts[0]) {
+          const float shift = kCholShift[pp];
+          XKV_TRY(xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, h2, B, l, l, l, shift, kPivotFloor, stream));
+          if (pp > 0) {
             // A pivot below twice the shift means the fp32 Gram of the basis was numerically indefinite (the pass before
             // left it too ill-conditioned: extreme outlier channels).  Such matrices redo the Cholesky with the heavy
             // shift of pass 0 -- the slabs still hold S -- which costs orthogonality (later passes restore it) but never
@@ -430,8 +362,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
             xkv_set_launch_predicate(P.redo_flags);
             int rc2 = xkv_reduce_slabs_batched(P.s_slabs, P.s_mat, B, P.sk, static_cast<long long>(l) * l, l, l, l, 1, l, stream);
             if (!rc2)
-              rc2 = xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, nt > 3 ? h2 : nullptr, B, l, l, l, o.shifts[0],
-                                               o.pivot_floor, stream);
+              rc2 = xkv_cholesky_inverse_limbs(P.s_mat, P.linv, h0, h1, h2, B, l, l, l, kCholShift[0], kPivotFloor, stream);
             xkv_set_launch_predicate(cond ? P.pass_flags : nullptr);
             if (rc2) return rc2;
           }
@@ -439,11 +370,11 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
         if (track) XKV_TRY(xkv_rdiag_update(P.rdiag, P.linv, B, l, l, stream));
         // Q = Linv Y, computed as Q^T = Y^T Linv^T with the result stored transposed (same memory, same order of products):
         // the long dimension n becomes M, the sketch width l becomes N, which the CTA-pair GEMM tiles without padding
-        // (l = 576 as 3 x 192 columns, 832 as 4 x 208)
+        // (l = 576 as 3 x 192 columns, 832 as 4 x 208).  A basis that is orthonormalised again later needs only the
+        // 3 leading limb terms (orthonormal to ~1e-5 instead of ~1e-7; a product cannot break down).
         for (int b = 0; b < B; ++b) {
           xkv_gemm_problem p = swap_roles(problem(P.linv_l[b][0], P.linv_l[b][1], P.linv_l[b][2], l, 0, P.lh[b], P.lm[b],
-                                                  P.ll[b], nn, 1, cond ? cur[b] : nxt[b], nn, l, n, l,
-                                                  (o.solve_terms == 3 && !final_call) ? 3 : nt));
+                                                  P.ll[b], nn, 1, cond ? cur[b] : nxt[b], nn, l, n, l, final_call ? 6 : 3));
           p.run_if = cond ? P.pass_flags + b : nullptr;
           ps.push_back(p);
         }
@@ -467,41 +398,33 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
   };
 
   // ---- 2-3. Gaussian range finder ----
-  for (int b = 0; b < B; ++b) XKV_TRY(xkv_fill_gaussian_bf16(P.lh[b], l, n, nn, o.seed + 7919ull * b, stream));
+  for (int b = 0; b < B; ++b) XKV_TRY(xkv_fill_gaussian_bf16(P.lh[b], l, n, nn, kSeed + 7919ull * b, stream));
   XKV_TRY(apply_gram(1));
-  XKV_TRY(cholqr(o.first_passes, false, false, 0, false, o.power_iters == 0));
+  XKV_TRY(cholqr(false, false, false));
   XKV_TRY(mark());  // 3: range finder
 
-  // ---- 4. power steps ----
+  // ---- 4. power steps (3-term limb products) ----
   // The first step is plain (the range finder's triangular factor says nothing about eigenvalues); from the
-  // second step on the shift c = spectral_shift * lambda_l comes from diag(R) of the step before.
-  const bool use_shift = o.spectral_shift > 0.f && o.shift_tail > 0 && o.power_iters > 1;
-  if (use_shift) XKV_CHECK_CUDA(cudaMemsetAsync(P.shift_dev, 0, XKV_MAX_BATCH * sizeof(float), st));
-  for (int it = 0; it < o.power_iters; ++it) {
-    const int pterms = o.power_terms == 6 ? 6 : 3;
-    XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, pterms == 6 ? P.ll : nullptr, B, l, n, nn, nn, stream));
-    XKV_TRY(apply_gram(pterms));
-    const bool shifted = use_shift && it > 0;
-    if (shifted)
-      XKV_TRY(xkv_ritz_shift_update(P.rdiag, B, l, o.shift_tail < l ? o.shift_tail : l, o.spectral_shift, P.shift_dev, stream));
-    // From step `single_pass_from` on the basis entering the step is orthonormal to ~1e-5 and ordered by dominance,
-    // so the row-normalised product is well conditioned: ONE pass with the second pass's parameters (small shift,
-    // 6-term Gram) orthonormalises it; the first, heavily shifted pass is only needed while the sketch is raw.
-    const bool last = it == o.power_iters - 1;
-    const bool single = o.single_pass_from > 0 && it >= o.single_pass_from && !(last && o.final_passes > 1 && o.single_pass_last == 0);
-    XKV_TRY(cholqr(single ? 1 : (last ? o.final_passes : o.passes), shifted, use_shift && it + 1 < o.power_iters,
-                   single ? 1 : 0, single && o.second_pass_min_pivot > 0.f, last));
+  // second step on the shift c = kSpectralShift * lambda_l comes from diag(R) of the step before.
+  XKV_CHECK_CUDA(cudaMemsetAsync(P.shift_dev, 0, XKV_MAX_BATCH * sizeof(float), st));
+  for (int it = 0; it < kPowerSteps; ++it) {
+    XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, nullptr, B, l, n, nn, nn, stream));
+    XKV_TRY(apply_gram(3));
+    if (it > 0) XKV_TRY(xkv_ritz_shift_update(P.rdiag, B, l, kShiftTail, kSpectralShift, P.shift_dev, stream));
+    const bool last = it == kPowerSteps - 1;
+    XKV_TRY(cholqr(it > 0, !last, last));
   }
   XKV_TRY(mark());  // 4: power iterations
 
   // ---- 5. windowed Rayleigh-Ritz ----
-  if (P.rr) {
-    const int nw = P.nw;
-    const int r0 = P.r0, wl = P.wl;
+  // window 0: basis rows [r0, l) straddling row r, whose top wl Ritz vectors replace rows [r0, r); window 1: rows
+  // [0, W), diagonalised for the leading singular values
+  {
+    const int r0 = l - W, wl = r - r0;
     auto w0 = [&](int w) { return w == 0 ? r0 : 0; };   // first basis row of window w
     XKV_TRY(xkv_split_bf16_batched(cur, P.lh, P.lm, P.ll, B, l, n, nn, nn, stream));
     for (int b = 0; b < B; ++b)
-      for (int w = 0; w < nw; ++w)
+      for (int w = 0; w < 2; ++w)
         ps.push_back(swap_roles(problem(row_bf16(P.lh[b], w0(w), nn), row_bf16(P.lm[b], w0(w), nn),
                                         row_bf16(P.ll[b], w0(w), nn), nn, 0, P.g_limb[b][0], P.g_limb[b][1], P.g_limb[b][2],
                                         nn, 0, P.yw[b][w], nn, W, n, n, 6)));   // as (G Qw^T)^T: M = n in CTA pairs, N = W
@@ -512,7 +435,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
       void *h0[2 * XKV_MAX_BATCH], *h1[2 * XKV_MAX_BATCH], *h2[2 * XKV_MAX_BATCH];
       int cntw = 0;
       for (int b = 0; b < B; ++b)
-        for (int w = 0; w < nw; ++w) {
+        for (int w = 0; w < 2; ++w) {
           xs[cntw] = P.yw[b][w];
           h0[cntw] = P.yw_l[b][w][0], h1[cntw] = P.yw_l[b][w][1], h2[cntw] = P.yw_l[b][w][2];
           ++cntw;
@@ -523,7 +446,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
       }
     }
     for (int b = 0; b < B; ++b)
-      for (int w = 0; w < nw; ++w) {
+      for (int w = 0; w < 2; ++w) {
         xkv_gemm_problem p =
             problem(row_bf16(P.lh[b], w0(w), nn), row_bf16(P.lm[b], w0(w), nn), row_bf16(P.ll[b], w0(w), nn), nn, 0,
                     P.yw_l[b][w][0], P.yw_l[b][w][1], P.yw_l[b][w][2], nn, 0, P.t_slabs[b][w], W, W, W, n, 6);
@@ -539,7 +462,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
     float* wptr[2 * XKV_MAX_BATCH];
     int cnt = 0;
     for (int b = 0; b < B; ++b)
-      for (int w = 0; w < nw; ++w) {
+      for (int w = 0; w < 2; ++w) {
         sptr[cnt] = P.t_slabs[b][w];
         toutp[cnt] = P.t_mat[b][w];
         tptr[cnt] = P.t_mat[b][w];
@@ -551,7 +474,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
       const int c = cnt - lo < XKV_MAX_BATCH ? cnt - lo : XKV_MAX_BATCH;
       XKV_TRY(xkv_reduce_slabs_batched(sptr + lo, toutp + lo, c, P.skw, static_cast<long long>(W) * W, W, W, W, 0, W, stream));
     }
-    XKV_TRY(xkv_jacobi_eigh(tptr, eptr, wptr, cnt, W, W, W, o.jacobi_sweeps, stream));
+    XKV_TRY(xkv_jacobi_eigh(tptr, eptr, wptr, cnt, W, W, W, kJacobiSweeps, stream));
     // rows [r0, r) of the basis <- top-wl Ritz vectors of the window: Vw = Wsel * Qw
     {
       const float* xs[XKV_MAX_BATCH];
@@ -567,7 +490,7 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
                            row_bf16(P.lm[b], r0, nn), row_bf16(P.ll[b], r0, nn), nn, 1,
                            cur[b] + static_cast<size_t>(r0) * nn, nn, wl, n, W, 6));
     XKV_TRY(run_gemms(ps, stream));
-    if (o.want_sigma && sigma_host)
+    if (sigma_host)
       for (int b = 0; b < B; ++b)
         if (sigma_host[b]) XKV_TRY(xkv_sqrt_clamp(P.evals[b][1], sigma_host[b], W, stream));
   }
@@ -582,11 +505,10 @@ static int factorize_impl(const void* const* X_host, int layers, int layer_cols,
 }
 
 extern "C" int xkv_factorize_batch(const void* const* X_host, int batch, int m, int n, int64_t ldx, int rank,
-                                   const xkv_factorize_options* opts, void* const* A_host, void* const* Vt_host,
-                                   void* const* V_host, float* const* sigma_host, float* const* gram_host,
-                                   int phase, void* workspace, size_t workspace_bytes,
-                                   void* const* stage_events_host, void* stream) {
-  return factorize_impl(X_host, 0, 0, batch, m, n, ldx, rank, opts, A_host, Vt_host, V_host, sigma_host, gram_host, phase,
+                                   void* const* A_host, void* const* Vt_host, void* const* V_host,
+                                   float* const* sigma_host, float* const* gram_host, int phase, void* workspace,
+                                   size_t workspace_bytes, void* const* stage_events_host, void* stream) {
+  return factorize_impl(X_host, 0, 0, batch, m, n, ldx, rank, A_host, Vt_host, V_host, sigma_host, gram_host, phase,
                         workspace, workspace_bytes, stage_events_host, stream);
 }
 
@@ -598,10 +520,10 @@ static int check_layers(int layers, int layer_cols, int64_t ld_layer) {
 }
 
 extern "C" int xkv_factorize_groups(const void* const* layer_ptrs_host, int batch, int layers, int layer_cols, int m,
-                                    int64_t ld_layer, int rank, const xkv_factorize_options* opts, void* const* A_host,
+                                    int64_t ld_layer, int rank, void* const* A_host,
                                     void* const* Vt_host, void* const* V_host, float* const* sigma_host, void* workspace,
                                     size_t workspace_bytes, void* const* stage_events_host, void* stream) {
   XKV_TRY(check_layers(layers, layer_cols, ld_layer));
-  return factorize_impl(layer_ptrs_host, layers, layer_cols, batch, m, layers * layer_cols, ld_layer, rank, opts, A_host,
+  return factorize_impl(layer_ptrs_host, layers, layer_cols, batch, m, layers * layer_cols, ld_layer, rank, A_host,
                         Vt_host, V_host, sigma_host, nullptr, 0, workspace, workspace_bytes, stage_events_host, stream);
 }

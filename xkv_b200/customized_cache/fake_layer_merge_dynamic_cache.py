@@ -141,8 +141,7 @@ class _GroupState:
 
 
 class FakeLayerMergingCache(DynamicCache):
-    def __init__(self, merge_setup: xKVConfig, factorize_options: Optional[factorize.FactorizeOptions] = None,
-                 compress_decode_tokens: bool = False, decode_capacity: int = 4096):
+    def __init__(self, merge_setup: xKVConfig, compress_decode_tokens: bool = False, decode_capacity: int = 4096):
         """``compress_decode_tokens`` (extension, off by default: the reference keeps decode tokens exact,
         cache:131): once every layer of a group has seen a decode token, its pre-RoPE key / value rows are
         projected onto the group's right factors (xkv_append_project) and leave the dense tail.  Up to
@@ -153,7 +152,6 @@ class FakeLayerMergingCache(DynamicCache):
         self.layer_class_to_replicate = _XkvLayer
         self.num_layers = merge_setup.num_layers
         self.merge_setup = merge_setup
-        self.factorize_options = factorize_options
         self._groups: Dict[int, _GroupState] = {}
         self._workspace: Optional[torch.Tensor] = None
         self._merge_cos_sin = (None, None, True)     # (cos, sin, re_apply_rope) of the prefill call being merged
@@ -252,7 +250,7 @@ class FakeLayerMergingCache(DynamicCache):
                     l.keys = self._rope_dense(l.keys, cos, sin)
             return
         (gf,) = compress.compress_groups([keys], [values], info.rank_k, info.rank_v, merge_key=merge_k,
-                                         merge_value=merge_v, opts=self.factorize_options, layer_ids=[ids],
+                                         merge_value=merge_v, layer_ids=[ids],
                                          extra_rows=self.decode_capacity)
         cos, sin, re_rope = self._merge_cos_sin
         cs = sn = None

@@ -12,10 +12,10 @@ Algorithm (every product is a tcgen05 GEMM of xkv_gemm.cu, everything stays on t
 caller's stream; nothing synchronises):
 
   1. Gram            G = X^T X            one pass over X, symmetric tile set, fp32 accumulation in TMEM
-  2. range finder    Y = G Omega           Omega Gaussian n x l, l = r + oversample
+  2. range finder    Y = G Omega           Omega Gaussian n x l, l = round_up(r + 64, 64)
   3. CholeskyQR      Q = orth(Y)           row-normalise, S = Y^T Y (6-term bf16-limb product ~ fp32),
                                            blocked Cholesky + explicit inverse, Q = Y L^-T; repeated
-  4. power steps     Y = (G - c I) Q; CholeskyQR   `power_iters` times (3-term limb product; two CholeskyQR passes
+  4. power steps     Y = (G - c I) Q; CholeskyQR   4 times (3-term limb product; two CholeskyQR passes
                      after the first step, ONE accurate pass after the others); from the second
                      step on c ~ lambda_l / 2 (lambda_l read off the diagonal of the previous step's
                      triangular factor), which does the work of ~6 plain steps in 4
@@ -43,35 +43,9 @@ from ._lib import XkvError
 
 @dataclass
 class FactorizeOptions:
-    power_iters: int = 4       # 1 plain + 3 spectrally shifted power steps do the work of ~6 plain ones
-    oversample: int = 64
-    first_passes: int = 2      # CholeskyQR passes after the range finder (ill-conditioned sketch)
-    passes: int = 2            # CholeskyQR passes after each power step
-    final_passes: int = 2      # passes after the last power step (orthonormal to ~1e-5 after two)
-    window: int = 128          # Rayleigh-Ritz window width (<= 160: A and V live in shared memory)
-    jacobi_sweeps: int = 3     # the window is near-diagonal; 3 sweeps reach the same error as 6 (tools/sweep_factorize.py)
-    rayleigh_ritz: bool = True
-    want_sigma: bool = True    # also diagonalise the leading window to report singular values
-    gram_split_k: int = 1
-    gram_chunk_tokens: int = 16384  # tensor-core accumulation length of the Gram; pieces are summed in fp32 by the epilogue
-    small_split_k: int = 8
-    shifts: tuple = (3e-4, 1e-6, 1e-7)   # diagonal shift of CholeskyQR pass 0, 1, 2, ...
-    pivot_floor: float = 1e-12
-    spectral_shift: float = 0.5   # c = spectral_shift * (estimate of lambda_l from diag(R)); 0 disables the shift
-    shift_tail: int = 8
-    single_pass_from: int = 1     # power steps with index >= this (> 0; 0 = never) use ONE CholeskyQR pass (small
-                                  # shift, 6-term Gram): their input basis is already orthonormal and ordered
-    single_pass_last: bool = True   # ... including the last step
-    pass0_terms: int = 6            # limb terms of the heavily shifted first pass; 3 breaks down on inputs with a few dominant
-                                    # channels (coherent limb rounding errors exceed the shift), 6 is ~fp32
-    heavy_redo: bool = True         # redo a lightly shifted pass with the heavy shift when its Cholesky broke down (device decision)
-    power_terms: int = 3            # limb terms of the power-step product Y = Q G
-    second_pass_min_pivot: float = 0.05   # single-pass steps: the DEVICE adds a second pass for every matrix whose first
-                                          # pass met a Cholesky pivot below this (steep spectrum at high rank); 0 = never
-    solve_terms: int = 3            # limb terms of Q = L^-1 Y in the passes a later pass / step re-orthonormalises (the last power
-                                    # step always uses 6); 3 vs 6: same full-size error to 4e-5, step -0.1 .. -0.8 ms
-    seed: int = 1234
-    profile: bool = False
+    """The factorisation's schedule is fixed in the library (DESIGN.md section 2); what a caller chooses is here."""
+
+    profile: bool = False   # record the driver's 7 stage events and report the stage times in Factors.timings
 
 
 @dataclass
@@ -95,39 +69,17 @@ def _round_up(x: int, k: int) -> int:
     return (x + k - 1) // k * k
 
 
-def sketch_width(rank: int, oversample: int = 64) -> int:
-    return _round_up(rank + oversample, 64)
+def sketch_width(rank: int) -> int:
+    """Columns of the driver's sketch of a rank-`rank` factorisation; the matrix must have at least as many."""
+    return _round_up(rank + 64, 64)
 
 
 _STAGES = ("gram_gemm", "gram_reduce_split", "range_finder", "power_iters", "rayleigh_ritz", "project")
 
 
-def _c_options(opts: FactorizeOptions) -> "_lib.FactorizeOptions":
-    o = _lib.FactorizeOptions()
-    _lib.load().xkv_factorize_default_options(C.byref(o))
-    o.power_iters, o.oversample = opts.power_iters, opts.oversample
-    o.first_passes, o.passes, o.final_passes = opts.first_passes, opts.passes, opts.final_passes
-    o.window, o.jacobi_sweeps = opts.window, opts.jacobi_sweeps
-    o.rayleigh_ritz, o.want_sigma = int(opts.rayleigh_ritz), int(opts.want_sigma)
-    o.gram_split_k, o.small_split_k = opts.gram_split_k, opts.small_split_k
-    o.gram_chunk_tokens = int(opts.gram_chunk_tokens)
-    for i in range(4):
-        o.shifts[i] = opts.shifts[min(i, len(opts.shifts) - 1)]
-    o.pivot_floor = opts.pivot_floor
-    o.spectral_shift, o.shift_tail = opts.spectral_shift, opts.shift_tail
-    o.single_pass_from, o.single_pass_last = int(opts.single_pass_from), int(opts.single_pass_last)
-    o.second_pass_min_pivot = float(opts.second_pass_min_pivot)
-    o.pass0_terms = int(opts.pass0_terms)
-    o.power_terms = int(opts.power_terms)
-    o.heavy_redo = int(opts.heavy_redo)
-    o.solve_terms = int(opts.solve_terms)
-    o.seed = opts.seed
-    return o
-
-
 def workspace_bytes(batch: int, m: int, n: int, rank: int, opts: Optional[FactorizeOptions] = None) -> int:
-    o = _c_options(opts or FactorizeOptions())
-    return int(_lib.load().xkv_factorize_workspace_bytes(batch, m, n, rank, C.byref(o)))
+    """Workspace of one driver call (0 for a problem the driver rejects); `opts` does not change it."""
+    return int(_lib.load().xkv_factorize_workspace_bytes(batch, m, n, rank))
 
 
 def layer_rows(t: torch.Tensor) -> Optional[torch.Tensor]:
@@ -146,17 +98,15 @@ def _factorize_chunks(items: Sequence, chunk: int, m: int, n: int, rank: int, op
                       workspace: Optional[torch.Tensor], extra_rows: int, dev, run) -> List[Factors]:
     """What factorize_groups and factorize_batch share: sizes (and if needed allocates) the workspace for `chunk` matrices,
     then per chunk of `items` allocates A (with `extra_rows` spare token rows behind it, for tokens appended later by
-    xkv_append_project), Vt, V and sigma, and makes the driver call ``run(part, co, outs, tail)`` — outs: the A / Vt / V /
+    xkv_append_project), Vt, V and sigma, and makes the driver call ``run(part, outs, tail)`` — outs: the A / Vt / V /
     sigma pointer arrays, tail: the workspace, its size, the stage events and the stream, in the C argument order.  With
     `opts.profile` the 7 stage events of every call are recorded and their intervals summed into each Factors.timings."""
     lib = _lib.load()
-    co = _c_options(opts)
-    need = int(lib.xkv_factorize_workspace_bytes(chunk, m, n, rank, C.byref(co)))
+    need = int(lib.xkv_factorize_workspace_bytes(chunk, m, n, rank))
     if need == 0:
         raise XkvError(lib.xkv_last_error().decode() or "factorize: invalid problem")
     if workspace is None or workspace.numel() * workspace.element_size() < need:
         workspace = torch.empty(need, dtype=torch.uint8, device=dev)
-    nsig = int(lib.xkv_factorize_sigma_count(rank, C.byref(co)))
     stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
     out: List[Factors] = []
     all_events = []
@@ -167,7 +117,7 @@ def _factorize_chunks(items: Sequence, chunk: int, m: int, n: int, rank: int, op
         a = [t[:m] for t in a_store]
         vt = [torch.empty(rank, n, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
         v = [torch.empty(n, rank, dtype=torch.bfloat16, device=dev) for _ in range(nb)]
-        sig = [torch.empty(nsig, dtype=torch.float32, device=dev) if nsig else None for _ in range(nb)]
+        sig = [torch.empty(_lib.FACTORIZE_SIGMA_COUNT, dtype=torch.float32, device=dev) for _ in range(nb)]
         ev_arr = None
         if opts.profile:
             events = [torch.cuda.Event(enable_timing=True) for _ in range(7)]
@@ -175,9 +125,9 @@ def _factorize_chunks(items: Sequence, chunk: int, m: int, n: int, rank: int, op
                 e.record()  # torch creates the cudaEvent lazily; recording materialises the handle
             ev_arr = (C.c_void_p * 7)(*[e.cuda_event for e in events])
             all_events.append(events)
-        outs = (ops._ptr_array(a), ops._ptr_array(vt), ops._ptr_array(v), ops._ptr_array(sig) if nsig else None)
+        outs = (ops._ptr_array(a), ops._ptr_array(vt), ops._ptr_array(v), ops._ptr_array(sig))
         tail = (C.c_void_p(workspace.data_ptr()), workspace.numel() * workspace.element_size(), ev_arr, stream)
-        run(part, co, outs, tail)
+        run(part, outs, tail)
         for b in range(nb):
             out.append(Factors(A=a[b], Vt=vt[b], V=v[b], rank=rank, sigma_lead=sig[b], A_storage=a_store[b]))
     if opts.profile:
@@ -214,32 +164,26 @@ def factorize_groups(groups: Sequence[Sequence[torch.Tensor]], rank: int, opts: 
     r = int(rank)
     per_call = max(1, min(_lib.MAX_BATCH, 64 // nl))     # XKV_MAX_LAYER_MAPS layer matrices per launch
 
-    def run(part, co, outs, tail):
+    def run(part, outs, tail):
         flat = [t for grp in part for t in grp]
-        _lib.check(lib.xkv_factorize_groups(ops._ptr_array(flat), len(part), nl, lc, m, ld, r, C.byref(co), *outs, *tail))
+        _lib.check(lib.xkv_factorize_groups(ops._ptr_array(flat), len(part), nl, lc, m, ld, r, *outs, *tail))
 
     return _factorize_chunks(groups, min(len(groups), per_call), m, nl * lc, r, opts, workspace, extra_rows,
                              groups[0][0].device, run)
 
 
 def factorize_batch(xs: Sequence[torch.Tensor], rank: int, opts: Optional[FactorizeOptions] = None,
-                    workspace: Optional[torch.Tensor] = None, process_group=None, extra_rows: int = 0,
-                    comm_events: Optional[list] = None) -> List[Factors]:
+                    workspace: Optional[torch.Tensor] = None, extra_rows: int = 0) -> List[Factors]:
     """Factorise a batch of equally-shaped token-major matrices (m x n bf16) at rank `rank`.
 
     One call into the library's stream-ordered driver (xkv_factorize_batch); batches larger than the
-    C-ABI's per-call limit are processed in chunks that reuse one workspace.
-
-    With `process_group` (torch.distributed, NCCL) the inputs are the LOCAL token shards of matrices whose
-    rows are split over the group's ranks: the local Gram matrices are summed with one all-reduce, every
-    rank derives the same right factor, and `A` holds the local rows only (DESIGN.md §6).  `comm_events`: optional
-    [start, end] CUDA events (enable_timing) recorded around the all-reduce; the payload bytes are appended."""
+    C-ABI's per-call limit are processed in chunks that reuse one workspace.  Matrices whose rows are split over
+    several GPUs go through :func:`factorize_token_sharded`."""
     opts = opts or FactorizeOptions()
     if len(xs) == 0:
         return []
     lib = _lib.load()
     m, n = xs[0].shape
-    dev = xs[0].device
     for x in xs:
         if not x.is_cuda:
             raise XkvError("factorize: CUDA tensors required (no CPU path)")
@@ -247,37 +191,11 @@ def factorize_batch(xs: Sequence[torch.Tensor], rank: int, opts: Optional[Factor
             raise XkvError("factorize: inputs must be equally-shaped row-major bf16 matrices")
     r = int(rank)
 
-    def run(part, co, outs, tail):
-        nb = len(part)
+    def run(part, outs, tail):
+        _lib.check(lib.xkv_factorize_batch(ops._ptr_array(part), len(part), m, n, part[0].stride(0), r, *outs, None, 0,
+                                           *tail))
 
-        def call(phase, grams):
-            _lib.check(lib.xkv_factorize_batch(ops._ptr_array(part), nb, m, n, part[0].stride(0), r, C.byref(co), *outs,
-                                               ops._ptr_array(grams) if grams is not None else None, phase, *tail))
-
-        if process_group is None:
-            call(0, None)
-            return
-        import torch.distributed as dist
-
-        # the only data-path collective: all-reduce(sum) of the local Gram matrices, upper triangles only
-        # (n^2 / 2 + 16 n floats per matrix instead of n^2: the Gram is symmetric)
-        grams = torch.empty(nb, n, n, dtype=torch.float32, device=dev)
-        call(1, list(grams))
-        per = ops.gram_packed_elems(n)
-        packed = torch.empty(nb, per, dtype=torch.float32, device=dev)
-        for b in range(nb):
-            ops.gram_pack_upper(grams[b], packed[b])
-        if comm_events is not None:
-            comm_events[0].record()
-        dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=process_group)
-        if comm_events is not None:
-            comm_events[1].record()
-            comm_events.append(packed.numel() * packed.element_size())
-        for b in range(nb):
-            ops.gram_unpack_upper(packed[b], grams[b])
-        call(2, list(grams))
-
-    return _factorize_chunks(xs, min(len(xs), _lib.MAX_BATCH), m, n, r, opts, workspace, extra_rows, dev, run)
+    return _factorize_chunks(xs, min(len(xs), _lib.MAX_BATCH), m, n, r, opts, workspace, extra_rows, xs[0].device, run)
 
 
 _chain_streams = {}
@@ -302,15 +220,14 @@ def factorize_token_sharded(jobs: Sequence, process_group, opts: Optional[Factor
     3. the owner alone runs the range finder / CholeskyQR / power steps / Rayleigh-Ritz of its matrices (phase 3) — the part
        that does not shrink with the number of token shards — and broadcasts the right factor Vt (r x n bf16);
     4. every rank projects its own rows, A_p = X_p V (phase 4).
-    With one matrix per rank or more the whole factorisation scales; `factorize_batch(process_group=...)` (all-reduce, every
-    rank repeats the small stages) remains for a single matrix.  Returns Factors with the LOCAL rows of A."""
+    With one matrix per rank or more the whole factorisation scales.  Returns Factors with the LOCAL rows of A.
+    `opts.profile` does not apply here.  `comm_events`: optional [start, end] CUDA events (enable_timing) recorded around
+    the exchanges; the payload bytes are appended."""
     import torch.distributed as dist
 
-    opts = opts or FactorizeOptions()
     lib = _lib.load()
     world = dist.get_world_size(process_group)
     me = dist.get_rank(process_group)
-    co = _c_options(opts)
     stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
     dev = jobs[0][0].device
     n = jobs[0][0].shape[1]
@@ -322,7 +239,7 @@ def factorize_token_sharded(jobs: Sequence, process_group, opts: Optional[Factor
         nb = len(vts_)
         m = xs[0].shape[0] if xs is not None else n
         _lib.check(lib.xkv_factorize_batch(
-            ops._ptr_array(xs) if xs is not None else None, nb, m, n, xs[0].stride(0) if xs is not None else n, r, C.byref(co),
+            ops._ptr_array(xs) if xs is not None else None, nb, m, n, xs[0].stride(0) if xs is not None else n, r,
             ops._ptr_array(a_s) if a_s is not None else None, ops._ptr_array(vts_), ops._ptr_array(vs) if vs is not None else None,
             None, ops._ptr_array(grams) if grams is not None else None, phase, C.c_void_p(ws.data_ptr()),
             ws.numel(), None, stream if on is None else C.c_void_p(on.cuda_stream)))
@@ -336,10 +253,10 @@ def factorize_token_sharded(jobs: Sequence, process_group, opts: Optional[Factor
     for i, (_, r) in enumerate(jobs):
         if i % world == me:
             owned.setdefault(r, []).append(i)
-    need = max(int(lib.xkv_factorize_workspace_bytes(1, max(m_loc, r), n, r, C.byref(co))) for _, r in jobs)
+    need = max(int(lib.xkv_factorize_workspace_bytes(1, max(m_loc, r), n, r)) for _, r in jobs)
     for r, idx in owned.items():
         for lo in range(0, len(idx), _lib.MAX_BATCH):
-            need = max(need, int(lib.xkv_factorize_workspace_bytes(len(idx[lo:lo + _lib.MAX_BATCH]), n, n, r, C.byref(co))))
+            need = max(need, int(lib.xkv_factorize_workspace_bytes(len(idx[lo:lo + _lib.MAX_BATCH]), n, n, r)))
     ws = torch.empty(need, dtype=torch.uint8, device=dev)
     gram = torch.empty(n, n, dtype=torch.float32, device=dev)
     packed = [torch.empty(per, dtype=torch.float32, device=dev) for _ in range(nj)]
@@ -371,7 +288,7 @@ def factorize_token_sharded(jobs: Sequence, process_group, opts: Optional[Factor
             chain_streams.append(st)
         with torch.cuda.stream(st):
             ws_r = ws if st is main_stream else torch.empty(
-                max(int(lib.xkv_factorize_workspace_bytes(len(idx[lo:lo + _lib.MAX_BATCH]), n, n, r, C.byref(co)))
+                max(int(lib.xkv_factorize_workspace_bytes(len(idx[lo:lo + _lib.MAX_BATCH]), n, n, r))
                     for lo in range(0, len(idx), _lib.MAX_BATCH)), dtype=torch.uint8, device=dev)
             for lo in range(0, len(idx), _lib.MAX_BATCH):
                 part = idx[lo:lo + _lib.MAX_BATCH]

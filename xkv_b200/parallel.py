@@ -4,9 +4,9 @@ Two natural shards (DESIGN.md §6):
 
 * layer groups are independent (reference cache:161-165 touches only the group's layers) — ranks own
   disjoint sets of groups and never exchange data on the hot path;
-* long contexts can be split by token rows — the only exchange is one all-reduce(sum) of each matrix's
-  n x n fp32 Gram (``factorize_batch(..., process_group=...)``), after which every rank derives the same
-  right factor and projects its own rows.
+* long contexts can be split by token rows (``factorize.factorize_token_sharded``) — each matrix's n x n fp32
+  Gram is summed over the ranks (one all-reduce of its packed upper triangle), the matrix's owner derives the right
+  factor and broadcasts it, and every rank projects its own rows.
 """
 from __future__ import annotations
 
