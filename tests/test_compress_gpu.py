@@ -41,7 +41,8 @@ def test_host_pipeline_equals_resident_path(chunk_groups):
 
 
 @pytest.mark.parametrize("g,h,s,d,rk,rv", [(4, 8, 4096, 128, 512, 768), (2, 2, 1000, 64, 64, 64), (3, 1, 2048, 512, 256, 256),
-                                           (8, 8, 2048, 128, 1024, 1536)])
+                                           (8, 8, 2048, 128, 1024, 1536),
+                                           (7, 8, 2048, 128, 896, 1344)])   # the non-uniform config's 7-layer group
 def test_in_place_and_packed_paths_give_bit_identical_factors(g, h, s, d, rk, rv):
     """Per-layer tensor maps (no gather, no packed copy) against the gather kernel + packed matrix: the same tiles in
     the same order, so the factors must be bit-identical.  Token-major layer tensors with a padded row stride (the MLA

@@ -89,6 +89,11 @@ def test_steep_spectrum_at_high_rank_meets_the_bf16_storage_floor():
         (4096, 4096, 500, 1.0),   # rank not a multiple of 64 (ragged Rayleigh-Ritz window)
         (4096, 4096, 1, 1.0),     # rank 1
         (3000, 4096, 37, 0.5),
+        # wide sketches, whose Cholesky runs on 16-CTA clusters (20 blocks and more)
+        (2048, 2048, 1216, 1.0),  # sketch width 1280: 20 blocks
+        (2048, 2048, 1536, 0.5),  # sketch width 1600: 25 blocks
+        (4096, 7168, 1344, 0.5),  # the 7-layer group of the non-uniform config
+        (4096, 8192, 1536, 0.5),  # config 4's V columns
     ],
 )
 def test_ragged_short_and_odd_inputs(tokens, cols, rank, alpha):
@@ -178,6 +183,30 @@ def test_batch_of_two_ranks_shapes_and_determinism():
     for a, b in zip(f1, f2):
         assert torch.equal(a.A, b.A) and torch.equal(a.Vt, b.Vt)   # same seed -> bit-identical factors
     assert not torch.equal(f1[0].Vt, f1[1].Vt)
+
+
+def test_full_batch_across_the_chunk_boundary():
+    """17 matrices in one factorize_batch call at rank 1216 (sketch width 1280, 20 Cholesky blocks): one driver call of
+    16 and one of 1.  Every matrix meets the bar against its own SVD, so a mix-up of the per-matrix pointers, seeds
+    (kSeed + 7919 b) or device flags of matrices 8..15 shows.  Position 0 of a call gets the same seed, and nothing the
+    driver chooses depends on the batch size (split-K factors depend on n only; the Cholesky's cluster size does not
+    change its arithmetic), so the 17th result equals a call on that matrix alone, and so does the first."""
+    from xkv_b200 import factorize, synthetic
+
+    rank, alphas = 1216, (0.5, 1.0)
+    xs = [synthetic.group_matrix(2048, 2048, alphas[i % 2], seed=300 + i, device="cuda") for i in range(17)]
+    fs = factorize.factorize_batch(xs, rank)
+    (last,) = factorize.factorize_batch([xs[16]], rank)
+    (first,) = factorize.factorize_batch([xs[0]], rank)
+    torch.cuda.synchronize()
+    for i, (x, f) in enumerate(zip(xs, fs)):
+        ref_hat, _ = _ref_fake_svd(x, rank)
+        e_ref, e_ours = _rel_err(x, ref_hat), _rel_err(x, f.reconstruct())
+        print(f"matrix {i} alpha={alphas[i % 2]}: err ref={e_ref:.6f} ours={e_ours:.6f}")
+        assert torch.isfinite(f.A).all() and torch.isfinite(f.Vt).all(), i
+        assert e_ours ** 2 <= (1.01 * e_ref) ** 2 + 3e-3 ** 2, i
+    assert torch.equal(fs[16].A, last.A) and torch.equal(fs[16].Vt, last.Vt)
+    assert torch.equal(fs[0].A, first.A) and torch.equal(fs[0].Vt, first.Vt)
 
 
 def test_rejects_rank_that_does_not_fit():

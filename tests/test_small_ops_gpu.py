@@ -90,6 +90,27 @@ def test_pass_flags_and_launch_predicate():
     ops.shift_normalize_rows(ys)
     torch.cuda.synchronize()
     assert torch.allclose(ys[0].norm(dim=1), torch.ones(8, device=dev), atol=1e-5)
+    # a full 16-matrix predicated Cholesky at sketch width 1600 (25 blocks, the widest clusters), every other matrix
+    # skipped: the skipped ones at b >= 8 keep S and Linv bit for bit, the others get what an unpredicated launch gives
+    l, batch = 1600, 16
+    torch.manual_seed(4)
+    grams = [_unit_row_gram(l).float() for _ in range(batch)]
+    flags = torch.tensor([b % 2 for b in range(batch)], device=dev, dtype=torch.int32)
+    ss = [g.clone() for g in grams]
+    linvs = [torch.full((l, l), 7.0, device=dev) for _ in range(batch)]
+    with ops.launch_predicate(flags):
+        ops.cholesky_inverse(ss, linvs, shift=1e-6)
+    singles = []
+    for b in range(1, batch, 2):
+        li = torch.full((l, l), float("nan"), device=dev)
+        ops.cholesky_inverse([grams[b].clone()], [li], shift=1e-6)
+        singles.append(li)
+    torch.cuda.synchronize()
+    for b in range(0, batch, 2):
+        assert torch.equal(ss[b], grams[b]), f"S of skipped matrix {b} was written"
+        assert (linvs[b] == 7.0).all(), f"Linv of skipped matrix {b} was written"
+    for b, li in zip(range(1, batch, 2), singles):
+        assert torch.equal(linvs[b], li), f"predicated matrix {b} differs from its own launch"
 
 
 def test_split_bf16_limbs_reconstruct_fp32():
@@ -170,7 +191,14 @@ def test_shift_normalize_rows_and_rdiag():
     assert torch.allclose(shifts, c_ref, rtol=1e-5)
 
 
-@pytest.mark.parametrize("l,cond", [(64, 10.0), (192, 1e3), (576, 1e4), (832, 1e2)])
+def _unit_row_gram(l):
+    """fp64 S = Y Y^T of an l x 3l Gaussian Y with unit rows: the Gram CholeskyQR factors (condition ~14 at any l)."""
+    y = torch.randn(l, 3 * l, device="cuda", dtype=torch.float64)
+    y = y / y.norm(dim=1, keepdim=True)
+    return y @ y.t()
+
+
+@pytest.mark.parametrize("l,cond", [(64, 10.0), (192, 1e3), (576, 1e4), (832, 1e2), (1600, 1e3)])
 def test_cholesky_inverse(l, cond):
     from xkv_b200 import ops
 
@@ -196,18 +224,26 @@ def test_cholesky_inverse(l, cond):
         assert err < 5e-3 * max(1.0, cond / 1e3), f"Linv S Linv^T deviates from I by {err}"
 
 
-@pytest.mark.parametrize("l,batch", [(128, 1), (320, 2), (576, 8), (1088, 2)])
+@pytest.mark.parametrize("l,batch", [
+    (128, 1), (320, 2), (576, 8), (1088, 2),
+    (256, 1), (512, 2), (1024, 3),   # 4, 8 and 16 blocks: the inverse phase's super-block pairs come out even
+    (1216, 1),                       # 19 blocks: the widest 8-CTA cluster
+    (1280, 1),                       # 20 blocks: the narrowest 16-CTA cluster
+    (1408, 2), (1600, 1),            # the sketch widths of ranks 1344 and 1536 (non-uniform config, config 4 V)
+    (1600, 16),                      # a full batch of the widest: 16 clusters of 16 CTAs if the device keeps them resident
+])
 def test_cholesky_inverse_limbs_match_fp32_inverse(l, batch):
     """The fused kernel's bf16 limbs of Linv (the GEMM operand) add up to the fp32 Linv it writes; the inverse
-    agrees with torch's Cholesky + triangular solve in fp64."""
+    agrees with torch's Cholesky + triangular solve in fp64.  The cluster size follows the number of 64-column blocks
+    (1, 2, 4, 8 CTAs; 16 from 20 blocks), so the widths cover every size.  S is well conditioned (~14 at any l), and
+    the fp32 error of its Cholesky inverse grows only slowly with l (LAPACK's fp32 factor and triangular solve: 2.4e-7
+    relative at l = 1088, 2.5e-7 at l = 1600), so the 1e-4 bound of the narrow cases holds for the widest ones too."""
     from xkv_b200 import ops
 
     torch.manual_seed(l + batch)
     ss, refs = [], []
     for b in range(batch):
-        y = torch.randn(l, 3 * l, device="cuda", dtype=torch.float64)
-        y = y / y.norm(dim=1, keepdim=True)
-        s = y @ y.t()
+        s = _unit_row_gram(l)
         refs.append(torch.linalg.inv(torch.linalg.cholesky(s + 1e-6 * torch.eye(l, device="cuda", dtype=torch.float64))))
         ss.append(s.float().contiguous())
     linvs = [torch.full((l, l), float("nan"), device="cuda") for _ in range(batch)]
@@ -219,9 +255,89 @@ def test_cholesky_inverse_limbs_match_fp32_inverse(l, batch):
         assert not torch.isnan(li).any()
         assert torch.equal(torch.triu(li, 1), torch.zeros_like(li))
         rel = (li.double() - refs[b]).abs().max().item() / refs[b].abs().max().item()
+        print(f"l={l} matrix {b}/{batch}: Linv rel. deviation {rel:.2e}")
         assert rel < 1e-4, f"Linv deviates from the fp64 inverse by {rel}"
         total = limbs[0][b].float() + limbs[1][b].float() + limbs[2][b].float()
         assert (total - li).abs().max().item() <= 1e-6 * li.abs().max().item()
+
+
+@pytest.mark.parametrize("l", [576, 1280, 1600])
+def test_cholesky_inverse_is_independent_of_batch_position_and_strides(l):
+    """The same S matrices in one 16-matrix launch and in 16 single-matrix launches give bit-identical Linv and limbs.
+    Each output tile's products are applied in a fixed (k, t) order whichever CTA of the cluster runs them, and the
+    matrices of a launch are independent along blockIdx.y; so neither the batch position nor the cluster size (from 20
+    blocks on, a single matrix gets 16 CTAs and a full batch 16 or 8 depending on how many 16-CTA clusters the device
+    keeps resident) may change a bit.  The batched launch also reads S and writes Linv with rows l + 64 apart and the
+    limbs with rows l + 24 apart; the NaN in the padding columns must stay untouched."""
+    from xkv_b200 import ops
+
+    torch.manual_seed(17 + l)
+    batch, nan = 16, float("nan")
+    grams = [_unit_row_gram(l).float() for _ in range(batch)]
+
+    def padded(pad, dtype):
+        return torch.full((l, l + pad), nan, device="cuda", dtype=dtype)
+
+    s_buf = [padded(64, torch.float32) for _ in range(batch)]
+    for buf, g in zip(s_buf, grams):
+        buf[:, :l] = g
+    li_buf = [padded(64, torch.float32) for _ in range(batch)]
+    limb_buf = [[padded(24, torch.bfloat16) for _ in range(batch)] for _ in range(3)]
+    ops.cholesky_inverse([t[:, :l] for t in s_buf], [t[:, :l] for t in li_buf], shift=1e-6, pivot_floor=1e-12,
+                         limbs=[[t[:, :l] for t in side] for side in limb_buf])
+    singles = []
+    for g in grams:
+        li = torch.full((l, l), nan, device="cuda")
+        limbs = [[torch.full((l, l), nan, device="cuda", dtype=torch.bfloat16)] for _ in range(3)]
+        ops.cholesky_inverse([g.clone()], [li], shift=1e-6, pivot_floor=1e-12, limbs=limbs)
+        singles.append((li, [side[0] for side in limbs]))
+    torch.cuda.synchronize()
+    for b, (li, limbs) in enumerate(singles):
+        assert not torch.isnan(li).any()
+        assert torch.equal(li_buf[b][:, :l], li), f"Linv of matrix {b} depends on the launch"
+        for i, (side, one) in enumerate(zip(limb_buf, limbs)):
+            assert torch.equal(side[b][:, :l], one), f"limb {i} of matrix {b} depends on the launch"
+        for t in [s_buf[b], li_buf[b]] + [side[b] for side in limb_buf]:
+            assert torch.isnan(t[:, l:]).all(), f"padding of matrix {b} was written"
+
+
+def test_cholesky_inverse_rejects_batches_with_mixed_layouts():
+    """The library takes one row stride for every S and Linv (S's) and one for every limb (hi[0]'s): a batch whose
+    matrices differ in shape or stride is refused before anything is launched.  (Every odd matrix here is larger than
+    what the library would address, so a launch that is not refused stays in bounds.)"""
+    from xkv_b200 import _lib, ops
+
+    l, nan = 128, float("nan")
+    s = _unit_row_gram(l).float()
+    big = _unit_row_gram(l + 64).float()
+
+    def linvs():
+        return [torch.full((l, l), nan, device="cuda") for _ in range(2)]
+
+    def limbs():
+        return [[torch.full((l, l), nan, device="cuda", dtype=torch.bfloat16) for _ in range(2)] for _ in range(3)]
+
+    wide = torch.full((l, l + 64), nan, device="cuda")
+    wide_limb = torch.full((l, l + 64), nan, device="cuda", dtype=torch.bfloat16)
+    cases = {
+        "Linv strided unlike S": ([s.clone(), s.clone()], [linvs()[0], wide[:, :l]], None),
+        "S strided unlike ss[0]": ([s.clone(), big[:l, :l]], linvs(), None),
+        "S of another size": ([s.clone(), big.clone()], linvs(), None),
+        "Linv of another size": ([s.clone(), s.clone()], [linvs()[0], torch.full((l + 64, l + 64), nan, device="cuda")],
+                                 None),
+        "fp64 S": ([s.clone(), s.double()], linvs(), None),
+        "mid limb strided unlike hi[0]": ([s.clone(), s.clone()], linvs(), limbs()),
+        "hi limb strided unlike hi[0]": ([s.clone(), s.clone()], linvs(), limbs()),
+    }
+    cases["mid limb strided unlike hi[0]"][2][1][1] = wide_limb[:, :l]
+    cases["hi limb strided unlike hi[0]"][2][0][1] = wide_limb[:, :l]
+    for name, (ss, lis, lb) in cases.items():
+        with pytest.raises(_lib.XkvError):
+            ops.cholesky_inverse(ss, lis, shift=1e-6, limbs=lb)
+            torch.cuda.synchronize()
+            pytest.fail(f"{name}: accepted")
+    torch.cuda.synchronize()
+    assert torch.isnan(wide).all() and torch.isnan(wide_limb).all()
 
 
 def test_cholesky_shift_keeps_indefinite_gram_finite():

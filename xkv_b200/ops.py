@@ -294,17 +294,37 @@ class launch_predicate:
 def cholesky_inverse(ss: Sequence[torch.Tensor], linvs: Sequence[torch.Tensor], shift: float = 0.0,
                      pivot_floor: float = 1e-12, limbs=None) -> None:
     """Batched (S + shift*I) = L L^T and Linv = L^{-1} in one cluster launch (S is destroyed); `limbs` =
-    (hi, mid, lo) lists of bf16 matrices that receive the limb split of Linv."""
+    (hi, mid, lo) lists of bf16 matrices that receive the limb split of Linv (mid / lo may be None).
+    The library takes one row stride for every S and Linv and one for every limb matrix: a batch whose matrices do
+    not share them would be read and written at the wrong addresses, so it is rejected."""
     _require_cuda(*ss, *linvs)
     l = ss[0].shape[0]
+    ld = ss[0].stride(0)
+    if len(linvs) != len(ss):
+        raise _lib.XkvError("cholesky_inverse: one Linv per S required")
+    for t in list(ss) + list(linvs):
+        if t.dtype != torch.float32 or tuple(t.shape) != (l, l) or t.stride() != (ld, 1):
+            raise _lib.XkvError(f"cholesky_inverse: every S and Linv must be a ({l}, {l}) fp32 matrix with the row stride "
+                                f"of ss[0] ({ld}) and unit inner stride")
     if limbs is None:
-        check(_lib.load().xkv_cholesky_inverse(_ptr_array(ss), _ptr_array(linvs), len(ss), l, ss[0].stride(0),
-                                               C.c_float(shift), C.c_float(pivot_floor), _stream()))
-    else:
-        hi, mid, lo = limbs
-        check(_lib.load().xkv_cholesky_inverse_limbs(_ptr_array(ss), _ptr_array(linvs), _ptr_array(hi), _ptr_array(mid),
-                                                     _ptr_array(lo), len(ss), l, ss[0].stride(0), hi[0].stride(0),
-                                                     C.c_float(shift), C.c_float(pivot_floor), _stream()))
+        check(_lib.load().xkv_cholesky_inverse(_ptr_array(ss), _ptr_array(linvs), len(ss), l, ld, C.c_float(shift),
+                                               C.c_float(pivot_floor), _stream()))
+        return
+    hi, mid, lo = limbs
+    _require_cuda(*hi, *(mid or []), *(lo or []))
+    ld_limb = hi[0].stride(0)
+    for side in (hi, mid, lo):
+        if side is None:
+            continue
+        if len(side) != len(ss):
+            raise _lib.XkvError("cholesky_inverse: one limb matrix per S required")
+        for t in side:
+            if t is not None and (t.dtype != torch.bfloat16 or tuple(t.shape) != (l, l) or t.stride() != (ld_limb, 1)):
+                raise _lib.XkvError(f"cholesky_inverse: every limb must be a ({l}, {l}) bf16 matrix with the row stride of "
+                                    f"hi[0] ({ld_limb}) and unit inner stride")
+    check(_lib.load().xkv_cholesky_inverse_limbs(_ptr_array(ss), _ptr_array(linvs), _ptr_array(hi), _ptr_array(mid),
+                                                 _ptr_array(lo), len(ss), l, ld, ld_limb, C.c_float(shift),
+                                                 C.c_float(pivot_floor), _stream()))
 
 
 def jacobi_eigh(ts: Sequence[torch.Tensor], evals: Sequence[torch.Tensor],
