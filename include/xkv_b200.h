@@ -250,6 +250,25 @@ XKV_API int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, int
                                        int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
                                        int64_t tail_stride_t, float scale, void* out, void* workspace,
                                        size_t workspace_bytes, void* stream, float* lse_out);
+/* One-sided group: exactly one of the layer's two slots is factored, the other stayed dense (merge_key or merge_value off,
+ * or a rank that does not fit one side).  Each side is given EITHER as factors (A_*, lda_*, r*, V*_layer, ldv_*; the dense
+ * pointer NULL) OR as a dense prefix slot (*_dense, *_stride_h, *_stride_t; A_* NULL):
+ *   k_dense    rotated prefix keys, element (t, h, d) at k_dense[h * k_stride_h + t * k_stride_t + d] (an (S, H, D) or
+ *              (H, S, D) view); cos / sin are not read for a dense key side
+ *   v_dense    prefix values, same addressing
+ * Both strides multiples of 8 elements, the base 16-byte aligned; q 16-byte aligned when the key side is dense.  Both sides
+ * factored or both dense is an error (use xkv_decode_attention_multi, or SDPA).  Everything else -- q / Tq / heads, the
+ * tail and its causal rule, scale, out, lse_out, bounds -- as xkv_decode_attention_multi.  Workspace:
+ * xkv_decode_half_workspace_bytes(Hq*Tq, S, T, value_width), value_width = rv for factored values, D for dense ones. */
+XKV_API size_t xkv_decode_half_workspace_bytes(int rows, int S, int T, int value_width);
+XKV_API int xkv_decode_attention_half(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                                      const void* Vk_layer, int64_t ldv_k, const void* k_dense, int64_t k_stride_h,
+                                      int64_t k_stride_t, const void* A_v, int64_t lda_v, int rv, const void* Vv_layer,
+                                      int64_t ldv_v, const void* v_dense, int64_t v_stride_h, int64_t v_stride_t, int S,
+                                      const void* cos, const void* sin, int64_t ld_cs, const void* k_tail,
+                                      const void* v_tail, int T, int64_t tail_stride_h, int64_t tail_stride_t,
+                                      float scale, void* out, void* workspace, size_t workspace_bytes, void* stream,
+                                      float* lse_out);
 /* test hook: 1 forces the tile-per-CTA scores kernel (otherwise chosen only when one head's slice of the right
  * factor exceeds 128 KiB of shared memory), 0 restores the automatic choice */
 XKV_API void xkv_decode_force_tiled(int on);

@@ -69,7 +69,8 @@ def xKV_llama_forward(  # noqa: N802
         assert isinstance(cache, FakeLayerMergingCache)
         cache.update(k_pre, v, self.layer_idx, mode="prefill", cos=cos, sin=sin, return_dense=False)
     elif cache is not None:
-        # decode: fused attention over the factored cache when the layer's group is factored, else the dense path.
+        # decode: fused attention over the factored cache when the layer's group is factored on at least one side (a
+        # one-sided group reads its other slot dense, in place), else the dense path.
         # The fused kernel attends over EVERY cached token; a sliding-window layer (Mistral / Qwen2 checkpoints with
         # config.sliding_window, reference mistral.py:69) whose context has outgrown its window must honour the mask
         # transformers built, so it takes the dense path (materialised K^ / V^ + SDPA with that mask).

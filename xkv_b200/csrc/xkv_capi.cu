@@ -64,8 +64,26 @@ int encode_tmap_2d_bf16(CUtensorMap* map, const void* base, uint64_t inner, uint
   return 0;
 }
 
+int encode_tmap_3d_bf16(CUtensorMap* map, const void* base, const uint64_t dims[3], const uint64_t strides_elems[2],
+                        const uint32_t box[3]) {
+  auto enc = tensor_map_encoder();
+  XKV_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled unavailable (no CUDA driver?)");
+  cuuint64_t gdim[3] = {dims[0], dims[1], dims[2]};
+  cuuint64_t gstride[2] = {strides_elems[0] * 2, strides_elems[1] * 2};   // bytes, dimensions 1 and 2
+  cuuint32_t bx[3] = {box[0], box[1], box[2]};
+  cuuint32_t estride[3] = {1, 1, 1};
+  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), gdim, gstride, bx, estride,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  XKV_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed (%d): base=%p dims=%llux%llux%llu strides=%llu,%llu",
+              static_cast<int>(r), base, static_cast<unsigned long long>(dims[0]), static_cast<unsigned long long>(dims[1]),
+              static_cast<unsigned long long>(dims[2]), static_cast<unsigned long long>(strides_elems[0]),
+              static_cast<unsigned long long>(strides_elems[1]));
+  return 0;
+}
+
 }  // namespace xkv
 
 extern "C" const char* xkv_last_error(void) { return xkv::error_buffer(); }
-extern "C" int xkv_version(void) { return 202; }
+extern "C" int xkv_version(void) { return 203; }
 extern "C" int64_t xkv_launch_count(void) { return xkv::g_launch_count.load(); }

@@ -1361,7 +1361,10 @@ __global__ void __launch_bounds__(256) combine_kernel(const float* __restrict__ 
 // the shared memory of every CTA of the cluster (distributed shared memory), and after one cluster barrier each CTA
 // contracts the whole U row with ITS D / RC_CL rows of the layer's value factor.  Replaces reduce_u_kernel +
 // combine_kernel (two launches and a round trip of U through L2) on the Llama path.
+// DENSE_V: the value slot of the group is dense (one-sided groups, xkv_decode_attention_half): the slabs hold
+// U_s = P_s V_h (rv = D columns) and the identity takes the place of Bv_l -- output dim d of a row is U[d] itself.
 constexpr int RC_CL = 8;
+template <bool DENSE_V>
 __global__ void __launch_bounds__(256) reduce_combine_kernel(const float* __restrict__ slabs, int nslabs, long long slab_stride,
                                                              int rv, const __nv_bfloat16* __restrict__ Bv, long long ldb,
                                                              const __nv_bfloat16* __restrict__ prob, long long ldp, int S, int T,
@@ -1413,9 +1416,13 @@ __global__ void __launch_bounds__(256) reduce_combine_kernel(const float* __rest
   for (int d = cr * dpc + warp; d < min(D, (cr + 1) * dpc); d += 8) {
     const __nv_bfloat16* row = Bv + static_cast<long long>(h * D + d) * ldb;
     float acc = 0.f;
-    for (int jj = lane * 2; jj < rv; jj += 64) {
-      const __nv_bfloat162 b2 = *reinterpret_cast<const __nv_bfloat162*>(row + jj);
-      acc = fmaf(u_s[jj], __bfloat162float(b2.x), fmaf(u_s[jj + 1], __bfloat162float(b2.y), acc));
+    if constexpr (DENSE_V) {
+      if (lane == 0) acc = u_s[d];
+    } else {
+      for (int jj = lane * 2; jj < rv; jj += 64) {
+        const __nv_bfloat162 b2 = *reinterpret_cast<const __nv_bfloat162*>(row + jj);
+        acc = fmaf(u_s[jj], __bfloat162float(b2.x), fmaf(u_s[jj + 1], __bfloat162float(b2.y), acc));
+      }
     }
     const int tv = T > 0 ? tail_visible(T, Tq, hq) : 0;   // causal: the tail tokens this row sees
     float acc_t = 0.f;
@@ -1423,6 +1430,298 @@ __global__ void __launch_bounds__(256) reduce_combine_kernel(const float* __rest
       acc_t = fmaf(__bfloat162float(prob[hq * ldp + S + t]), __bfloat162float(v_tail[h * sh + t * st + d]), acc_t);
     acc = warp_sum(fmaf(w_tail, acc_t, acc));
     if (lane == 0) out[hq * D + d] = __float2bfloat16_rn(acc * inv);
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// One-sided groups (xkv_decode_attention_half): one slot of the layer is factored, the other stayed dense (merge_key /
+// merge_value off, or a rank that does not fit one side).  The factored side runs the kernels above; the dense side runs
+// one of the two kernels below, feeding the same chunk-local softmax and the same slab reduction + combine.
+//
+//   dense keys    scores[r][t] = scale * q_r . K[t, h(r)]: a 128-token key tile (already rotated: RoPE was applied once,
+//                 when the group was merged) is the A operand of ONE tcgen05.mma per tile, M = 128 tokens, N = nq16 (the
+//                 kv head's q rows rounded up to 16, the pair kernel's q tile), K = D.  Every key tile is read once for all
+//                 q rows of its head.  Warp roles: 0 TMA, 1 MMA, 2..5 score read-out (the pair kernel's).
+//   dense values  U_c^T (D x nq16) = V_h tile^T . P_h^T accumulated in tensor memory over the 64-token blocks of softmax
+//                 chunk c: A = the value tile straight from the token-major slot (MN-major, M = D), B = the head's
+//                 probability rows (K-major).  One CTA per (kv head, chunk); every value tile is read once.  The fp32 slab
+//                 U_c goes to (nchunks, rows, D); reduce_combine_kernel<true> weights, sums and normalises the slabs.
+// Both read the dense slot through a 3-D tensor map {D, tokens, heads} (or {D, heads, tokens} when the head stride is
+// the smaller one: TMA wants the outer strides of a box in any order but the box layout is the same), so any
+// (S, H, D) / (H, S, D) view with strides that are multiples of 8 elements is read in place.
+// ---------------------------------------------------------------------------------------------
+constexpr int DN_THREADS = 192;     // TMA warp, MMA warp, four read-out warps (one per TMEM lane quarter)
+constexpr int DN_MAX_STAGES = 8;
+constexpr int DN_NACC = 4;          // score accumulators of nq16 columns (dense-key kernel)
+constexpr int DN_VBLK = 64;         // tokens per value block (dense-value kernel)
+
+struct alignas(64) DenseParams {
+  CUtensorMap slot_map;   // the dense slot, box {64 dims, tile tokens, 1 head} (dims ordered as slot_tok_dim says)
+  CUtensorMap rows_map;   // keys: q (rows x D), box {64, nq16}; values: probabilities (rows x S), box {64 tokens, nq16}
+  float* out;             // keys: scores (rows, ld_out); values: slabs (nchunks, rows, D)
+  long long ld_out;
+  int S, H, qpk, rows, stages;
+  int slot_tok_dim;       // 1: the map is {D, S, H}; 2: {D, H, S}
+  int kps;                // values: 64-token blocks per softmax chunk
+  float scale;
+};
+
+__device__ __forceinline__ void load_slot_tile(void* dst, const DenseParams& P, uint64_t* bar, int d0, int t0, int h) {
+  if (P.slot_tok_dim == 1)
+    tma_load_3d(dst, &P.slot_map, bar, d0, t0, h);
+  else
+    tma_load_3d(dst, &P.slot_map, bar, d0, h, t0);
+}
+
+template <int D, int NQ16>
+__global__ void __launch_bounds__(DN_THREADS, 1) decode_dense_scores_kernel(const __grid_constant__ DenseParams P) {
+  constexpr int NKC = D / 64;                     // 64-dim chunks of a key tile
+  constexpr int TILE_BYTES = NKC * DBM * 128;     // 128 tokens x D
+  constexpr int Q_BYTES = NKC * NQ16 * 128;       // the pair kernel's q tile with all nq16 rows in one CTA
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint8_t* sQ = smem;
+  uint8_t* sK = smem + Q_BYTES;
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(sK + P.stages * TILE_BYTES);
+  uint64_t* empty_bar = full_bar + DN_MAX_STAGES;
+  uint64_t* tfull_bar = empty_bar + DN_MAX_STAGES;   // [DN_NACC]
+  uint64_t* tempty_bar = tfull_bar + DN_NACC;        // [DN_NACC]
+  uint64_t* q_bar = tempty_bar + DN_NACC;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(q_bar + 1);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  // CTA -> kv head h and the token tiles slot, slot + nslots, ... (as decode_scores_mma2_kernel)
+  const int h = static_cast<int>(blockIdx.x) % P.H;
+  const int slot = static_cast<int>(blockIdx.x) / P.H;
+  const int nslots = (static_cast<int>(gridDim.x) - h + P.H - 1) / P.H;
+  const int ntiles = (P.S + DBM - 1) / DBM;
+
+  if (warp == 0 && lane == 0) {
+    for (int i = 0; i < P.stages; ++i) {
+      mbar_init(&full_bar[i], 1);
+      mbar_init(&empty_bar[i], 1);
+    }
+    for (int i = 0; i < DN_NACC; ++i) {
+      mbar_init(&tfull_bar[i], 1);
+      mbar_init(&tempty_bar[i], 4);   // one arrive per read-out warp
+    }
+    mbar_init(q_bar, 1);
+    mbar_fence_init();
+    tma_prefetch_desc(&P.slot_map);
+    tma_prefetch_desc(&P.rows_map);
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, 256);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  if (warp == 0) {
+    if (elect_one()) {
+      mbar_expect_tx(q_bar, Q_BYTES);
+#pragma unroll
+      for (int c = 0; c < NKC; ++c) tma_load_2d(sQ + c * NQ16 * 128, &P.rows_map, q_bar, c * 64, h * P.qpk);
+      int s = 0;
+      uint32_t ph = 0;
+      for (int tile = slot; tile < ntiles; tile += nslots) {
+        mbar_wait(&empty_bar[s], ph ^ 1u);
+        mbar_expect_tx(&full_bar[s], TILE_BYTES);
+#pragma unroll
+        for (int c = 0; c < NKC; ++c) load_slot_tile(sK + s * TILE_BYTES + c * DBM * 128, P, &full_bar[s], c * 64, tile * DBM, h);
+        if (++s == P.stages) {
+          s = 0;
+          ph ^= 1u;
+        }
+      }
+    }
+    __syncwarp();
+  } else if (warp == 1) {
+    // scores[128 tokens x nq16] = K tile (K-major: 128 B of dims per token row) * Q^T (K-major: 128 B of dims per q row)
+    constexpr uint32_t idesc = umma_idesc_bf16(DBM, NQ16, 0, 0);
+    if (elect_one()) {
+      mbar_wait(q_bar, 0);
+      const uint64_t q_desc0 = umma_desc_sw128(smem_u32(sQ), 16, 1024);
+      const uint64_t k_desc0 = umma_desc_sw128(smem_u32(sK), 16, 1024);
+      int s = 0, acc = 0;
+      uint32_t ph = 0, acc_ph = 0u;
+      for (int tile = slot; tile < ntiles; tile += nslots) {
+        mbar_wait(&tempty_bar[acc], ((acc_ph >> acc) & 1u) ^ 1u);
+        mbar_wait(&full_bar[s], ph);
+        tc_fence_after();
+        const uint32_t d_addr = tmem_base + static_cast<uint32_t>(acc * NQ16);
+        const uint64_t k_desc = k_desc0 + static_cast<uint64_t>((s * TILE_BYTES) >> 4);
+#pragma unroll
+        for (int k = 0; k < D / 16; ++k)
+          umma_bf16_ss(d_addr, k_desc + static_cast<uint64_t>(((k >> 2) * DBM * 128 + (k & 3) * 32) >> 4),
+                       q_desc0 + static_cast<uint64_t>(((k >> 2) * NQ16 * 128 + (k & 3) * 32) >> 4), idesc, k > 0 ? 1u : 0u);
+        umma_commit(&empty_bar[s]);
+        umma_commit(&tfull_bar[acc]);
+        acc_ph ^= 1u << acc;
+        acc = (acc + 1) % DN_NACC;
+        if (++s == P.stages) {
+          s = 0;
+          ph ^= 1u;
+        }
+      }
+    }
+    __syncwarp();
+  } else {
+    // ===== score read-out (the pair kernel's): thread = token, the qpk score columns in groups of 8 =====
+    const int qd = warp & 3;
+    const int row = qd * 32 + lane;
+    int acc = 0;
+    uint32_t acc_ph = 0u;
+    for (int tile = slot; tile < ntiles; tile += nslots) {
+      const int tok = tile * DBM + row;
+      mbar_wait(&tfull_bar[acc], (acc_ph >> acc) & 1u);
+      tc_fence_after();
+      uint32_t v[NQ16 / 8][8];
+      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(qd * 32) << 16) + static_cast<uint32_t>(acc * NQ16);
+      __syncwarp();
+#pragma unroll
+      for (int c = 0; c < NQ16 / 8; ++c)
+        if (c == 0 || c * 8 < P.qpk) tmem_ld_32x8(taddr + static_cast<uint32_t>(c * 8), v[c]);
+      tmem_ld_wait();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&tempty_bar[acc]);
+      if (tok < P.S) {
+#pragma unroll
+        for (int c = 0; c < NQ16 / 8; ++c)
+#pragma unroll
+          for (int g = 0; g < 8; ++g)
+            if (c * 8 + g < P.qpk)
+              P.out[static_cast<long long>(h * P.qpk + c * 8 + g) * P.ld_out + tok] = __uint_as_float(v[c][g]) * P.scale;
+      }
+      acc_ph ^= 1u << acc;
+      acc = (acc + 1) % DN_NACC;
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 256);
+  }
+}
+
+template <int D, int NQ16>
+__global__ void __launch_bounds__(DN_THREADS, 1) decode_dense_values_kernel(const __grid_constant__ DenseParams P) {
+  constexpr int NKC = D / 64;
+  constexpr int CHUNK_BYTES = DN_VBLK * 128;                  // 64 tokens x 64 dims: one MN-major chunk of M
+  constexpr int V_BYTES = 2 * CHUNK_BYTES;                    // M = 128 (D = 64: the upper chunk is zero)
+  constexpr int STAGE_BYTES = V_BYTES + NQ16 * 128;           // + the head's probability rows of the block
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + P.stages * STAGE_BYTES);
+  uint64_t* empty_bar = full_bar + DN_MAX_STAGES;
+  uint64_t* tfull_bar = empty_bar + DN_MAX_STAGES;
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tfull_bar + 1);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int h = static_cast<int>(blockIdx.x) % P.H;
+  const int ch = static_cast<int>(blockIdx.x) / P.H;     // softmax chunk: tokens [ch * kps * 64, (ch + 1) * kps * 64)
+  const int t0 = ch * P.kps * DN_VBLK;
+  const int t1 = min(P.S, t0 + P.kps * DN_VBLK);
+  const int nkb = (t1 - t0 + DN_VBLK - 1) / DN_VBLK;    // >= 1: the host drops empty chunks
+
+  if constexpr (D == 64) {
+    // rows 64..127 of the M = 128 product read this chunk: zeros, never loaded (their TMEM lanes are not read out)
+    for (int i = threadIdx.x; i < P.stages * CHUNK_BYTES / 16; i += DN_THREADS) {
+      const int st = i / (CHUNK_BYTES / 16), o = i - st * (CHUNK_BYTES / 16);
+      reinterpret_cast<uint4*>(smem + st * STAGE_BYTES + CHUNK_BYTES)[o] = make_uint4(0u, 0u, 0u, 0u);
+    }
+    fence_proxy_async_smem();
+  }
+  if (warp == 0 && lane == 0) {
+    for (int i = 0; i < P.stages; ++i) {
+      mbar_init(&full_bar[i], 1);
+      mbar_init(&empty_bar[i], 1);
+    }
+    mbar_init(tfull_bar, 1);
+    mbar_fence_init();
+    tma_prefetch_desc(&P.slot_map);
+    tma_prefetch_desc(&P.rows_map);
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, 64);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  if (warp == 0) {
+    if (elect_one()) {
+      int s = 0;
+      uint32_t ph = 0;
+      for (int kb = 0; kb < nkb; ++kb) {
+        const int tok = t0 + kb * DN_VBLK;
+        uint8_t* st = smem + s * STAGE_BYTES;
+        mbar_wait(&empty_bar[s], ph ^ 1u);
+        mbar_expect_tx(&full_bar[s], NKC * CHUNK_BYTES + NQ16 * 128);
+#pragma unroll
+        for (int c = 0; c < NKC; ++c) load_slot_tile(st + c * CHUNK_BYTES, P, &full_bar[s], c * 64, tok, h);
+        // tokens past S are zero in both operands (the maps end at S): the tail probabilities beyond the prefix stay out
+        tma_load_2d(st + V_BYTES, &P.rows_map, &full_bar[s], tok, h * P.qpk);
+        if (++s == P.stages) {
+          s = 0;
+          ph ^= 1u;
+        }
+      }
+    }
+    __syncwarp();
+  } else if (warp == 1) {
+    // U^T[D x nq16] += V tile^T (MN-major: 128 B of dims per token row, chunks of 64 dims CHUNK_BYTES apart) * P^T
+    // (K-major: 128 B of tokens per q row); K = 16 tokens per instruction: +2048 B on A, +32 B on B
+    constexpr uint32_t idesc = umma_idesc_bf16(128, NQ16, 1, 0);
+    if (elect_one()) {
+      const uint64_t a_desc0 = umma_desc_sw128(smem_u32(smem), CHUNK_BYTES, 1024);
+      const uint64_t b_desc0 = umma_desc_sw128(smem_u32(smem + V_BYTES), 16, 1024);
+      int s = 0;
+      uint32_t ph = 0;
+      for (int kb = 0; kb < nkb; ++kb) {
+        mbar_wait(&full_bar[s], ph);
+        tc_fence_after();
+        const uint64_t so = static_cast<uint64_t>((s * STAGE_BYTES) >> 4);
+#pragma unroll
+        for (int k = 0; k < DN_VBLK / 16; ++k)
+          umma_bf16_ss(tmem_base, a_desc0 + so + static_cast<uint64_t>((k * 2048) >> 4), b_desc0 + so + static_cast<uint64_t>((k * 32) >> 4),
+                       idesc, (kb > 0 || k > 0) ? 1u : 0u);
+        umma_commit(&empty_bar[s]);
+        if (++s == P.stages) {
+          s = 0;
+          ph ^= 1u;
+        }
+      }
+      umma_commit(tfull_bar);
+    }
+    __syncwarp();
+  } else {
+    // ===== read-out: thread = output dim d (TMEM lane), the qpk q-row columns in groups of 8 =====
+    const int qd = warp & 3;
+    const int d = qd * 32 + lane;
+    if (qd * 32 < D) {
+      mbar_wait(tfull_bar, 0);
+      tc_fence_after();
+      uint32_t v[NQ16 / 8][8];
+      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(qd * 32) << 16);
+      __syncwarp();
+#pragma unroll
+      for (int c = 0; c < NQ16 / 8; ++c)
+        if (c == 0 || c * 8 < P.qpk) tmem_ld_32x8(taddr + static_cast<uint32_t>(c * 8), v[c]);
+      tmem_ld_wait();
+      float* slab = P.out + (static_cast<long long>(ch) * P.rows + h * P.qpk) * D + d;
+#pragma unroll
+      for (int c = 0; c < NQ16 / 8; ++c)
+#pragma unroll
+        for (int g = 0; g < 8; ++g)
+          if (c * 8 + g < P.qpk) slab[static_cast<long long>(c * 8 + g) * D] = __uint_as_float(v[c][g]);
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 64);
   }
 }
 
@@ -1655,38 +1954,125 @@ extern "C" size_t xkv_decode_workspace_bytes(int Hq, int S, int T, int rv) {
   return b + 1024;
 }
 
-// Multi-token step: q / out (Hq * Tq, D), row hq * Tq + t = query token t of q head hq; the last Tq of the T tail tokens
-// are the queries' own and attention among them is causal.  Internally every per-head quantity is per ROW (rows = Hq Tq,
-// qpk below = rows per kv head).
-extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
-                                          const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,
-                                          const void* Vv_layer, int64_t ldv_v, int S, const void* cos, const void* sin,
-                                          int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
-                                          int64_t tail_stride_t, float scale, void* out, void* workspace,
-                                          size_t workspace_bytes, void* stream, float* lse_out) {
-  XKV_REQUIRE(q && A_k && Vk_layer && A_v && Vv_layer && out && workspace, "decode: null argument");
-  XKV_REQUIRE(D == 64 || D == 128, "decode: head_dim %d not supported (64 or 128)", D);
-  XKV_REQUIRE(Tq >= 1, "decode: Tq=%d query tokens (at least 1)", Tq);
-  XKV_REQUIRE(H >= 1 && Hq >= 1 && Hq % H == 0, "decode: unsupported head counts Hq=%d H=%d", Hq, H);
-  XKV_REQUIRE((Hq / H) * Tq <= 64 && Hq * Tq <= 512,
-              "decode: %d q heads per kv head x %d query tokens (at most 64 rows per kv head) and %d q heads (at most 512 "
-              "rows in all) is past the fused kernel's bounds", Hq / H, Tq, Hq);
-  XKV_REQUIRE(S >= 1 && T >= 0 && rk >= 1 && rv >= 1 && rv % 2 == 0, "decode: bad sizes");
-  // a single query may come without a tail (xkv_decode_attention); several queries attend to their own tokens
-  XKV_REQUIRE(Tq == 1 || T >= Tq, "decode: the tail (T=%d) must hold the Tq=%d query tokens", T, Tq);
-  XKV_REQUIRE(T == 0 || (k_tail && v_tail), "decode: tail pointers missing");
-  XKV_REQUIRE((cos == nullptr) == (sin == nullptr), "decode: cos and sin must both be given or both be null");
-  XKV_REQUIRE(cos == nullptr || ld_cs % 8 == 0, "decode: cos/sin row stride must be a multiple of 8");
-  const int rows = Hq * Tq;
-  XKV_REQUIRE(workspace_bytes >= xkv_decode_workspace_bytes(rows, S, T, rv), "decode: workspace too small");
-  XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "decode: workspace must be 256-byte aligned");
+// A dense slot of a one-sided group: (H, S, D) or (S, H, D) view, unit inner stride
+struct DenseSlot {
+  const void* ptr;
+  int64_t stride_h, stride_t;
+};
+
+// 3-D tensor map over a dense slot: box {64 dims, `tile` tokens, 1 head}; the token and head dimensions go in the order
+// of their strides.  Returns the map's token dimension (1 or 2) through tok_dim.
+static int encode_slot_map(CUtensorMap* map, const DenseSlot& slot, int D, int S, int H, int tile, int* tok_dim) {
+  const bool tok_first = slot.stride_t <= slot.stride_h;
+  const uint64_t dims[3] = {static_cast<uint64_t>(D), static_cast<uint64_t>(tok_first ? S : H), static_cast<uint64_t>(tok_first ? H : S)};
+  const uint64_t strides[2] = {static_cast<uint64_t>(tok_first ? slot.stride_t : slot.stride_h),
+                               static_cast<uint64_t>(tok_first ? slot.stride_h : slot.stride_t)};
+  const uint32_t box[3] = {64u, tok_first ? static_cast<uint32_t>(tile) : 1u, tok_first ? 1u : static_cast<uint32_t>(tile)};
+  *tok_dim = tok_first ? 1 : 2;
+  return encode_tmap_3d_bf16(map, slot.ptr, dims, strides, box);
+}
+
+// Chunks of the dense-value product: about one wave of (kv head, chunk) CTAs, at most 64 (the slab reduction's limit),
+// no empty chunk.
+static int dense_value_chunks(int S, int H) {
+  const int nkb = (S + DN_VBLK - 1) / DN_VBLK;
+  int split = device_sm_count() / H;
+  if (split > nkb) split = nkb;
+  if (split > 64) split = 64;
+  if (split < 1) split = 1;
+  const int per = (nkb + split - 1) / split;
+  return (nkb + per - 1) / per;
+}
+
+template <int D, int NQ16>
+static int launch_dense_kernel(bool values, const DenseParams& p, int grid, size_t smem, cudaStream_t st) {
+  static PerDevice<bool> configured;
+  if (!configured()) {
+    XKV_CHECK_CUDA(cudaFuncSetAttribute(decode_dense_scores_kernel<D, NQ16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        static_cast<int>(R_SMEM_LIMIT)));
+    XKV_CHECK_CUDA(cudaFuncSetAttribute(decode_dense_values_kernel<D, NQ16>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        static_cast<int>(R_SMEM_LIMIT)));
+    configured() = true;
+  }
+  if (values)
+    decode_dense_values_kernel<D, NQ16><<<grid, DN_THREADS, smem, st>>>(p);
+  else
+    decode_dense_scores_kernel<D, NQ16><<<grid, DN_THREADS, smem, st>>>(p);
+  XKV_LAUNCHED();
+  return 0;
+}
+
+template <int D>
+static int launch_dense_d(bool values, const DenseParams& p, int nq16, int grid, size_t smem, cudaStream_t st) {
+  switch (nq16) {
+    case 16: return launch_dense_kernel<D, 16>(values, p, grid, smem, st);
+    case 32: return launch_dense_kernel<D, 32>(values, p, grid, smem, st);
+    case 48: return launch_dense_kernel<D, 48>(values, p, grid, smem, st);
+    default: return launch_dense_kernel<D, 64>(values, p, grid, smem, st);
+  }
+}
+
+// scores[r][t] = scale * q_r . K[t, h(r)] over the dense (already rotated) prefix keys: decode_dense_scores_kernel,
+// one CTA per (kv head, slot) up to one per SM.
+static int launch_dense_scores(const void* q, int rows, int H, int D, const DenseSlot& k, int S, float scale, float* scores,
+                               long long ldl, cudaStream_t st) {
+  static thread_local DenseParams p;
+  std::memset(&p, 0, sizeof(p));
+  const int qpk = rows / H, nq16 = pair_nq16(qpk);
+  int rc = encode_slot_map(&p.slot_map, k, D, S, H, DBM, &p.slot_tok_dim);
+  if (rc) return rc;
+  rc = encode_tmap_2d_bf16(&p.rows_map, q, D, rows, D, 64, nq16);
+  if (rc) return rc;
+  p.out = scores, p.ld_out = ldl, p.S = S, p.H = H, p.qpk = qpk, p.rows = rows, p.scale = scale;
+  const size_t tile = static_cast<size_t>(D / 64) * DBM * 128, fixed = static_cast<size_t>(D / 64) * nq16 * 128 + 1024 + 512;
+  p.stages = static_cast<int>((R_SMEM_LIMIT - fixed) / tile);
+  if (p.stages > DN_MAX_STAGES) p.stages = DN_MAX_STAGES;
+  const int ntiles = (S + DBM - 1) / DBM;
+  int grid = device_sm_count() < ntiles * H ? device_sm_count() : ntiles * H;
+  if (grid < H) grid = H;
+  const size_t smem = fixed + p.stages * tile;
+  return D == 128 ? launch_dense_d<128>(false, p, nq16, grid, smem, st) : launch_dense_d<64>(false, p, nq16, grid, smem, st);
+}
+
+// slabs[c] (rows, D) = P[:, chunk c] V (kv head of the row) over the dense prefix values: decode_dense_values_kernel,
+// one CTA per (kv head, chunk)
+static int launch_dense_values(const __nv_bfloat16* prob, long long ldp, int rows, int H, int D, const DenseSlot& v, int S,
+                               int kps, int nchunks, float* slabs, cudaStream_t st) {
+  static thread_local DenseParams p;
+  std::memset(&p, 0, sizeof(p));
+  const int qpk = rows / H, nq16 = pair_nq16(qpk);
+  int rc = encode_slot_map(&p.slot_map, v, D, S, H, DN_VBLK, &p.slot_tok_dim);
+  if (rc) return rc;
+  rc = encode_tmap_2d_bf16(&p.rows_map, prob, S, rows, ldp, 64, nq16);
+  if (rc) return rc;
+  p.out = slabs, p.ld_out = D, p.S = S, p.H = H, p.qpk = qpk, p.rows = rows, p.kps = kps;
+  const size_t stage = 2 * DN_VBLK * 128 + static_cast<size_t>(nq16) * 128, fixed = 1024 + 512;
+  p.stages = static_cast<int>((R_SMEM_LIMIT - fixed) / stage);
+  if (p.stages > DN_MAX_STAGES) p.stages = DN_MAX_STAGES;
+  const size_t smem = fixed + p.stages * stage;
+  return D == 128 ? launch_dense_d<128>(true, p, nq16, H * nchunks, smem, st)
+                  : launch_dense_d<64>(true, p, nq16, H * nchunks, smem, st);
+}
+
+// The fused chain behind xkv_decode_attention_multi (both sides factored: A_k and A_v given) and
+// xkv_decode_attention_half (one side given as a dense slot instead): scores of the prefix, chunk-local softmax with the
+// causal tail, the value product per chunk, slab reduction + combine.  Arguments are checked by the callers.
+static int decode_chain(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                        const void* Vk_layer, int64_t ldv_k, const DenseSlot& k_dense, const void* A_v, int64_t lda_v, int rv,
+                        const void* Vv_layer, int64_t ldv_v, const DenseSlot& v_dense, int S, const void* cos,
+                        const void* sin, int64_t ld_cs, const void* k_tail, const void* v_tail, int T,
+                        int64_t tail_stride_h, int64_t tail_stride_t, float scale, void* out, void* workspace,
+                        void* stream, float* lse_out) {
   cudaStream_t st = as_stream(stream);
+  const bool dense_k = A_k == nullptr, dense_v = A_v == nullptr;
+  const int rows = Hq * Tq;
   const int qpk = rows / H;
+  const int vw = dense_v ? D : rv;   // columns of U: the value factor's rank, or head_dim for a dense value slot
   const size_t L = static_cast<size_t>(S) + T;
   const long long ldl = static_cast<long long>((L + 63) / 64 * 64);
   const int nkb_s = (S + 63) / 64;
   (void)nkb_s;
-  const int split = decode_split_k(S, rv, rows);
+  const int split = dense_v ? dense_value_chunks(S, H) : decode_split_k(S, rv, rows);
   char* w = static_cast<char*>(workspace);
   float* scores = reinterpret_cast<float*>(w);
   w += al(rows * ldl * 4);
@@ -1696,10 +2082,11 @@ extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, 
   float* chunk_max = rowsum + rows * SM_MAX_CHUNKS;
   w += al(2 * rows * SM_MAX_CHUNKS * 4);
   float* u_slabs = reinterpret_cast<float*>(w);
-  w += al(static_cast<size_t>(split + 1) * rows * rv * 4);
+  w += al(static_cast<size_t>(split + 1) * rows * vw * 4);
 
-  // ---- scores of the compressed prefix: fused reconstruct + RoPE + q.K ----
-  int rc = launch_scores(q, rows, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, S, cos, sin, ld_cs, scale, scores, ldl, st);
+  // ---- scores of the prefix: fused reconstruct + RoPE + q.K, or q.K over the dense rotated keys ----
+  int rc = dense_k ? launch_dense_scores(q, rows, H, D, k_dense, S, scale, scores, ldl, st)
+                   : launch_scores(q, rows, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, S, cos, sin, ld_cs, scale, scores, ldl, st);
   if (rc) return rc;
   // ---- softmax with chunk-local maxima: chunk c = token range of split-K slab c, last chunk = the dense tail ----
   const int nkb_p = (S + 63) / 64;
@@ -1711,6 +2098,32 @@ extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, 
                                                           tail_stride_t, qpk, D, scale, prob, ldl, chunk_max, rowsum, nullptr, nullptr,
                                                           0.f);
   XKV_LAUNCHED();
+  if (dense_v) {
+    // ---- U_c = P[:, chunk c] V_h per softmax chunk, then o = (sum_c w_c U_c + P_tail V_tail) / rowsum ----
+    rc = launch_dense_values(prob, ldl, rows, H, D, v_dense, S, kps, split, u_slabs, st);
+    if (rc) return rc;
+    cudaLaunchConfig_t cfg;
+    std::memset(&cfg, 0, sizeof(cfg));
+    cfg.gridDim = dim3(rows, RC_CL, 1);
+    cfg.blockDim = dim3(256, 1, 1);
+    cfg.dynamicSmemBytes = D * sizeof(float);
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 1;
+    attr[0].val.clusterDim.y = RC_CL;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, reduce_combine_kernel<true>, static_cast<const float*>(u_slabs), split,
+                                      static_cast<long long>(rows) * D, D, static_cast<const __nv_bfloat16*>(nullptr),
+                                      0LL, static_cast<const __nv_bfloat16*>(prob), ldl, S, T, Tq,
+                                      static_cast<const __nv_bfloat16*>(v_tail), static_cast<long long>(tail_stride_h),
+                                      static_cast<long long>(tail_stride_t), static_cast<const float*>(rowsum), qpk, D,
+                                      static_cast<__nv_bfloat16*>(out), static_cast<const float*>(chunk_max), nchunks, lse_out));
+    XKV_LAUNCHED();
+    return 0;
+  }
   // ---- U = P[:, :S] * A_v  (tokens are the contraction: P K-major, A_v MN-major) ----
   xkv_gemm_problem gp;
   std::memset(&gp, 0, sizeof(gp));
@@ -1745,7 +2158,7 @@ extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, 
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, reduce_combine_kernel, static_cast<const float*>(u_slabs), split,
+    XKV_CHECK_CUDA(cudaLaunchKernelEx(&cfg, reduce_combine_kernel<false>, static_cast<const float*>(u_slabs), split,
                                       static_cast<long long>(rows) * rv, rv, static_cast<const __nv_bfloat16*>(Vv_layer),
                                       static_cast<long long>(ldv_v), static_cast<const __nv_bfloat16*>(prob), ldl, S, T, Tq,
                                       static_cast<const __nv_bfloat16*>(v_tail), static_cast<long long>(tail_stride_h),
@@ -1764,6 +2177,80 @@ extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, 
       static_cast<__nv_bfloat16*>(out), chunk_max, nchunks, lse_out);
   XKV_LAUNCHED();
   return 0;
+}
+
+// Multi-token step: q / out (Hq * Tq, D), row hq * Tq + t = query token t of q head hq; the last Tq of the T tail tokens
+// are the queries' own and attention among them is causal.  Internally every per-head quantity is per ROW (rows = Hq Tq,
+// qpk below = rows per kv head).
+extern "C" int xkv_decode_attention_multi(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                                          const void* Vk_layer, int64_t ldv_k, const void* A_v, int64_t lda_v, int rv,
+                                          const void* Vv_layer, int64_t ldv_v, int S, const void* cos, const void* sin,
+                                          int64_t ld_cs, const void* k_tail, const void* v_tail, int T, int64_t tail_stride_h,
+                                          int64_t tail_stride_t, float scale, void* out, void* workspace,
+                                          size_t workspace_bytes, void* stream, float* lse_out) {
+  XKV_REQUIRE(q && A_k && Vk_layer && A_v && Vv_layer && out && workspace, "decode: null argument");
+  XKV_REQUIRE(D == 64 || D == 128, "decode: head_dim %d not supported (64 or 128)", D);
+  XKV_REQUIRE(Tq >= 1, "decode: Tq=%d query tokens (at least 1)", Tq);
+  XKV_REQUIRE(H >= 1 && Hq >= 1 && Hq % H == 0, "decode: unsupported head counts Hq=%d H=%d", Hq, H);
+  XKV_REQUIRE((Hq / H) * Tq <= 64 && Hq * Tq <= 512,
+              "decode: %d q heads per kv head x %d query tokens (at most 64 rows per kv head) and %d q heads (at most 512 "
+              "rows in all) is past the fused kernel's bounds", Hq / H, Tq, Hq);
+  XKV_REQUIRE(S >= 1 && T >= 0 && rk >= 1 && rv >= 1 && rv % 2 == 0, "decode: bad sizes");
+  // a single query may come without a tail (xkv_decode_attention); several queries attend to their own tokens
+  XKV_REQUIRE(Tq == 1 || T >= Tq, "decode: the tail (T=%d) must hold the Tq=%d query tokens", T, Tq);
+  XKV_REQUIRE(T == 0 || (k_tail && v_tail), "decode: tail pointers missing");
+  XKV_REQUIRE((cos == nullptr) == (sin == nullptr), "decode: cos and sin must both be given or both be null");
+  XKV_REQUIRE(cos == nullptr || ld_cs % 8 == 0, "decode: cos/sin row stride must be a multiple of 8");
+  XKV_REQUIRE(workspace_bytes >= xkv_decode_workspace_bytes(Hq * Tq, S, T, rv), "decode: workspace too small");
+  XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "decode: workspace must be 256-byte aligned");
+  const DenseSlot none = {nullptr, 0, 0};
+  return decode_chain(q, Hq, Tq, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, none, A_v, lda_v, rv, Vv_layer, ldv_v, none, S, cos,
+                      sin, ld_cs, k_tail, v_tail, T, tail_stride_h, tail_stride_t, scale, out, workspace, stream, lse_out);
+}
+
+extern "C" size_t xkv_decode_half_workspace_bytes(int rows, int S, int T, int value_width) {
+  // the layout of xkv_decode_workspace_bytes; the slabs are value_width (r_v, or head_dim for a dense value slot) wide
+  return xkv_decode_workspace_bytes(rows, S, T, value_width);
+}
+
+extern "C" int xkv_decode_attention_half(const void* q, int Hq, int Tq, int H, int D, const void* A_k, int64_t lda_k, int rk,
+                                         const void* Vk_layer, int64_t ldv_k, const void* k_dense, int64_t k_stride_h,
+                                         int64_t k_stride_t, const void* A_v, int64_t lda_v, int rv, const void* Vv_layer,
+                                         int64_t ldv_v, const void* v_dense, int64_t v_stride_h, int64_t v_stride_t, int S,
+                                         const void* cos, const void* sin, int64_t ld_cs, const void* k_tail,
+                                         const void* v_tail, int T, int64_t tail_stride_h, int64_t tail_stride_t,
+                                         float scale, void* out, void* workspace, size_t workspace_bytes, void* stream,
+                                         float* lse_out) {
+  const bool kf = A_k != nullptr, vf = A_v != nullptr;
+  XKV_REQUIRE(!(kf && k_dense) && !(vf && v_dense), "decode_half: a side is given both as factors and as a dense slot");
+  XKV_REQUIRE((kf || k_dense) && (vf || v_dense), "decode_half: the key and the value side each need factors or a dense slot");
+  XKV_REQUIRE(kf != vf,
+              "decode_half: exactly one side must be factored (both factored: xkv_decode_attention_multi; both dense: SDPA)");
+  XKV_REQUIRE(q && out && workspace && (!kf || Vk_layer) && (!vf || Vv_layer), "decode_half: null argument");
+  XKV_REQUIRE(D == 64 || D == 128, "decode_half: head_dim %d not supported (64 or 128)", D);
+  XKV_REQUIRE(Tq >= 1, "decode_half: Tq=%d query tokens (at least 1)", Tq);
+  XKV_REQUIRE(H >= 1 && Hq >= 1 && Hq % H == 0, "decode_half: unsupported head counts Hq=%d H=%d", Hq, H);
+  XKV_REQUIRE((Hq / H) * Tq <= 64 && Hq * Tq <= 512,
+              "decode_half: %d q heads per kv head x %d query tokens (at most 64 rows per kv head) and %d q heads (at most "
+              "512 rows in all) is past the fused kernel's bounds", Hq / H, Tq, Hq);
+  XKV_REQUIRE(S >= 1 && T >= 0 && (!kf || rk >= 1) && (!vf || (rv >= 1 && rv % 2 == 0)), "decode_half: bad sizes");
+  XKV_REQUIRE(Tq == 1 || T >= Tq, "decode_half: the tail (T=%d) must hold the Tq=%d query tokens", T, Tq);
+  XKV_REQUIRE(T == 0 || (k_tail && v_tail), "decode_half: tail pointers missing");
+  XKV_REQUIRE((cos == nullptr) == (sin == nullptr), "decode_half: cos and sin must both be given or both be null");
+  XKV_REQUIRE(cos == nullptr || ld_cs % 8 == 0, "decode_half: cos/sin row stride must be a multiple of 8");
+  const void* dense = kf ? v_dense : k_dense;
+  const int64_t sh = kf ? v_stride_h : k_stride_h, stt = kf ? v_stride_t : k_stride_t;
+  // TMA reads the slot in place: 16-byte aligned base, strides of whole 16-byte units (a slot is never copied)
+  XKV_REQUIRE((reinterpret_cast<uintptr_t>(dense) & 15) == 0 && sh > 0 && stt > 0 && sh % 8 == 0 && stt % 8 == 0,
+              "decode_half: the dense %s slot needs a 16-byte aligned base and head / token strides that are positive "
+              "multiples of 8 elements (got %lld / %lld)", kf ? "value" : "key", static_cast<long long>(sh),
+              static_cast<long long>(stt));
+  XKV_REQUIRE(kf || (reinterpret_cast<uintptr_t>(q) & 15) == 0, "decode_half: q must be 16-byte aligned");
+  XKV_REQUIRE(workspace_bytes >= xkv_decode_half_workspace_bytes(Hq * Tq, S, T, vf ? rv : D), "decode_half: workspace too small");
+  XKV_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "decode_half: workspace must be 256-byte aligned");
+  const DenseSlot ks = {k_dense, k_stride_h, k_stride_t}, vs = {v_dense, v_stride_h, v_stride_t};
+  return decode_chain(q, Hq, Tq, H, D, A_k, lda_k, rk, Vk_layer, ldv_k, ks, A_v, lda_v, rv, Vv_layer, ldv_v, vs, S, cos, sin,
+                      ld_cs, k_tail, v_tail, T, tail_stride_h, tail_stride_t, scale, out, workspace, stream, lse_out);
 }
 
 extern "C" int xkv_decode_attention_lse(const void* q, int Hq, int H, int D, const void* A_k, int64_t lda_k, int rk,

@@ -77,4 +77,8 @@ int device_sm_count();
 int encode_tmap_2d_bf16(CUtensorMap* map, const void* base, uint64_t inner, uint64_t outer, uint64_t ld_elems,
                         uint32_t box_inner, uint32_t box_outer);
 
+// Encode a 3-D bf16 tensor map: dims[0] contiguous, dims[1] / dims[2] `strides_elems` apart (any order), 128-byte swizzle.
+int encode_tmap_3d_bf16(CUtensorMap* map, const void* base, const uint64_t dims[3], const uint64_t strides_elems[2],
+                        const uint32_t box[3]);
+
 }  // namespace xkv

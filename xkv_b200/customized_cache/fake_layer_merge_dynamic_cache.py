@@ -352,36 +352,56 @@ class FakeLayerMergingCache(DynamicCache):
                scaling: float, key_pre_rope: Optional[torch.Tensor] = None, cos: Optional[torch.Tensor] = None,
                sin: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
         """Decode step of one layer: append the Tq new (post-RoPE) tokens and attend over the factored cache with
-        the fused kernel, causally among the new tokens.  query (1, Hq, Tq, D) -> (1, Hq, Tq, D).  Returns None, having
-        appended nothing, when the layer is not factored on both sides or the step is past the fused kernel's bounds
-        ((Hq / H) * Tq > 64 or Hq * Tq > 512); the caller then uses the dense path.  key_pre_rope / cos / sin of the new
-        positions are only needed when decode tokens are folded into the factors (compress_decode_tokens); the fold
-        runs at single-token steps only, since the tokens of a multi-token step may still be rejected (crop)."""
+        the fused kernel, causally among the new tokens.  query (1, Hq, Tq, D) -> (1, Hq, Tq, D).  A group factored on
+        both sides runs ops.decode_attention; a one-sided group (one slot factored, the other kept dense by the merge flags
+        or by a rank that does not fit it) runs ops.decode_attention_half over the factors and the layer's dense slot
+        (``dense_k``: rotated keys, ``dense_v``: the prefill's values).  Returns None, having appended nothing, when the
+        layer is not factored on either side or the step is past the fused kernels' bounds ((Hq / H) * Tq > 64 or
+        Hq * Tq > 512); the caller then uses the dense path.  key_pre_rope / cos / sin of the new positions are only needed
+        when decode tokens are folded into the factors (compress_decode_tokens); the fold runs at single-token steps of
+        groups factored on both sides only, since the tokens of a multi-token step may still be rejected (crop) and a
+        one-sided group has no factor to fold its dense side into: there the decode tokens stay dense and exact."""
         layer = self._layer(layer_idx)
         st = layer.group
-        if st is None or st.factors.key is None or st.factors.value is None:
+        if st is None:
+            return None
+        fk, fv = st.factors.key, st.factors.value
+        if (fk is None and layer.dense_k is None) or (fv is None and layer.dense_v is None) or (fk is None and fv is None):
             return None
         hq, tq = query.shape[1], query.shape[2]
         h, d = st.heads, st.head_dim
         if (hq // h) * tq > 64 or hq * tq > 512:
             return None
-        fold = self.compress_decode_tokens and key_pre_rope is not None
+        one_sided = fk is None or fv is None
+        fold = self.compress_decode_tokens and key_pre_rope is not None and not one_sided
         layer.append_tail(key, value, key_pre_rope if fold else None)
         if fold and layer_idx == st.layer_ids[0] and st.re_apply_rope and cos is not None:
             cs = cos.reshape(-1, cos.shape[-1])[-tq:].to(torch.bfloat16)
             sn = sin.reshape(-1, sin.shape[-1])[-tq:].to(torch.bfloat16)
             st.tail_rope.extend(zip(cs, sn))
         rows = slice(layer.index_in_group * h * d, (layer.index_in_group + 1) * h * d)
-        fk, fv = st.factors.key, st.factors.value
-        need = ops.decode_workspace_bytes(hq * tq, layer.prefill_len, layer.tail_len, fv.rank)
+        n_tok = layer.prefill_len
+        if one_sided:
+            need = ops.decode_half_workspace_bytes(hq * tq, n_tok, layer.tail_len, fv.rank if fv is not None else d)
+        else:
+            need = ops.decode_workspace_bytes(hq * tq, n_tok, layer.tail_len, fv.rank)
         if self._workspace is None or self._workspace.numel() < need:
             self._workspace = torch.empty(int(need * 1.25) + 4096, dtype=torch.uint8, device=query.device)
-        n_tok = layer.prefill_len
-        out = ops.decode_attention(
-            query[0, :, 0, :] if tq == 1 else query[0], fk.A_storage[:n_tok], fk.V[rows], fv.A_storage[:n_tok], fv.V[rows],
-            h, st.cos[:n_tok] if st.re_apply_rope else None, st.sin[:n_tok] if st.re_apply_rope else None,
-            layer.tail_k[0, :, : layer.tail_len], layer.tail_v[0, :, : layer.tail_len], scaling,
-            workspace=self._workspace)
+        q = query[0, :, 0, :] if tq == 1 else query[0]
+        cos_k = st.cos[:n_tok] if st.re_apply_rope and fk is not None else None
+        sin_k = st.sin[:n_tok] if st.re_apply_rope and fk is not None else None
+        k_tail, v_tail = layer.tail_k[0, :, : layer.tail_len], layer.tail_v[0, :, : layer.tail_len]
+        if one_sided:
+            # dense slots as token-major (S, H, D) views of the (1, H, S, D) tensors the merge kept
+            out = ops.decode_attention_half(
+                q, h, a_k=fk.A_storage[:n_tok] if fk is not None else None, vk_layer=fk.V[rows] if fk is not None else None,
+                k_dense=layer.dense_k[0, :, :n_tok].transpose(0, 1) if fk is None else None,
+                a_v=fv.A_storage[:n_tok] if fv is not None else None, vv_layer=fv.V[rows] if fv is not None else None,
+                v_dense=layer.dense_v[0, :, :n_tok].transpose(0, 1) if fv is None else None,
+                cos=cos_k, sin=sin_k, k_tail=k_tail, v_tail=v_tail, scale=scaling, workspace=self._workspace)
+        else:
+            out = ops.decode_attention(q, fk.A_storage[:n_tok], fk.V[rows], fv.A_storage[:n_tok], fv.V[rows], h, cos_k, sin_k,
+                                       k_tail, v_tail, scaling, workspace=self._workspace)
         if fold and tq == 1 and layer_idx == st.layer_ids[-1]:
             self._fold_tail(st)
         return out[None, :, None, :] if tq == 1 else out[None]
@@ -416,6 +436,8 @@ class FakeLayerMergingCache(DynamicCache):
         append the result to A_k / A_v.  The tokens leave the dense tails.  Each token's RoPE row was recorded when
         it was appended (``st.tail_rope``); if the tails are not uniform (a layer took the dense path for a step, a
         pre-RoPE copy is missing, a RoPE row is missing) nothing is folded and the tokens simply stay dense (exact)."""
+        if st.factors.key is None or st.factors.value is None:
+            return   # a one-sided group keeps its decode tokens dense: its dense slot has no factor to take them
         layers = [self._layer(i) for i in st.layer_ids]
         t = layers[0].tail_len
         if t == 0 or any(l.tail_len != t or l.tail_kpre is None or l.kpre_from > 0 for l in layers):

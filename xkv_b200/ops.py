@@ -413,6 +413,80 @@ def decode_attention(q: torch.Tensor, a_k: torch.Tensor, vk_layer: torch.Tensor,
     return out
 
 
+def decode_half_workspace_bytes(rows: int, s: int, t: int, value_width: int) -> int:
+    return int(_lib.load().xkv_decode_half_workspace_bytes(rows, s, t, value_width))
+
+
+def _dense_slot(x: torch.Tensor, s: int, h: int, d: int, name: str) -> Tuple[int, int]:
+    """(head stride, token stride) of a dense prefix slot given as an (S, H, D) or (H, S, D) view."""
+    if x.dim() != 3 or x.dtype != torch.bfloat16 or x.stride(-1) != 1:
+        raise _lib.XkvError(f"decode_attention_half: {name} must be a bf16 (S, H, D) or (H, S, D) view with unit inner stride")
+    if tuple(x.shape) == (s, h, d):
+        return x.stride(1), x.stride(0)
+    if tuple(x.shape) == (h, s, d):
+        return x.stride(0), x.stride(1)
+    raise _lib.XkvError(f"decode_attention_half: {name} has shape {tuple(x.shape)}, expected ({s}, {h}, {d}) or ({h}, {s}, {d})")
+
+
+def decode_attention_half(q: torch.Tensor, num_kv_heads: int, *, a_k: Optional[torch.Tensor] = None,
+                          vk_layer: Optional[torch.Tensor] = None, k_dense: Optional[torch.Tensor] = None,
+                          a_v: Optional[torch.Tensor] = None, vv_layer: Optional[torch.Tensor] = None,
+                          v_dense: Optional[torch.Tensor] = None, cos: Optional[torch.Tensor] = None,
+                          sin: Optional[torch.Tensor] = None, k_tail: Optional[torch.Tensor] = None,
+                          v_tail: Optional[torch.Tensor] = None, scale: float, out: Optional[torch.Tensor] = None,
+                          workspace: Optional[torch.Tensor] = None, lse_out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """:func:`decode_attention` for a one-sided group: exactly one side is factored (a_k / vk_layer, or a_v / vv_layer),
+    the other is the dense prefix slot (k_dense: rotated keys, or v_dense), an (S, H, D) or (H, S, D) view with unit inner
+    stride read in place (strides multiples of 8 elements, else XkvError; it is never copied).  cos / sin rotate a
+    factored key side only.  q, the tail, lse_out, the multi-token form and the bounds are those of decode_attention."""
+    _require_cuda(q, a_k, vk_layer, k_dense, a_v, vv_layer, v_dense, cos, sin, k_tail, v_tail, out, workspace, lse_out)
+    if (a_k is None) == (k_dense is None) or (a_v is None) == (v_dense is None):
+        raise _lib.XkvError("decode_attention_half: give each side either as factors or as a dense slot")
+    if (a_k is None) == (a_v is None):
+        raise _lib.XkvError("decode_attention_half: exactly one side must be factored (both factored: decode_attention; "
+                            "both dense: SDPA)")
+    if q.dim() not in (2, 3):
+        raise _lib.XkvError("decode_attention_half: q must be (Hq, D) or (Hq, Tq, D)")
+    hq, d = q.shape[0], q.shape[-1]
+    tq = q.shape[1] if q.dim() == 3 else 1
+    if lse_out is not None and (lse_out.dtype != torch.float32 or lse_out.numel() < hq * tq or not lse_out.is_contiguous()):
+        raise _lib.XkvError("decode_attention_half: lse_out must be a contiguous CUDA fp32 tensor of Hq * Tq elements")
+    s = (a_k if a_k is not None else a_v).shape[0]
+    h = num_kv_heads
+    for name, x in (("q", q), ("a_k", a_k), ("vk_layer", vk_layer), ("a_v", a_v), ("vv_layer", vv_layer)):
+        if x is not None and (x.dtype != torch.bfloat16 or x.stride(-1) != 1):
+            raise _lib.XkvError(f"decode_attention_half: {name} must be bf16 with unit inner stride")
+    if (a_k is not None and vk_layer is None) or (a_v is not None and vv_layer is None):
+        raise _lib.XkvError("decode_attention_half: a factored side needs its right factor rows (vk_layer / vv_layer)")
+    ksh, kst = _dense_slot(k_dense, s, h, d, "k_dense") if k_dense is not None else (0, 0)
+    vsh, vst = _dense_slot(v_dense, s, h, d, "v_dense") if v_dense is not None else (0, 0)
+    if not q.is_contiguous():
+        q = q.contiguous()
+    if cos is not None and (cos.dtype != torch.bfloat16 or cos.stride(-1) != 1 or cos.shape[0] < s):
+        raise _lib.XkvError("decode_attention_half: cos/sin must be bf16 (S, D) tables")
+    t = 0 if k_tail is None else k_tail.shape[1]
+    sh = st = 0
+    if t > 0:
+        if k_tail.stride() != v_tail.stride() or k_tail.stride(-1) != 1:
+            raise _lib.XkvError("decode_attention_half: k_tail / v_tail must share strides, unit inner stride")
+        sh, st = k_tail.stride(0), k_tail.stride(1)
+    rk = a_k.shape[1] if a_k is not None else 0
+    rv = a_v.shape[1] if a_v is not None else 0
+    need = decode_half_workspace_bytes(hq * tq, s, t, rv if a_v is not None else d)
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty(need, dtype=torch.uint8, device=q.device)
+    if out is None:
+        out = torch.empty(*q.shape, dtype=torch.bfloat16, device=q.device)
+    check(_lib.load().xkv_decode_attention_half(
+        _ptr(q), hq, tq, h, d, _ptr(a_k), a_k.stride(0) if a_k is not None else 0, rk, _ptr(vk_layer),
+        vk_layer.stride(0) if vk_layer is not None else 0, _ptr(k_dense), ksh, kst, _ptr(a_v),
+        a_v.stride(0) if a_v is not None else 0, rv, _ptr(vv_layer), vv_layer.stride(0) if vv_layer is not None else 0,
+        _ptr(v_dense), vsh, vst, s, _ptr(cos), _ptr(sin), cos.stride(0) if cos is not None else 0,
+        _ptr(k_tail if t else None), _ptr(v_tail if t else None), t, sh, st, C.c_float(scale), _ptr(out),
+        C.c_void_p(workspace.data_ptr()), workspace.numel(), _stream(), _ptr(lse_out)))
+    return out
+
+
 def decode_absorbed(q_hat: torch.Tensor, a: torch.Tensor, scale: float, row_scale: Optional[torch.Tensor] = None,
                     bias_q: Optional[torch.Tensor] = None, bias_k: Optional[torch.Tensor] = None,
                     workspace: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
